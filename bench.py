@@ -6,13 +6,15 @@ One STEP = one pass of the hot path (frame scan + length-CRC check, Example inde
 cast + per-band normalise + label one-hot) over one batch = 24 shards x 250 records (the 6000-chip dataset
 of configs[0]), record = 262 391 B in, 786 432 + 2 621 440 B of float32 out.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = records/s with the shards already resident in HBM;
 `e2e` = the same through the public API starting from pinned HOST buffers (H2D of every shard and D2H of
 the per-record tables/status inside the timed region); `roofline` = algorithmic bytes of the dominant
 kernel / its CUDA-event time vs the measured HBM copy bandwidth; `cpu_baseline` = the oracle restatement
 of the reference's CPU path on a bounded sample.  --impl reference times only that CPU path.
+--dump-outputs DIR writes a seeded sample of what the last timed step computed (see dump_outputs); the inputs are
+generated from fixed seeds, so two builds given the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -157,6 +159,7 @@ def run_ours(args, rank, world):
 
         def consume(img, tgt, status, table):
             bad.add_((table.hdr_dev.index_select(0, idx014) - want).abs().sum())
+            return img, tgt, status, table                      # kept in CapturedPass.results (for --dump-outputs)
         return ops.CapturedPass(pipe, source, consume), bad
 
     pass_res, bad_res = make_pass(shards)
@@ -231,6 +234,8 @@ def run_ours(args, rank, world):
     ms, bad = timed(step_resident, args.steps, args.warmup)
     clocks = sampler.stop()
     assert int(bad.cpu()) == 0, "parse status != 0"
+    if args.dump_outputs and rank == 0:                         # before the e2e pass reuses the pipeline's buffers
+        dump_outputs(args.dump_outputs, pass_res.results[-pipe.depth:], idx014)
     launches = pass_res.launches_per_replay * args.steps        # our kernels inside the timed region (graph nodes)
     step_kernel_events()                                    # warm-up of the un-pipelined order
     del kern_events[:]
@@ -308,6 +313,30 @@ def run_ours(args, rank, world):
         dist.destroy_process_group()
     if rank == 0:
         print(json.dumps(line))
+
+
+DUMP_SEED = 2002
+DUMP_SAMPLES = 1 << 20                  # per shard and output array: 2 x 3 x 4 MiB = 24 MiB written in all
+
+
+def dump_outputs(out_dir, results, hdr_fields):
+    """Write what the last timed step handed its consumer, so that two builds can be compared output for output.
+
+    A shard's output buffers are recycled `depth` shards later, so after the step the results of the last `depth` shards
+    are the ones still on the device.  Their normalised images and one-hot labels (0.85 GB per shard) are sampled at
+    DUMP_SAMPLES positions drawn once from DUMP_SEED; the per-record status and the table header (records, scan status,
+    records failing the data CRC) are written whole."""
+    import torch
+    rng = np.random.default_rng(DUMP_SEED)
+    dev = results[0][0].device
+    picks = [torch.from_numpy(np.sort(rng.choice(results[0][i].numel(), DUMP_SAMPLES, replace=False))).to(dev) for i in (0, 1)]
+    arrays = {"image_sample": torch.stack([r[0].reshape(-1)[picks[0]] for r in results]),
+              "onehot_sample": torch.stack([r[1].reshape(-1)[picks[1]] for r in results]),
+              "record_status": torch.stack([r[2] for r in results]).to(torch.float32),
+              "shard_header": torch.stack([r[3].hdr_dev.index_select(0, hdr_fields) for r in results]).to(torch.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def _mosaic_traffic(chips_per_s, peak):
@@ -712,7 +741,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the secondary per-config kernel rates (N=1 only)")
     ap.add_argument("--traffic", type=float, default=None, help="dram bytes per launch from an ncu --set full capture")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of the last step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
