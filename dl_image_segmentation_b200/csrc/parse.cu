@@ -131,6 +131,17 @@ struct RecCache {
     uint64_t img_off, img_len, tgt_off, tgt_len;
 };
 
+// NORM_ONEHOT template: both payloads are BytesList, the record has the sink's band count and each payload is exactly
+// as long as the record's own dimensions say.  Anything else is status 2 (the reference's decode_raw + reshape raises);
+// rec_lookup (whether the sinks run) and finalize_record (the status) both ask here, so they cannot disagree.
+__device__ __forceinline__ bool norm_template_ok(const b2_example_index* ix, int C) {
+    if (ix->img_kind != 1 || ix->tgt_kind != 1 || ix->channels != C) return false;
+    if (ix->height < 0 || ix->width < 0 || ix->tgt_height < 0 || ix->tgt_width < 0) return false;
+    const uint64_t hw = (uint64_t)ix->height * (uint64_t)ix->width;   // < 2^62; C <= 64 (check_sink)
+    const uint64_t thw = (uint64_t)ix->tgt_height * (uint64_t)ix->tgt_width;
+    return hw < (1ull << 48) && hw * (uint64_t)C == ix->img_len && thw == ix->tgt_len;
+}
+
 template <int kMode>
 __device__ __forceinline__ void rec_lookup(const ParseArgs& a, uint32_t w, RecCache& c) {
     uint32_t r;
@@ -156,7 +167,7 @@ __device__ __forceinline__ void rec_lookup(const ParseArgs& a, uint32_t w, RecCa
         if (kMode == B2_SINK_RAW) ok = ok && il <= a.sink.img_stride && tl <= a.sink.tgt_stride;
         if (kMode == B2_SINK_NORM_ONEHOT) {
             const uint64_t K = (uint64_t)a.sink.num_classes;
-            ok = ok && ix->img_kind == 1 && ix->tgt_kind == 1 && il * 4 <= a.sink.img_stride && tl * K * 4 <= a.sink.tgt_stride &&
+            ok = ok && norm_template_ok(ix, a.sink.channels) && il * 4 <= a.sink.img_stride && tl * K * 4 <= a.sink.tgt_stride &&
                  il < (1ull << 31) && tl * K < (1ull << 31);
         }
         if (ok) {
@@ -298,7 +309,7 @@ __device__ inline void finalize_record(const ParseArgs& a, const RecRef& j, uint
             if (ix->img_len > a.sink.img_stride || ix->tgt_len > a.sink.tgt_stride) st = 3;
         } else {
             const uint64_t K = (uint64_t)a.sink.num_classes;
-            if (ix->img_kind != 1 || ix->tgt_kind != 1) st = 2;
+            if (!norm_template_ok(ix, a.sink.channels)) st = 2;
             else if (ix->img_len * 4 > a.sink.img_stride || ix->tgt_len * K * 4 > a.sink.tgt_stride ||
                      ix->img_len >= (1ull << 31) || ix->tgt_len * K >= (1ull << 31)) st = 3;
         }
@@ -661,19 +672,35 @@ struct LaunchCfg {
 };
 LaunchCfg g_cfg[64];
 
-size_t dyn_bytes(int mode, int K) {
-    size_t d = (size_t)stages_for(mode) * kBufBytes;
-    if (mode == B2_SINK_NORM_ONEHOT && K <= kHotMaxK) d += (size_t)(kTileThreads / 32) * kHotBlocks * (kHotLabels * K + 4) * sizeof(float);
-    return d;
+constexpr size_t dyn_bytes(int mode, int K) {
+    return (size_t)stages_for(mode) * kBufBytes +
+           (mode == B2_SINK_NORM_ONEHOT && K <= kHotMaxK ? (size_t)(kTileThreads / 32) * kHotBlocks * (kHotLabels * K + 4) * sizeof(float) : 0);
+}
+// The one-hot blocks at K = kHotMaxK need 145 KiB; the kernel's static shared memory (~9 KiB, ptxas -v) comes on top, and
+// both must fit the 227 KiB a block may opt into on sm_100.
+constexpr size_t kNormDynMax = dyn_bytes(B2_SINK_NORM_ONEHOT, kHotMaxK);
+
+// Raise a kernel's dynamic shared-memory ceiling to dyn after checking that static + dyn fits the device's per-block limit.
+template <typename F>
+int set_dyn_smem(F* kernel, size_t dyn, int device) {
+    cudaFuncAttributes fa;
+    B2_CUDA(cudaFuncGetAttributes(&fa, kernel));
+    int optin = 0;
+    B2_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+    B2_REQUIRE(fa.sharedSizeBytes + dyn <= (size_t)optin, "fused parse: shared memory of the largest launch exceeds the per-block limit");
+    B2_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+    return 0;
 }
 
 int launch_fused(b2_ctx* ctx, const ParseArgs& pa, uint64_t max_tiles, cudaStream_t s) {
     LaunchCfg& cfg = g_cfg[ctx->device & 63];
     if (!cfg.ready) {
-        B2_CUDA(cudaFuncSetAttribute(fused_parse_kernel<B2_SINK_NONE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-        B2_CUDA(cudaFuncSetAttribute(fused_parse_kernel<B2_SINK_RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-        B2_CUDA(cudaFuncSetAttribute(fused_parse_kernel<B2_SINK_NORM_ONEHOT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-        B2_CUDA(cudaFuncSetAttribute(fused_parse_kernel<B2_SINK_NORM_ONEHOT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
+        // opt-in ceilings; NORM_ONEHOT: what its largest launch (K = kHotMaxK) asks for.  A ceiling only: occupancy
+        // follows each launch's actual request.
+        if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NONE>, 96 * 1024, ctx->device)) return e;
+        if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_RAW>, 96 * 1024, ctx->device)) return e;
+        if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NORM_ONEHOT>, kNormDynMax, ctx->device)) return e;
+        if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NORM_ONEHOT, true>, kNormDynMax, ctx->device)) return e;
         cfg.ready = true;
     }
     // persistent grid: as many CTAs as fit on the GPU at once (4 per SM), never more than there are chunks

@@ -380,7 +380,6 @@ def parse_shard(si: ShardIndex, mode, verify_crc=True, mean=None, std=None, num_
     elif mode == "norm_onehot":
         sink.mode = _lib.SINK_NORM_ONEHOT
         K = int(num_classes)
-        C = int(idx["channels"][0])
         il, tl = int(idx["img_len"].max()), int(idx["tgt_len"].max())
         if (il * 4) % 16 or (tl * K * 4) % 16:
             il, tl = _align16(il), _align16(tl)
@@ -389,8 +388,10 @@ def parse_shard(si: ShardIndex, mode, verify_crc=True, mean=None, std=None, num_
             torch.empty((count, tl * K), dtype=torch.float32, device=ctx.device))
         mean_d = to_device(np.asarray(mean, dtype=np.float32) if not isinstance(mean, torch.Tensor) else mean, ctx.device)
         std_d = to_device(np.asarray(std, dtype=np.float32) if not isinstance(std, torch.Tensor) else std, ctx.device)
-        if mean_d.numel() != C or std_d.numel() != C:
-            raise B2Error("parse_shard: mean/std must have %d entries" % C)
+        # the band count is the sink's, as in parse_table: a record with another band count gets status 2
+        C = int(mean_d.numel())
+        if std_d.numel() != C:
+            raise B2Error("parse_shard: mean/std must have one entry per band")
         sink.img_out, sink.img_stride = img_buf.data_ptr(), img_buf.stride(0) * 4
         sink.tgt_out, sink.tgt_stride = tgt_buf.data_ptr(), tgt_buf.stride(0) * 4
         sink.mean, sink.std, sink.channels, sink.num_classes = mean_d.data_ptr(), std_d.data_ptr(), C, K

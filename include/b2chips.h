@@ -148,7 +148,9 @@ typedef struct {
 } b2_parse_sink;
 
 /* One fused pass over the records: CRC verify + payload scatter/cast.  status_dev[i]: 0 ok, 1 data-CRC mismatch
- * (TF: DataLossError), 2 index status != 0, 3 payload larger than its output stride.  Uses the context workspace:
+ * (TF: DataLossError), 2 index status != 0, or in NORM_ONEHOT mode a record that does not fit the template (a payload
+ * that is not BytesList, image/channels != sink channels, image length != height*width*channels, target length !=
+ * target height*width), 3 payload larger than its output stride.  Uses the context workspace:
  * calls on one context must be stream-ordered (b2_tfrecord_parse_table has no such restriction). */
 int b2_tfrecord_parse(b2_ctx* ctx, const uint8_t* shard_dev, uint64_t shard_nbytes, const uint64_t* rec_offsets_dev,
                       const uint64_t* rec_lens_dev, const b2_example_index* index_dev, int n,

@@ -22,8 +22,9 @@ def one_hot(label, num_classes):
     label = np.asarray(label)
     if label.ndim and label.shape[-1] == 1 and label.ndim == 3:
         label = label[..., 0]
+    # value equality, no cast: a float label that is NaN, infinite, negative or not integral is no class
     k = np.arange(num_classes, dtype=np.int64)
-    return (label[..., None].astype(np.int64) == k).astype(np.float32)
+    return (label[..., None] == k).astype(np.float32)
 
 
 def band_stats(img, valid=None):
