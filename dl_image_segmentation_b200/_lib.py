@@ -12,7 +12,7 @@ LIB_PATH = os.environ.get("B2CHIPS_LIB") or os.path.join(_HERE, "libb2chips.so")
 
 # element type codes (b2chips.h)
 B2_U8, B2_U16, B2_I16, B2_U32, B2_I32, B2_F32, B2_F64, B2_I8 = range(8)
-SINK_NONE, SINK_RAW, SINK_NORM_ONEHOT = 0, 1, 2
+SINK_NONE, SINK_RAW, SINK_NORM_ONEHOT, SINK_NORM_ONEHOT_F32 = 0, 1, 2, 3
 
 
 class B2Error(RuntimeError):

@@ -110,4 +110,18 @@ __device__ __forceinline__ uint4 ld_nc(const uint4* p) {
     return r;
 }
 
+// The class of a label, or -1 for an all-zero one-hot row: the value must equal an integer k < K.  NaN, +-inf,
+// negative and non-integral labels have no class; -0.0 is class 0.  The standalone one-hot (normalise.cu) and the
+// fused parse (parse.cu) both ask here, so the two cannot diverge.
+template <typename L>
+__device__ __forceinline__ int label_class(L lab, int K);
+template <>
+__device__ __forceinline__ int label_class<uint8_t>(uint8_t lab, int K) { return (int)lab < K ? (int)lab : -1; }
+template <>
+__device__ __forceinline__ int label_class<float>(float lab, int K) {
+    if (!(lab >= 0.0f && lab < (float)K)) return -1;       // also rejects NaN
+    const int k = (int)lab;
+    return (float)k == lab ? k : -1;
+}
+
 }  // namespace b2

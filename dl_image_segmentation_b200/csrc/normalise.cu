@@ -169,16 +169,6 @@ normalise_u8_lut_kernel(const uint8_t* __restrict__ img, const float* __restrict
 // memory, sets one 1.0f per valid label, streams the block out with coalesced 16-byte stores and clears its ones again.
 // ~12 instructions per label instead of ~50 per float4: the per-float4 kernel is issue-bound at 60 % of HBM.
 constexpr int kHotBlockMaxK = 24;                     // 2 x 256 x K floats <= 48 KiB of dynamic shared memory
-template <typename L>
-__device__ __forceinline__ int label_class(L lab, int K);
-template <>
-__device__ __forceinline__ int label_class<uint8_t>(uint8_t lab, int K) { return (int)lab < K ? (int)lab : -1; }
-template <>
-__device__ __forceinline__ int label_class<float>(float lab, int K) {
-    if (!(lab >= 0.0f && lab < (float)K)) return -1;       // also rejects NaN
-    const int k = (int)lab;
-    return (float)k == lab ? k : -1;
-}
 
 template <typename L>
 __global__ void __launch_bounds__(256)

@@ -55,7 +55,11 @@ constexpr int kHotBlocks = B2_HOT_BLOCKS;            // blocks per warp: the bul
 // short of shared memory (the one-hot blocks), so two do; the CRC-only and raw-copy passes are bound by the CRC chain
 // and by how well the bulk loads hide behind it: four buffers (ncu: a third of their stall samples were consumers
 // waiting for a tile with two).
-__host__ __device__ constexpr int stages_for(int mode) { return mode == B2_SINK_NORM_ONEHOT ? B2_STAGES : 4; }
+// The two normalise + one-hot modes (uint8 BytesList and float32 FloatList payloads) share every resource decision.
+__host__ __device__ constexpr bool is_norm(int mode) { return mode == B2_SINK_NORM_ONEHOT || mode == B2_SINK_NORM_ONEHOT_F32; }
+// bytes per payload element: 1 for BytesList, 4 for packed FloatList
+__host__ __device__ constexpr uint32_t elem_bytes(int mode) { return mode == B2_SINK_NORM_ONEHOT_F32 ? 4u : 1u; }
+__host__ __device__ constexpr int stages_for(int mode) { return is_norm(mode) ? B2_STAGES : 4; }
 constexpr int kMaxStages = 4;
 constexpr int kConsumerWarps = kTileThreads / 32;
 constexpr int kCtaThreads = kTileThreads + 32;   // 8 consumer warps + 1 producer warp
@@ -131,15 +135,26 @@ struct RecCache {
     uint64_t img_off, img_len, tgt_off, tgt_len;
 };
 
-// NORM_ONEHOT template: both payloads are BytesList, the record has the sink's band count and each payload is exactly
-// as long as the record's own dimensions say.  Anything else is status 2 (the reference's decode_raw + reshape raises);
-// rec_lookup (whether the sinks run) and finalize_record (the status) both ask here, so they cannot disagree.
+// Normalise + one-hot template: both payloads are BytesList (NORM_ONEHOT) or both packed FloatList (NORM_ONEHOT_F32),
+// the record has the sink's band count and each payload is exactly as long as the record's own dimensions say.
+// Anything else is status 2 (the reference's decode_raw / parse + reshape raises); rec_lookup (whether the sinks run)
+// and finalize_record (the status) both ask here, so they cannot disagree.
+template <int kMode>
 __device__ __forceinline__ bool norm_template_ok(const b2_example_index* ix, int C) {
-    if (ix->img_kind != 1 || ix->tgt_kind != 1 || ix->channels != C) return false;
+    constexpr int kKind = kMode == B2_SINK_NORM_ONEHOT_F32 ? 2 : 1;
+    constexpr uint64_t kEB = elem_bytes(kMode);
+    if (ix->img_kind != kKind || ix->tgt_kind != kKind || ix->channels != C) return false;
     if (ix->height < 0 || ix->width < 0 || ix->tgt_height < 0 || ix->tgt_width < 0) return false;
     const uint64_t hw = (uint64_t)ix->height * (uint64_t)ix->width;   // < 2^62; C <= 64 (check_sink)
     const uint64_t thw = (uint64_t)ix->tgt_height * (uint64_t)ix->tgt_width;
-    return hw < (1ull << 48) && hw * (uint64_t)C == ix->img_len && thw == ix->tgt_len;
+    return hw < (1ull << 48) && hw * (uint64_t)C * kEB == ix->img_len && thw * kEB == ix->tgt_len;
+}
+
+// NORM_ONEHOT_F32 output fit: each payload's floats fit its row and there are fewer than 2^31 image elements and one-hot
+// floats (the sink indexes elements with 32 bits).
+__device__ __forceinline__ bool f32_rows_fit(const b2_example_index* ix, const b2_parse_sink& sink) {
+    const uint64_t ie = ix->img_len >> 2, te = ix->tgt_len >> 2, K = (uint64_t)sink.num_classes;
+    return ie * 4 <= sink.img_stride && te * K * 4 <= sink.tgt_stride && ie < (1ull << 31) && te * K < (1ull << 31);
 }
 
 template <int kMode>
@@ -167,9 +182,10 @@ __device__ __forceinline__ void rec_lookup(const ParseArgs& a, uint32_t w, RecCa
         if (kMode == B2_SINK_RAW) ok = ok && il <= a.sink.img_stride && tl <= a.sink.tgt_stride;
         if (kMode == B2_SINK_NORM_ONEHOT) {
             const uint64_t K = (uint64_t)a.sink.num_classes;
-            ok = ok && norm_template_ok(ix, a.sink.channels) && il * 4 <= a.sink.img_stride && tl * K * 4 <= a.sink.tgt_stride &&
+            ok = ok && norm_template_ok<kMode>(ix, a.sink.channels) && il * 4 <= a.sink.img_stride && tl * K * 4 <= a.sink.tgt_stride &&
                  il < (1ull << 31) && tl * K < (1ull << 31);
         }
+        if (kMode == B2_SINK_NORM_ONEHOT_F32) ok = ok && norm_template_ok<kMode>(ix, a.sink.channels) && f32_rows_fit(ix, a.sink);
         if (ok) {
             c.flags = 2;
             c.img_off = ix->img_off;
@@ -266,11 +282,17 @@ __device__ __forceinline__ float norm_fast(float d, float sd, float rc) {
     return __fmaf_rn(rem, rc, q);
 }
 
+// FloatList label l's class (-1: all-zero row), from payload bytes [4l, 4l+4) at buffer offset base
+__device__ __forceinline__ int f32_label(const uint32_t* buf32, uint32_t base, uint32_t l, int K) {
+    return label_class<float>(__uint_as_float(smem_u32_unaligned(buf32, base + 4 * l)), K);
+}
+
 struct RecRef {   // what finalize_record needs to know about the record
     uint32_t r, nt;
     uint64_t d0, d1;
 };
 
+template <int kMode>
 __device__ inline void finalize_record(const ParseArgs& a, const RecRef& j, uint32_t acc) {
     const uint32_t r = j.r;
     const uint64_t d0 = j.d0, len = j.d1 - j.d0;
@@ -307,9 +329,12 @@ __device__ inline void finalize_record(const ParseArgs& a, const RecRef& j, uint
         if (ix->status != 0) st = 2;
         else if (a.sink.mode == B2_SINK_RAW) {
             if (ix->img_len > a.sink.img_stride || ix->tgt_len > a.sink.tgt_stride) st = 3;
+        } else if (kMode == B2_SINK_NORM_ONEHOT_F32) {
+            if (!norm_template_ok<kMode>(ix, a.sink.channels)) st = 2;
+            else if (!f32_rows_fit(ix, a.sink)) st = 3;
         } else {
             const uint64_t K = (uint64_t)a.sink.num_classes;
-            if (!norm_template_ok(ix, a.sink.channels)) st = 2;
+            if (!norm_template_ok<B2_SINK_NORM_ONEHOT>(ix, a.sink.channels)) st = 2;
             else if (ix->img_len * 4 > a.sink.img_stride || ix->tgt_len * K * 4 > a.sink.tgt_stride ||
                      ix->img_len >= (1ull << 31) || ix->tgt_len * K >= (1ull << 31)) st = 3;
         }
@@ -337,6 +362,7 @@ struct RunAcc {          // shared-memory meeting point of the eight consumer wa
 // merges { CRC, tiles } into the record's 64-bit accumulator with an atomic XOR and an atomic add on the same address
 // (applied in program order, so no fences are needed), finalising the record when its tile count is complete.  The other warps are already working
 // on the next tile.
+template <int kMode>
 __device__ __forceinline__ void run_flush(const ParseArgs& a, Run& run, uint32_t& s, uint32_t& run_seq, bool want_crc,
                                           RunAcc* racc) {
     const int tid = threadIdx.x, lane = tid & 31;
@@ -363,7 +389,7 @@ __device__ __forceinline__ void run_flush(const ParseArgs& a, Run& run, uint32_t
             if ((uint32_t)(upd >> 32) == run.nt) {
                 *acc = 0ull;               // re-arm for the next launch; nobody else touches a finished record
                 RecRef rr{run.r, run.nt, run.d0, run.d1};
-                finalize_record(a, rr, (uint32_t)upd);
+                finalize_record<kMode>(a, rr, (uint32_t)upd);
             }
         }
     }
@@ -393,7 +419,7 @@ __device__ __forceinline__ void run_flush(const ParseArgs& a, Run& run, uint32_t
 // CONSUMERS (CRC, payload sinks).  They meet only through mbarriers: full[s] flips when tile s has landed, empty[s]
 // when all eight consumer warps are done with it — there is no __syncthreads in the steady state.
 template <int kMode, bool kProf = false>
-__global__ void __launch_bounds__(kCtaThreads, kMode == B2_SINK_NORM_ONEHOT ? 3 : 5)
+__global__ void __launch_bounds__(kCtaThreads, is_norm(kMode) ? 3 : 5)
 fused_parse_kernel(const ParseArgs a) {
     constexpr int kStages = stages_for(kMode);
     static_assert(kStages <= kMaxStages && kRunSlots > kStages, "ring sizes");
@@ -413,7 +439,7 @@ fused_parse_kernel(const ParseArgs a) {
     float* hot_all = reinterpret_cast<float*>(dyn + kStages * kBufBytes);
 
     if (want_crc) load_crc_tables(&cs, a.tab);
-    if (kMode == B2_SINK_NORM_ONEHOT) {
+    if (is_norm(kMode)) {
         if (tid == 0) s_exact_div = 0;
         for (int c = tid; c < C; c += kCtaThreads) {
             s_mean[c] = a.sink.mean[c];
@@ -432,7 +458,7 @@ fused_parse_kernel(const ParseArgs a) {
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
-    if (kMode == B2_SINK_NORM_ONEHOT) {
+    if (kMode == B2_SINK_NORM_ONEHOT) {   // NORM_ONEHOT_F32 always divides: float inputs have no finite set to check
         int bad = 0;
         for (int i = tid; i < C * 256; i += kCtaThreads) {
             const int c = i >> 8;
@@ -481,7 +507,7 @@ fused_parse_kernel(const ParseArgs a) {
     // image loop stride: the largest S <= 256 with 4 S a multiple of C, so that a thread's four bytes always fall on
     // the same four bands and their constants stay in registers
     uint32_t img_S = kTileThreads;
-    if (kMode == B2_SINK_NORM_ONEHOT) {
+    if (is_norm(kMode)) {
         const uint32_t m = (C % 4 == 0) ? C / 4 : ((C % 2 == 0) ? C / 2 : C);
         img_S = kTileThreads - (kTileThreads % m);
     }
@@ -503,7 +529,7 @@ fused_parse_kernel(const ParseArgs a) {
         const TileJob& j = job[slot];
         const uint32_t flags = j.flags;
         const bool valid = (flags & 1) != 0;
-        if (run.open && (!valid || j.r != run.r || j.tile != run.last_tile + 1)) run_flush(a, run, s, run_seq, want_crc, racc);
+        if (run.open && (!valid || j.r != run.r || j.tile != run.last_tile + 1)) run_flush<kMode>(a, run, s, run_seq, want_crc, racc);
         PROF_MARK(5);
         if (flags & 4) break;
         if (valid) {
@@ -530,17 +556,22 @@ fused_parse_kernel(const ParseArgs a) {
                 if (a.sink.tgt_out)
                     sink_raw(buf32, buf8, ts, te, j.tgt_off, j.tgt_len, static_cast<uint8_t*>(a.sink.tgt_out) + (uint64_t)(j.r & a.row_mask) * a.sink.tgt_stride);
             }
-            if (kMode == B2_SINK_NORM_ONEHOT && (flags & 2)) {
-                // ---- uint8 image -> (x-mean)/std float32
+            if (is_norm(kMode) && (flags & 2)) {
+                // payload elements are kEB bytes: uint8 (NORM_ONEHOT) or little-endian float32 (NORM_ONEHOT_F32)
+                constexpr uint32_t kEB = elem_bytes(kMode);
+                // ---- image -> (x-mean)/std float32
                 const uint64_t ipo = j.img_off, ipl64 = j.img_len;
                 if (a.sink.img_out && ipl64 && ipo < te && ipo + ipl64 > ts && (uint32_t)tid < img_S) {
                     float* dst = reinterpret_cast<float*>(static_cast<uint8_t*>(a.sink.img_out) + (uint64_t)(j.r & a.row_mask) * a.sink.img_stride);
                     const uint64_t po = ipo;
-                    const uint32_t pl = (uint32_t)ipl64;
-                    const uint64_t lo = po > ts ? po : ts, hi = (po + pl < te) ? po + pl : te;
-                    // float4 group g = image bytes [4g, 4g+4); owned by the tile that holds its first byte
-                    const uint32_t g_lo = (uint32_t)((lo - po + 3) >> 2), g_hi = (uint32_t)((hi - po + 3) >> 2), full4 = pl >> 2;
-                    const uint32_t base = (uint32_t)(po - ts);  // wraps when po < ts; base + 4g is back in [0, kTile)
+                    const uint32_t pl = (uint32_t)(ipl64 / kEB);   // elements
+                    const uint64_t lo = po > ts ? po : ts, hi = (po + (uint64_t)pl * kEB < te) ? po + (uint64_t)pl * kEB : te;
+                    // float4 group g = image elements [4g, 4g+4) = payload bytes [4 kEB g, 4 kEB (g+1)); owned by the tile
+                    // that holds its first byte, its last bytes may sit in the halo
+                    const uint32_t g_lo = (uint32_t)((lo - po + 4 * kEB - 1) / (4 * kEB)), g_hi = (uint32_t)((hi - po + 4 * kEB - 1) / (4 * kEB)),
+                                   full4 = pl >> 2;
+                    // wraps when po < ts; base + 4 kEB g is back in [0, kTile) (mod 2^32)
+                    const uint32_t base = (uint32_t)(po - ts);
                     uint32_t g = g_lo + tid;
                     float mu[4], sd[4], rc[4];
                     {
@@ -554,18 +585,27 @@ fused_parse_kernel(const ParseArgs a) {
                         }
                     }
                     for (; g < g_hi; g += img_S) {
-                        const uint32_t x = smem_u32_unaligned(buf32, base + 4 * g);
                         float f[4];
+                        if constexpr (kEB == 1) {
+                            const uint32_t x = smem_u32_unaligned(buf32, base + 4 * g);
 #pragma unroll
-                        for (int k = 0; k < 4; k++) {
-                            // byte k -> float, exactly: 0x4B000000 | v is 2^23 + v
-                            const float v = __uint_as_float(__byte_perm(x, 0x4B000000u, 0x7540 + k)) - 8388608.0f;
-                            const float d = __fsub_rn(v, mu[k]);
-                            f[k] = exact_div ? __fdiv_rn(d, sd[k]) : norm_fast(d, sd[k], rc[k]);
+                            for (int k = 0; k < 4; k++) {
+                                // byte k -> float, exactly: 0x4B000000 | v is 2^23 + v
+                                const float v = __uint_as_float(__byte_perm(x, 0x4B000000u, 0x7540 + k)) - 8388608.0f;
+                                const float d = __fsub_rn(v, mu[k]);
+                                f[k] = exact_div ? __fdiv_rn(d, sd[k]) : norm_fast(d, sd[k], rc[k]);
+                            }
+                        } else {
+                            // FloatList payloads start at any byte residue: four funnel-shifted words
+#pragma unroll
+                            for (int k = 0; k < 4; k++) {
+                                const float v = __uint_as_float(smem_u32_unaligned(buf32, base + 16 * g + 4 * k));
+                                f[k] = __fdiv_rn(__fsub_rn(v, mu[k]), sd[k]);
+                            }
                         }
                         if (g < full4) {
                             st_cs(reinterpret_cast<float4*>(dst) + g, make_float4(f[0], f[1], f[2], f[3]));
-                        } else {   // the payload's last 1..3 bytes
+                        } else {   // the payload's last 1..3 elements
                             if (4 * g + 0 < pl) dst[4 * g + 0] = f[0];
                             if (4 * g + 1 < pl) dst[4 * g + 1] = f[1];
                             if (4 * g + 2 < pl) dst[4 * g + 2] = f[2];
@@ -573,13 +613,13 @@ fused_parse_kernel(const ParseArgs a) {
                     }
                 }
                 PROF_MARK(2);
-                // ---- uint8 target -> one-hot float32
+                // ---- target -> one-hot float32
                 const uint64_t tpo = j.tgt_off, tpl64 = j.tgt_len;
                 if (a.sink.tgt_out && tpl64 && tpo < te && tpo + tpl64 > ts) {
                     float* dst = reinterpret_cast<float*>(static_cast<uint8_t*>(a.sink.tgt_out) + (uint64_t)(j.r & a.row_mask) * a.sink.tgt_stride);
                     const uint64_t po = tpo;
-                    const uint32_t pl = (uint32_t)tpl64;
-                    const uint64_t lo = po > ts ? po : ts, hi = (po + pl < te) ? po + pl : te;
+                    const uint32_t pl = (uint32_t)(tpl64 / kEB);   // labels
+                    const uint64_t lo = po > ts ? po : ts, hi = (po + (uint64_t)pl * kEB < te) ? po + (uint64_t)pl * kEB : te;
                     const uint32_t base = (uint32_t)(po - ts);
                     if (use_hot) {
                         // Each warp owns blocks of kHotLabels*K floats in shared memory — zero except ONE 1.0f per label,
@@ -587,7 +627,7 @@ fused_parse_kernel(const ParseArgs a) {
                         // bulk store; out-of-range labels write a dummy float past the block, so nothing is predicated.
                         // Work unit = 4 labels (4K floats: a whole number of 16-byte groups, 16-byte aligned in the
                         // output); a unit belongs to the tile holding its first label, later labels may sit in the halo.
-                        const uint32_t j_lo = (uint32_t)((lo - po + 3) >> 2), j_hi = (uint32_t)((hi - po + 3) >> 2);
+                        const uint32_t j_lo = (uint32_t)((lo - po + 4 * kEB - 1) / (4 * kEB)), j_hi = (uint32_t)((hi - po + 4 * kEB - 1) / (4 * kEB));
                         const uint32_t L_beg = 4 * j_lo, L_end = (4 * j_hi < pl) ? 4 * j_hi : pl;
                         for (uint32_t L0 = L_beg + warp * kHotLabels; L0 < L_end; L0 += kConsumerWarps * kHotLabels) {
                             const uint32_t hb = kHotBlocks > 1 ? (hot_it & 1) : 0;
@@ -600,13 +640,24 @@ fused_parse_kernel(const ParseArgs a) {
                             constexpr uint32_t kPerLane = kHotLabels / 32;
                             const uint32_t l0 = L0 + kPerLane * lane;
                             uint32_t slot0 = hot_dummy, slot1 = hot_dummy;
-                            if (l0 < L_end) {
-                                const uint32_t lab = buf8[base + l0];
-                                if (lab < (uint32_t)K) slot0 = (kPerLane * lane) * K + lab;
-                            }
-                            if (kPerLane > 1 && l0 + 1 < L_end) {
-                                const uint32_t lab = buf8[base + l0 + 1];
-                                if (lab < (uint32_t)K) slot1 = (kPerLane * lane + 1) * K + lab;
+                            if constexpr (kEB == 1) {
+                                if (l0 < L_end) {
+                                    const uint32_t lab = buf8[base + l0];
+                                    if (lab < (uint32_t)K) slot0 = (kPerLane * lane) * K + lab;
+                                }
+                                if (kPerLane > 1 && l0 + 1 < L_end) {
+                                    const uint32_t lab = buf8[base + l0 + 1];
+                                    if (lab < (uint32_t)K) slot1 = (kPerLane * lane + 1) * K + lab;
+                                }
+                            } else {
+                                if (l0 < L_end) {
+                                    const int k = f32_label(buf32, base, l0, K);
+                                    if (k >= 0) slot0 = (kPerLane * lane) * K + k;
+                                }
+                                if (kPerLane > 1 && l0 + 1 < L_end) {
+                                    const int k = f32_label(buf32, base, l0 + 1, K);
+                                    if (k >= 0) slot1 = (kPerLane * lane + 1) * K + k;
+                                }
                             }
                             hot[slot0] = 1.0f;
                             hot[slot1] = 1.0f;
@@ -624,7 +675,8 @@ fused_parse_kernel(const ParseArgs a) {
                     } else {
                         // generic path (K > 32): float4 group g holds one-hot floats [4g, 4g+4), owned by the tile of label 4g/K
                         const uint32_t nfl = pl * (uint32_t)K;
-                        const uint32_t g_lo = (uint32_t)(((lo - po) * K + 3) >> 2), g_hi = (uint32_t)(((hi - po) * K + 3) >> 2), full4 = nfl >> 2;
+                        const uint32_t g_lo = (uint32_t)(((lo - po + kEB - 1) / kEB * K + 3) >> 2),
+                                       g_hi = (uint32_t)(((hi - po + kEB - 1) / kEB * K + 3) >> 2), full4 = nfl >> 2;
                         for (uint32_t g = g_lo + tid; g < g_hi; g += kTileThreads) {
                             const uint32_t f0 = 4 * g;
                             uint32_t l = f0 / (uint32_t)K;
@@ -632,7 +684,9 @@ fused_parse_kernel(const ParseArgs a) {
                             float f[4];
 #pragma unroll
                             for (int k = 0; k < 4; k++) {
-                                const uint32_t lab = (l < pl) ? buf8[base + l] : 0xFFFFFFFFu;
+                                uint32_t lab;
+                                if constexpr (kEB == 1) lab = (l < pl) ? buf8[base + l] : 0xFFFFFFFFu;
+                                else lab = (l < pl) ? (uint32_t)f32_label(buf32, base, l, K) : 0xFFFFFFFFu;
                                 f[k] = (lab == cc) ? 1.0f : 0.0f;
                                 if (++cc == (uint32_t)K) {
                                     cc = 0;
@@ -656,7 +710,7 @@ fused_parse_kernel(const ParseArgs a) {
         if (lane == 0) mbar_arrive(&empty[slot]);   // this warp is done with the buffer and its job
         PROF_MARK(4);
     }
-    if (kMode == B2_SINK_NORM_ONEHOT && lane == 0) bulk_wait_read<0>();   // shared memory must outlive the bulk stores
+    if (is_norm(kMode) && lane == 0) bulk_wait_read<0>();   // shared memory must outlive the bulk stores
     PROF_END();
 }
 
@@ -674,7 +728,7 @@ LaunchCfg g_cfg[64];
 
 constexpr size_t dyn_bytes(int mode, int K) {
     return (size_t)stages_for(mode) * kBufBytes +
-           (mode == B2_SINK_NORM_ONEHOT && K <= kHotMaxK ? (size_t)(kTileThreads / 32) * kHotBlocks * (kHotLabels * K + 4) * sizeof(float) : 0);
+           (is_norm(mode) && K <= kHotMaxK ? (size_t)(kTileThreads / 32) * kHotBlocks * (kHotLabels * K + 4) * sizeof(float) : 0);
 }
 // The one-hot blocks at K = kHotMaxK need 145 KiB; the kernel's static shared memory (~9 KiB, ptxas -v) comes on top, and
 // both must fit the 227 KiB a block may opt into on sm_100.
@@ -695,22 +749,24 @@ int set_dyn_smem(F* kernel, size_t dyn, int device) {
 int launch_fused(b2_ctx* ctx, const ParseArgs& pa, uint64_t max_tiles, cudaStream_t s) {
     LaunchCfg& cfg = g_cfg[ctx->device & 63];
     if (!cfg.ready) {
-        // opt-in ceilings; NORM_ONEHOT: what its largest launch (K = kHotMaxK) asks for.  A ceiling only: occupancy
-        // follows each launch's actual request.
+        // opt-in ceilings; NORM_ONEHOT and NORM_ONEHOT_F32: what their largest launch (K = kHotMaxK) asks for.  A
+        // ceiling only: occupancy follows each launch's actual request.
         if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NONE>, 96 * 1024, ctx->device)) return e;
         if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_RAW>, 96 * 1024, ctx->device)) return e;
         if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NORM_ONEHOT>, kNormDynMax, ctx->device)) return e;
         if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NORM_ONEHOT, true>, kNormDynMax, ctx->device)) return e;
+        if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NORM_ONEHOT_F32>, kNormDynMax, ctx->device)) return e;
         cfg.ready = true;
     }
     // persistent grid: as many CTAs as fit on the GPU at once (4 per SM), never more than there are chunks
     const uint64_t chunks = (max_tiles + pa.q - 1) / pa.q;
-    const uint64_t resident = (uint64_t)ctx->sm_count * (pa.sink.mode == B2_SINK_NORM_ONEHOT ? 3 : 5);
+    const uint64_t resident = (uint64_t)ctx->sm_count * (is_norm(pa.sink.mode) ? 3 : 5);
     const unsigned grid = (unsigned)(chunks < resident ? chunks : resident);
     const size_t dyn = dyn_bytes(pa.sink.mode, pa.sink.num_classes);
     switch (pa.sink.mode) {
         case B2_SINK_NONE: fused_parse_kernel<B2_SINK_NONE><<<grid, kCtaThreads, dyn, s>>>(pa); break;
         case B2_SINK_RAW: fused_parse_kernel<B2_SINK_RAW><<<grid, kCtaThreads, dyn, s>>>(pa); break;
+        case B2_SINK_NORM_ONEHOT_F32: fused_parse_kernel<B2_SINK_NORM_ONEHOT_F32><<<grid, kCtaThreads, dyn, s>>>(pa); break;
         default:
             if (pa.prof) fused_parse_kernel<B2_SINK_NORM_ONEHOT, true><<<grid, kCtaThreads, dyn, s>>>(pa);
             else fused_parse_kernel<B2_SINK_NORM_ONEHOT><<<grid, kCtaThreads, dyn, s>>>(pa);
@@ -722,12 +778,13 @@ int launch_fused(b2_ctx* ctx, const ParseArgs& pa, uint64_t max_tiles, cudaStrea
 }
 
 int check_sink(const b2_parse_sink* sink, const char* who) {
-    if (sink->mode == B2_SINK_NORM_ONEHOT) {
+    if (is_norm(sink->mode)) {
+        const std::string m = sink->mode == B2_SINK_NORM_ONEHOT ? ": NORM_ONEHOT" : ": NORM_ONEHOT_F32";
         B2_REQUIRE(sink->mean && sink->std && sink->channels >= 1 && sink->channels <= 64 && sink->num_classes >= 1,
-                   std::string(who) + ": NORM_ONEHOT needs mean/std, 1..64 channels and num_classes >= 1");
+                   std::string(who) + m + " needs mean/std, 1..64 channels and num_classes >= 1");
         B2_REQUIRE((reinterpret_cast<uintptr_t>(sink->img_out) & 15) == 0 && (sink->img_stride & 15) == 0 &&
                    (reinterpret_cast<uintptr_t>(sink->tgt_out) & 15) == 0 && (sink->tgt_stride & 15) == 0,
-                   std::string(who) + ": NORM_ONEHOT outputs and strides must be 16-byte aligned");
+                   std::string(who) + m + " outputs and strides must be 16-byte aligned");
     } else {
         B2_REQUIRE(sink->mode == B2_SINK_NONE || sink->mode == B2_SINK_RAW, std::string(who) + ": unknown sink mode");
     }
@@ -745,7 +802,9 @@ uint32_t dev_row_mask() {
 }
 
 // Tiles per scheduler chunk (= the longest run whose per-thread CRC state is carried): 2 keeps the output streams of the
-// normalise + one-hot pass balanced; the CRC-only and raw passes amortise the per-run alignment multiply over 8.
+// uint8 normalise + one-hot pass balanced; the CRC-only, raw and float32 normalise + one-hot passes amortise the per-run
+// alignment multiply over 8 (NORM_ONEHOT_F32 reads 4 bytes per output float and is CRC-bound: cfg3 records with CRC
+// take 6.2 us at q = 2, 5.5 us at 4, 5.4 us at 8 on a B200 at 1000 W).
 uint32_t tiles_per_cta(int mode) {
 #ifdef B2_DEV_KNOBS
     static int q = -1;

@@ -356,7 +356,9 @@ def parse_shard(si: ShardIndex, mode, verify_crc=True, mean=None, std=None, num_
     """Run the fused parse kernel over records [first, first+count).  Returns (img_buf, tgt_buf, status_dev).
 
     mode 'raw': img_buf (count, img_stride) uint8 holding each record's payload bytes as stored;
-    mode 'norm_onehot': img_buf (count, img_len) float32, tgt_buf (count, tgt_len*K) float32;
+    mode 'norm_onehot': uint8 BytesList records -> img_buf (count, img_len) float32, tgt_buf (count, tgt_len*K) float32;
+    mode 'norm_onehot_f32': packed float32 FloatList records (the higher-dtype array format) -> the same outputs, with
+    img_len / tgt_len counted in float elements (the index's byte lengths / 4);
     mode 'none': CRC verification only.
     """
     ctx = get_ctx(si.shard.device)
@@ -377,10 +379,12 @@ def parse_shard(si: ShardIndex, mode, verify_crc=True, mean=None, std=None, num_
             torch.empty((count, tstr), dtype=torch.uint8, device=ctx.device))
         sink.img_out, sink.img_stride = img_buf.data_ptr(), img_buf.stride(0)
         sink.tgt_out, sink.tgt_stride = tgt_buf.data_ptr(), tgt_buf.stride(0)
-    elif mode == "norm_onehot":
-        sink.mode = _lib.SINK_NORM_ONEHOT
+    elif mode in ("norm_onehot", "norm_onehot_f32"):
+        f32 = mode == "norm_onehot_f32"
+        sink.mode = _lib.SINK_NORM_ONEHOT_F32 if f32 else _lib.SINK_NORM_ONEHOT
         K = int(num_classes)
-        il, tl = int(idx["img_len"].max()), int(idx["tgt_len"].max())
+        esz = 4 if f32 else 1
+        il, tl = int(idx["img_len"].max()) // esz, int(idx["tgt_len"].max()) // esz
         if (il * 4) % 16 or (tl * K * 4) % 16:
             il, tl = _align16(il), _align16(tl)
         img_buf, tgt_buf = out if out is not None else (
@@ -483,8 +487,8 @@ def _make_sink(ctx, mode, verify_crc, mean, std, num_classes, channels, img_buf,
         sink.mode = _lib.SINK_RAW
         sink.img_out, sink.img_stride = img_buf.data_ptr(), img_buf.stride(0) * img_buf.element_size()
         sink.tgt_out, sink.tgt_stride = tgt_buf.data_ptr(), tgt_buf.stride(0) * tgt_buf.element_size()
-    elif mode == "norm_onehot":
-        sink.mode = _lib.SINK_NORM_ONEHOT
+    elif mode in ("norm_onehot", "norm_onehot_f32"):
+        sink.mode = _lib.SINK_NORM_ONEHOT_F32 if mode == "norm_onehot_f32" else _lib.SINK_NORM_ONEHOT
         sink.img_out, sink.img_stride = img_buf.data_ptr(), img_buf.stride(0) * 4
         sink.tgt_out, sink.tgt_stride = tgt_buf.data_ptr(), tgt_buf.stride(0) * 4
         sink.mean, sink.std = mean.data_ptr(), std.data_ptr()
@@ -501,7 +505,8 @@ def parse_table(st: ShardTable, mode, img_elems=0, tgt_elems=0, verify_crc=True,
 
     The record count lives on the device, so outputs are sized for st.max_records rows:
     mode 'raw': (max_records, img_elems) / (max_records, tgt_elems) uint8 rows of payload bytes as stored;
-    mode 'norm_onehot': (max_records, img_elems) float32 and (max_records, tgt_elems*K) float32;
+    mode 'norm_onehot' (uint8 BytesList records) and 'norm_onehot_f32' (packed float32 FloatList records):
+    (max_records, img_elems) float32 and (max_records, tgt_elems*K) float32, sizes in elements (H*W*C and H*W);
     mode 'none': CRC verification only.  A payload longer than its row gives status 3.
     Returns (img_buf, tgt_buf, status_dev[max_records]); rows / entries >= the record count are untouched.
     """
@@ -513,7 +518,7 @@ def parse_table(st: ShardTable, mode, img_elems=0, tgt_elems=0, verify_crc=True,
         img_buf, tgt_buf = out if out is not None else (
             torch.empty((cap, _align16(max(1, img_elems))), dtype=torch.uint8, device=ctx.device),
             torch.empty((cap, _align16(max(1, tgt_elems))), dtype=torch.uint8, device=ctx.device))
-    elif mode == "norm_onehot":
+    elif mode in ("norm_onehot", "norm_onehot_f32"):
         K = int(num_classes)
         mean = to_device(np.asarray(mean, dtype=np.float32) if not isinstance(mean, torch.Tensor) else mean, ctx.device)
         std = to_device(np.asarray(std, dtype=np.float32) if not isinstance(std, torch.Tensor) else std, ctx.device)

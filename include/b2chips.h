@@ -131,17 +131,21 @@ int b2_tfrecord_table_layout(uint64_t shard_nbytes, uint64_t max_records, uint64
 int b2_tfrecord_open(b2_ctx* ctx, const uint8_t* shard_dev, uint64_t shard_nbytes, uint64_t max_records,
                      uint8_t* table_dev, b2_stream stream);
 
-enum { B2_SINK_NONE = 0, B2_SINK_RAW = 1, B2_SINK_NORM_ONEHOT = 2 };
+enum { B2_SINK_NONE = 0, B2_SINK_RAW = 1, B2_SINK_NORM_ONEHOT = 2, B2_SINK_NORM_ONEHOT_F32 = 3 };
 typedef struct {
     int32_t mode;        /* B2_SINK_NONE: CRC only.  RAW: payload bytes copied as stored (uint8 arrays; packed
                             little-endian float32 == float arrays).  NORM_ONEHOT: uint8 image -> normalised float32,
-                            uint8 target -> one-hot float32 (K classes).                                      */
+                            uint8 target -> one-hot float32 (K classes).  NORM_ONEHOT_F32: the same outputs from
+                            packed float32 FloatList payloads (the higher-dtype array records): image ->
+                            (x - mean[c]) / std[c] with IEEE float32 division, target -> one-hot where a label
+                            equal to an integer k < K is class k (-0.0 is class 0; NaN, +-inf, negative,
+                            non-integral and >= K labels give an all-zero row).                              */
     int32_t verify_crc;  /* non-zero: compute each record's data CRC and compare with the stored masked CRC   */
     void* img_out;       /* record i lands at img_out + i*img_stride (bytes)                                  */
     uint64_t img_stride;
     void* tgt_out;
     uint64_t tgt_stride;
-    const float* mean;   /* (channels) device, NORM_ONEHOT only                                               */
+    const float* mean;   /* (channels) device, NORM_ONEHOT and NORM_ONEHOT_F32 only                           */
     const float* std;
     int32_t channels;
     int32_t num_classes;
@@ -150,7 +154,11 @@ typedef struct {
 /* One fused pass over the records: CRC verify + payload scatter/cast.  status_dev[i]: 0 ok, 1 data-CRC mismatch
  * (TF: DataLossError), 2 index status != 0, or in NORM_ONEHOT mode a record that does not fit the template (a payload
  * that is not BytesList, image/channels != sink channels, image length != height*width*channels, target length !=
- * target height*width), 3 payload larger than its output stride.  Uses the context workspace:
+ * target height*width), 3 payload larger than its output stride.  NORM_ONEHOT_F32 (as parse_higher_dtype_array_proto
+ * followed by normalise and one-hot): 2 also for a payload that is not packed FloatList (a BytesList record included),
+ * image/channels != sink channels, image length != 4*height*width*channels bytes, target length != 4*target
+ * height*width bytes or a negative dimension; 3 for a payload longer than its output row or of 2^31 elements or more
+ * (image elements, or target elements * K).  Unpacked FloatList is status 2 from the index.  Uses the context workspace:
  * calls on one context must be stream-ordered (b2_tfrecord_parse_table has no such restriction). */
 int b2_tfrecord_parse(b2_ctx* ctx, const uint8_t* shard_dev, uint64_t shard_nbytes, const uint64_t* rec_offsets_dev,
                       const uint64_t* rec_lens_dev, const b2_example_index* index_dev, int n,
