@@ -119,9 +119,9 @@ template <>
 __device__ __forceinline__ int label_class<uint8_t>(uint8_t lab, int K) { return (int)lab < K ? (int)lab : -1; }
 template <>
 __device__ __forceinline__ int label_class<float>(float lab, int K) {
-    if (!(lab >= 0.0f && lab < (float)K)) return -1;       // also rejects NaN
+    if (!(lab >= 0.0f && lab < 2147483648.0f)) return -1;  // also rejects NaN; below 2^31 the int conversion is exact
     const int k = (int)lab;
-    return (float)k == lab ? k : -1;
+    return (float)k == lab && k < K ? k : -1;             // k < K in integers: (float)K would round above 2^24
 }
 
 }  // namespace b2

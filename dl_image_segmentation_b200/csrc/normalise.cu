@@ -73,13 +73,6 @@ normalise_kernel(const T* __restrict__ img, const float* __restrict__ mean, cons
     }
 }
 
-template <typename L>
-__device__ __forceinline__ bool label_is(L lab, uint32_t k);
-template <>
-__device__ __forceinline__ bool label_is<uint8_t>(uint8_t lab, uint32_t k) { return (uint32_t)lab == k; }
-template <>
-__device__ __forceinline__ bool label_is<float>(float lab, uint32_t k) { return lab == (float)k; }
-
 // One thread per output float4 of the one-hot tensor: floats [4g, 4g+4) of the flattened (n_pixels*K) array.  The
 // (label, class) position of the first float advances by a constant per grid stride: no division in the loop.
 template <typename L>
@@ -98,14 +91,14 @@ onehot_kernel(const L* __restrict__ label, uint64_t n_pixels, int K, float* __re
         uint64_t l = l0;
         uint32_t c = c0;
         float f[4];
-        L lab = (l < n_pixels) ? __ldg(label + l) : (L)0;
+        int cls = (l < n_pixels) ? label_class<L>(__ldg(label + l), K) : -1;   // -1 equals no class index
 #pragma unroll
         for (int k = 0; k < 4; k++) {
-            f[k] = (l < n_pixels && label_is<L>(lab, c)) ? 1.0f : 0.0f;
+            f[k] = (cls == (int)c) ? 1.0f : 0.0f;
             if (++c == (uint32_t)K) {
                 c = 0;
                 l++;
-                if (k < 3) lab = (l < n_pixels) ? __ldg(label + l) : (L)0;
+                if (k < 3) cls = (l < n_pixels) ? label_class<L>(__ldg(label + l), K) : -1;
             }
         }
         if (f0 + 4 <= n_fl) {

@@ -28,8 +28,6 @@
 //   * when the run ends, one GF(2)[x] multiplication by x^(-128 i) aligns thread i's state with the tile end,
 //     the states XOR together, and one more multiplication by a tabulated power of x moves the partial to the
 //     end of the record.  The 0xFFFFFFFF init is XORed into the first four data bytes.
-#include <cstring>
-
 #include "tfrecord_common.cuh"
 
 #ifndef B2_WAIT_HINT_NS
@@ -135,26 +133,25 @@ struct RecCache {
     uint64_t img_off, img_len, tgt_off, tgt_len;
 };
 
-// Normalise + one-hot template: both payloads are BytesList (NORM_ONEHOT) or both packed FloatList (NORM_ONEHOT_F32),
-// the record has the sink's band count and each payload is exactly as long as the record's own dimensions say.
-// Anything else is status 2 (the reference's decode_raw / parse + reshape raises); rec_lookup (whether the sinks run)
-// and finalize_record (the status) both ask here, so they cannot disagree.
+// The sinks' whole verdict on a record, in one place so that rec_lookup (whether they run) and finalize_record (the
+// status) cannot disagree.  0: they run.  2: the index refused the record, or it does not fit the normalise + one-hot
+// template: both payloads BytesList (NORM_ONEHOT) or packed FloatList (NORM_ONEHOT_F32), the sink's band count, payloads
+// as long as the record's dimensions say (else the reference's decode_raw / reshape raises).  3: a payload does not fit
+// its output row, or has 2^31 elements or more (the sinks index elements with 32 bits).
 template <int kMode>
-__device__ __forceinline__ bool norm_template_ok(const b2_example_index* ix, int C) {
+__device__ __forceinline__ int32_t sink_status(const b2_example_index* ix, const b2_parse_sink& sink) {
+    if (ix->status != 0) return 2;
+    if (kMode == B2_SINK_RAW) return ix->img_len <= sink.img_stride && ix->tgt_len <= sink.tgt_stride ? 0 : 3;
     constexpr int kKind = kMode == B2_SINK_NORM_ONEHOT_F32 ? 2 : 1;
     constexpr uint64_t kEB = elem_bytes(kMode);
-    if (ix->img_kind != kKind || ix->tgt_kind != kKind || ix->channels != C) return false;
-    if (ix->height < 0 || ix->width < 0 || ix->tgt_height < 0 || ix->tgt_width < 0) return false;
+    const int C = sink.channels;
+    if (ix->img_kind != kKind || ix->tgt_kind != kKind || ix->channels != C) return 2;
+    if (ix->height < 0 || ix->width < 0 || ix->tgt_height < 0 || ix->tgt_width < 0) return 2;
     const uint64_t hw = (uint64_t)ix->height * (uint64_t)ix->width;   // < 2^62; C <= 64 (check_sink)
     const uint64_t thw = (uint64_t)ix->tgt_height * (uint64_t)ix->tgt_width;
-    return hw < (1ull << 48) && hw * (uint64_t)C * kEB == ix->img_len && thw * kEB == ix->tgt_len;
-}
-
-// NORM_ONEHOT_F32 output fit: each payload's floats fit its row and there are fewer than 2^31 image elements and one-hot
-// floats (the sink indexes elements with 32 bits).
-__device__ __forceinline__ bool f32_rows_fit(const b2_example_index* ix, const b2_parse_sink& sink) {
-    const uint64_t ie = ix->img_len >> 2, te = ix->tgt_len >> 2, K = (uint64_t)sink.num_classes;
-    return ie * 4 <= sink.img_stride && te * K * 4 <= sink.tgt_stride && ie < (1ull << 31) && te * K < (1ull << 31);
+    if (hw >= (1ull << 48) || hw * (uint64_t)C * kEB != ix->img_len || thw * kEB != ix->tgt_len) return 2;
+    const uint64_t ie = hw * (uint64_t)C, te = thw, K = (uint64_t)sink.num_classes;
+    return ie * 4 <= sink.img_stride && te * K * 4 <= sink.tgt_stride && ie < (1ull << 31) && te * K < (1ull << 31) ? 0 : 3;
 }
 
 template <int kMode>
@@ -177,21 +174,12 @@ __device__ __forceinline__ void rec_lookup(const ParseArgs& a, uint32_t w, RecCa
     c.img_off = c.img_len = c.tgt_off = c.tgt_len = 0;
     if (kMode != B2_SINK_NONE && a.index != nullptr) {
         const b2_example_index* ix = a.index + r;
-        bool ok = ix->status == 0;
-        const uint64_t il = ix->img_len, tl = ix->tgt_len;
-        if (kMode == B2_SINK_RAW) ok = ok && il <= a.sink.img_stride && tl <= a.sink.tgt_stride;
-        if (kMode == B2_SINK_NORM_ONEHOT) {
-            const uint64_t K = (uint64_t)a.sink.num_classes;
-            ok = ok && norm_template_ok<kMode>(ix, a.sink.channels) && il * 4 <= a.sink.img_stride && tl * K * 4 <= a.sink.tgt_stride &&
-                 il < (1ull << 31) && tl * K < (1ull << 31);
-        }
-        if (kMode == B2_SINK_NORM_ONEHOT_F32) ok = ok && norm_template_ok<kMode>(ix, a.sink.channels) && f32_rows_fit(ix, a.sink);
-        if (ok) {
+        if (sink_status<kMode>(ix, a.sink) == 0) {
             c.flags = 2;
             c.img_off = ix->img_off;
-            c.img_len = il;
+            c.img_len = ix->img_len;
             c.tgt_off = ix->tgt_off;
-            c.tgt_len = tl;
+            c.tgt_len = ix->tgt_len;
         }
     }
 }
@@ -244,10 +232,15 @@ __device__ __forceinline__ void make_job(const ParseArgs& a, uint32_t w, RecCach
     }
 }
 
+// whether tile [ts, te) holds any byte of payload [po, po + len) (absolute)
+__device__ __forceinline__ bool tile_holds(uint64_t ts, uint64_t te, uint64_t po, uint64_t len) {
+    return len != 0 && po < te && po + len > ts;
+}
+
 // raw byte copy of payload range [po, po+pl) (absolute) into dst, for the part owned by tile [ts, te)
 __device__ __forceinline__ void sink_raw(const uint32_t* buf32, const uint8_t* buf8, uint64_t ts, uint64_t te,
                                          uint64_t po, uint64_t pl, uint8_t* dst) {
-    if (pl == 0 || po >= te || po + pl <= ts) return;
+    if (!tile_holds(ts, te, po, pl)) return;
     const bool al = (reinterpret_cast<uintptr_t>(dst) & 15) == 0;
     const uint64_t lo = po > ts ? po : ts, hi = (po + pl < te) ? po + pl : te;  // absolute bytes in this tile
     if (al) {
@@ -282,9 +275,153 @@ __device__ __forceinline__ float norm_fast(float d, float sd, float rc) {
     return __fmaf_rn(rem, rc, q);
 }
 
-// FloatList label l's class (-1: all-zero row), from payload bytes [4l, 4l+4) at buffer offset base
-__device__ __forceinline__ int f32_label(const uint32_t* buf32, uint32_t base, uint32_t l, int K) {
-    return label_class<float>(__uint_as_float(smem_u32_unaligned(buf32, base + 4 * l)), K);
+// The sinks below write the part of payload [po, po + len) (absolute bytes; elements of kEB bytes: uint8 or little-endian
+// float32) that tile [ts, te) owns.  Callers check tile_holds before computing the output row (keeps registers down).
+// base = po - ts: the payload start in the tile buffer (wraps when po < ts; base + kEB * element is in [0, kTile) mod 2^32).
+
+// float4 group g of an output row of n floats (full4 = n / 4 whole groups): one streaming store, or the last 1..3 floats
+__device__ __forceinline__ void store_group(float* dst, uint32_t g, uint32_t full4, uint32_t n, const float (&f)[4]) {
+    if (g < full4) st_cs(reinterpret_cast<float4*>(dst) + g, make_float4(f[0], f[1], f[2], f[3]));
+    else for (uint32_t k = 0; k < 3; k++) if (4 * g + k < n) dst[4 * g + k] = f[k];
+}
+
+// label l's class (-1: all-zero row)
+template <uint32_t kEB>
+__device__ __forceinline__ int payload_class(const uint8_t* buf8, const uint32_t* buf32, uint32_t base, uint32_t l, int K) {
+    if constexpr (kEB == 1) return label_class<uint8_t>(buf8[base + l], K);
+    else return label_class<float>(__uint_as_float(smem_u32_unaligned(buf32, base + 4 * l)), K);
+}
+
+// image -> (x - mean) / std float32; thread tid < S takes float4 groups tid, tid + S, ... (S: img_S in the kernel)
+template <uint32_t kEB>
+__device__ __forceinline__ void sink_image(const uint32_t* buf32, uint64_t ts, uint64_t te, uint64_t po, uint64_t len,
+                                           float* dst, uint32_t S, const float* s_mean, const float* s_std,
+                                           const float* s_rcp, int C, bool exact_div) {
+    const uint32_t pl = (uint32_t)(len / kEB);   // elements
+    const uint64_t lo = po > ts ? po : ts, hi = (po + (uint64_t)pl * kEB < te) ? po + (uint64_t)pl * kEB : te;
+    // float4 group g = image elements [4g, 4g+4) = payload bytes [4 kEB g, 4 kEB (g+1)); owned by the tile that holds its
+    // first byte, its last bytes may sit in the halo
+    const uint32_t g_lo = (uint32_t)((lo - po + 4 * kEB - 1) / (4 * kEB)), g_hi = (uint32_t)((hi - po + 4 * kEB - 1) / (4 * kEB)),
+                   full4 = pl >> 2;
+    const uint32_t base = (uint32_t)(po - ts);
+    uint32_t g = g_lo + threadIdx.x;
+    float mu[4], sd[4], rc[4];
+    {
+        uint32_t ch = (4u * g) % (uint32_t)C;
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            mu[k] = s_mean[ch];
+            sd[k] = s_std[ch];
+            rc[k] = s_rcp[ch];
+            ch = (ch + 1 == (uint32_t)C) ? 0 : ch + 1;
+        }
+    }
+    for (; g < g_hi; g += S) {
+        float f[4];
+        if constexpr (kEB == 1) {
+            const uint32_t x = smem_u32_unaligned(buf32, base + 4 * g);
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                // byte k -> float, exactly: 0x4B000000 | v is 2^23 + v
+                const float v = __uint_as_float(__byte_perm(x, 0x4B000000u, 0x7540 + k)) - 8388608.0f;
+                const float d = __fsub_rn(v, mu[k]);
+                f[k] = exact_div ? __fdiv_rn(d, sd[k]) : norm_fast(d, sd[k], rc[k]);
+            }
+        } else {
+            // FloatList payloads start at any byte residue: four funnel-shifted words
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                const float v = __uint_as_float(smem_u32_unaligned(buf32, base + 16 * g + 4 * k));
+                f[k] = __fdiv_rn(__fsub_rn(v, mu[k]), sd[k]);
+            }
+        }
+        store_group(dst, g, full4, pl, f);
+    }
+}
+
+// A consumer warp's kHotBlocks one-hot blocks of kHotLabels*K floats + 4 (float kHotLabels*K is a dummy, never stored)
+struct HotBlocks {
+    float* blk;                     // this warp's first block
+    uint32_t a0, a1, b0, b1;        // the floats this lane set last time in block 0 / block 1
+    uint32_t it;                    // blocks filled so far
+};
+
+// label -> one-hot float32, K <= kHotMaxK.  A warp's blocks are zero but for ONE 1.0f per label (a label costs one 4-byte
+// shared-memory write) and go to HBM with one TMA bulk store each; labels without a class write the dummy, so nothing is
+// predicated.  Work unit = 4 labels (4K floats: whole 16-byte groups, 16-byte aligned in the output), owned by the tile
+// holding its first label; later labels may sit in the halo.
+template <uint32_t kEB>
+__device__ __forceinline__ void sink_onehot_smem(const uint8_t* buf8, const uint32_t* buf32, uint64_t ts, uint64_t te,
+                                                 uint64_t po, uint64_t len, float* dst, int K, HotBlocks& h) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t pl = (uint32_t)(len / kEB);   // labels
+    const uint64_t lo = po > ts ? po : ts, hi = (po + (uint64_t)pl * kEB < te) ? po + (uint64_t)pl * kEB : te;
+    const uint32_t base = (uint32_t)(po - ts);
+    const uint32_t dummy = kHotLabels * K;
+    const uint32_t j_lo = (uint32_t)((lo - po + 4 * kEB - 1) / (4 * kEB)), j_hi = (uint32_t)((hi - po + 4 * kEB - 1) / (4 * kEB));
+    const uint32_t L_beg = 4 * j_lo, L_end = (4 * j_hi < pl) ? 4 * j_hi : pl;
+    for (uint32_t L0 = L_beg + warp * kHotLabels; L0 < L_end; L0 += kConsumerWarps * kHotLabels) {
+        const uint32_t hb = kHotBlocks > 1 ? (h.it & 1) : 0;
+        h.it++;
+        float* hot = h.blk + hb * (kHotLabels * K + 4);
+        if (lane == 0) bulk_wait_read<kHotBlocks - 1>();   // the store that last used this block has read it
+        __syncwarp();
+        hot[hb ? h.b0 : h.a0] = 0.0f;
+        hot[hb ? h.b1 : h.a1] = 0.0f;
+        constexpr uint32_t kPerLane = kHotLabels / 32;
+        const uint32_t l0 = L0 + kPerLane * lane;
+        uint32_t slot0 = dummy, slot1 = dummy;
+        if (l0 < L_end) {
+            const int k = payload_class<kEB>(buf8, buf32, base, l0, K);
+            if (k >= 0) slot0 = (kPerLane * lane) * K + k;
+        }
+        if (kPerLane > 1 && l0 + 1 < L_end) {
+            const int k = payload_class<kEB>(buf8, buf32, base, l0 + 1, K);
+            if (k >= 0) slot1 = (kPerLane * lane + 1) * K + k;
+        }
+        hot[slot0] = 1.0f;
+        hot[slot1] = 1.0f;
+        if (hb) { h.b0 = slot0; h.b1 = slot1; } else { h.a0 = slot0; h.a1 = slot1; }
+        fence_proxy_async();
+        __syncwarp();
+        const uint32_t nl = (L_end - L0 < (uint32_t)kHotLabels) ? L_end - L0 : (uint32_t)kHotLabels;
+        const uint32_t nfl = nl * K, nb16 = (nfl * 4) & ~15u;
+        if (lane == 0) {
+            if (nb16) bulk_s2g(dst + (size_t)L0 * K, hot, nb16);
+            bulk_commit();
+        }
+        if ((uint32_t)lane < (nfl & 3)) dst[(size_t)L0 * K + (nfl & ~3u) + lane] = hot[(nfl & ~3u) + lane];
+    }
+}
+
+// label -> one-hot float32 for any K (used above kHotMaxK): float4 group g holds one-hot floats [4g, 4g+4), owned by the
+// tile of label 4g/K
+template <uint32_t kEB>
+__device__ __forceinline__ void sink_onehot_generic(const uint8_t* buf8, const uint32_t* buf32, uint64_t ts, uint64_t te,
+                                                    uint64_t po, uint64_t len, float* dst, int K) {
+    const uint32_t pl = (uint32_t)(len / kEB);   // labels
+    const uint64_t lo = po > ts ? po : ts, hi = (po + (uint64_t)pl * kEB < te) ? po + (uint64_t)pl * kEB : te;
+    const uint32_t base = (uint32_t)(po - ts);
+    const uint32_t nfl = pl * (uint32_t)K;
+    const uint32_t g_lo = (uint32_t)(((lo - po + kEB - 1) / kEB * K + 3) >> 2),
+                   g_hi = (uint32_t)(((hi - po + kEB - 1) / kEB * K + 3) >> 2), full4 = nfl >> 2;
+    for (uint32_t g = g_lo + threadIdx.x; g < g_hi; g += kTileThreads) {
+        const uint32_t f0 = 4 * g;
+        uint32_t l = f0 / (uint32_t)K;
+        uint32_t cc = f0 - l * (uint32_t)K;
+        float f[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            // a label without a class reads as 0xFFFFFFFF, which equals no class index
+            const uint32_t lab = (l < pl) ? (uint32_t)payload_class<kEB>(buf8, buf32, base, l, K) : 0xFFFFFFFFu;
+            f[k] = (lab == cc) ? 1.0f : 0.0f;
+            if (++cc == (uint32_t)K) {
+                cc = 0;
+                l++;
+            }
+        }
+        store_group(dst, g, full4, nfl, f);
+    }
 }
 
 struct RecRef {   // what finalize_record needs to know about the record
@@ -324,21 +461,7 @@ __device__ inline void finalize_record(const ParseArgs& a, const RecRef& j, uint
         }
         if (stored != mask_crc(crc)) st = 1;
     }
-    if (st == 0 && a.index && a.sink.mode != B2_SINK_NONE) {
-        const b2_example_index* ix = a.index + r;
-        if (ix->status != 0) st = 2;
-        else if (a.sink.mode == B2_SINK_RAW) {
-            if (ix->img_len > a.sink.img_stride || ix->tgt_len > a.sink.tgt_stride) st = 3;
-        } else if (kMode == B2_SINK_NORM_ONEHOT_F32) {
-            if (!norm_template_ok<kMode>(ix, a.sink.channels)) st = 2;
-            else if (!f32_rows_fit(ix, a.sink)) st = 3;
-        } else {
-            const uint64_t K = (uint64_t)a.sink.num_classes;
-            if (!norm_template_ok<B2_SINK_NORM_ONEHOT>(ix, a.sink.channels)) st = 2;
-            else if (ix->img_len * 4 > a.sink.img_stride || ix->tgt_len * K * 4 > a.sink.tgt_stride ||
-                     ix->img_len >= (1ull << 31) || ix->tgt_len * K >= (1ull << 31)) st = 3;
-        }
-    }
+    if (kMode != B2_SINK_NONE && st == 0 && a.index) st = sink_status<kMode>(a.index + r, a.sink);
     a.status[r] = st;
     if (st != 0 && a.n_bad) atomicAdd(reinterpret_cast<unsigned long long*>(a.n_bad), 1ull);
 }
@@ -361,12 +484,14 @@ struct RunAcc {          // shared-memory meeting point of the eight consumer wa
 // shared-memory slot and counts itself; the warp that arrives last moves the partial to the end of the record and
 // merges { CRC, tiles } into the record's 64-bit accumulator with an atomic XOR and an atomic add on the same address
 // (applied in program order, so no fences are needed), finalising the record when its tile count is complete.  The other warps are already working
-// on the next tile.
+// on the next tile.  Every warp flushes a run in the same loop iteration `it`, at most one run per iteration, and its
+// slot is `it` mod kRunSlots: a slot comes round again kRunSlots iterations later, and no warp can be more than kStages
+// (< kRunSlots) iterations ahead of the slowest, whose arrival on the buffer's empty barrier the producer waits for.
 template <int kMode>
-__device__ __forceinline__ void run_flush(const ParseArgs& a, Run& run, uint32_t& s, uint32_t& run_seq, bool want_crc,
+__device__ __forceinline__ void run_flush(const ParseArgs& a, Run& run, uint32_t& s, uint32_t it, bool want_crc,
                                           RunAcc* racc) {
     const int tid = threadIdx.x, lane = tid & 31;
-    RunAcc* ra = racc + (run_seq & (kRunSlots - 1));
+    RunAcc* ra = racc + (it & (kRunSlots - 1));
     const bool crc = want_crc && run.d1 - run.d0 >= 4;
     if (crc) {
         uint32_t t = multmodp_fast(__ldg(&a.tab->xinv16[tid]), s);
@@ -395,7 +520,6 @@ __device__ __forceinline__ void run_flush(const ParseArgs& a, Run& run, uint32_t
     }
     s = 0;
     run.open = false;
-    run_seq++;
 }
 
 // Development aid: cycles spent by lane 0 of every consumer warp in each phase of the tile loop (B2_PARSE_PROFILE=1).
@@ -512,14 +636,10 @@ fused_parse_kernel(const ParseArgs a) {
         img_S = kTileThreads - (kTileThreads % m);
     }
     uint32_t s = 0;                       // running CRC state of this thread
-    uint32_t run_seq = 0;
     Run run;
     run.open = false;
-    // this warp's one-hot blocks; float kHotLabels*K of a block is a dummy that is never stored
-    float* hot_w = hot_all + warp * kHotBlocks * (kHotLabels * K + 4);
     const uint32_t hot_dummy = kHotLabels * K;
-    uint32_t slotA0 = hot_dummy, slotA1 = hot_dummy, slotB0 = hot_dummy, slotB1 = hot_dummy;   // floats this lane set last time
-    uint32_t hot_it = 0;
+    HotBlocks hot{hot_all + warp * kHotBlocks * (kHotLabels * K + 4), hot_dummy, hot_dummy, hot_dummy, hot_dummy, 0};
     PROF_BEGIN();
 
     for (uint32_t it = 0;; it++) {
@@ -529,7 +649,7 @@ fused_parse_kernel(const ParseArgs a) {
         const TileJob& j = job[slot];
         const uint32_t flags = j.flags;
         const bool valid = (flags & 1) != 0;
-        if (run.open && (!valid || j.r != run.r || j.tile != run.last_tile + 1)) run_flush<kMode>(a, run, s, run_seq, want_crc, racc);
+        if (run.open && (!valid || j.r != run.r || j.tile != run.last_tile + 1)) run_flush<kMode>(a, run, s, it, want_crc, racc);
         PROF_MARK(5);
         if (flags & 4) break;
         if (valid) {
@@ -557,151 +677,16 @@ fused_parse_kernel(const ParseArgs a) {
                     sink_raw(buf32, buf8, ts, te, j.tgt_off, j.tgt_len, static_cast<uint8_t*>(a.sink.tgt_out) + (uint64_t)(j.r & a.row_mask) * a.sink.tgt_stride);
             }
             if (is_norm(kMode) && (flags & 2)) {
-                // payload elements are kEB bytes: uint8 (NORM_ONEHOT) or little-endian float32 (NORM_ONEHOT_F32)
                 constexpr uint32_t kEB = elem_bytes(kMode);
-                // ---- image -> (x-mean)/std float32
-                const uint64_t ipo = j.img_off, ipl64 = j.img_len;
-                if (a.sink.img_out && ipl64 && ipo < te && ipo + ipl64 > ts && (uint32_t)tid < img_S) {
-                    float* dst = reinterpret_cast<float*>(static_cast<uint8_t*>(a.sink.img_out) + (uint64_t)(j.r & a.row_mask) * a.sink.img_stride);
-                    const uint64_t po = ipo;
-                    const uint32_t pl = (uint32_t)(ipl64 / kEB);   // elements
-                    const uint64_t lo = po > ts ? po : ts, hi = (po + (uint64_t)pl * kEB < te) ? po + (uint64_t)pl * kEB : te;
-                    // float4 group g = image elements [4g, 4g+4) = payload bytes [4 kEB g, 4 kEB (g+1)); owned by the tile
-                    // that holds its first byte, its last bytes may sit in the halo
-                    const uint32_t g_lo = (uint32_t)((lo - po + 4 * kEB - 1) / (4 * kEB)), g_hi = (uint32_t)((hi - po + 4 * kEB - 1) / (4 * kEB)),
-                                   full4 = pl >> 2;
-                    // wraps when po < ts; base + 4 kEB g is back in [0, kTile) (mod 2^32)
-                    const uint32_t base = (uint32_t)(po - ts);
-                    uint32_t g = g_lo + tid;
-                    float mu[4], sd[4], rc[4];
-                    {
-                        uint32_t ch = (4u * g) % (uint32_t)C;
-#pragma unroll
-                        for (int k = 0; k < 4; k++) {
-                            mu[k] = s_mean[ch];
-                            sd[k] = s_std[ch];
-                            rc[k] = s_rcp[ch];
-                            ch = (ch + 1 == (uint32_t)C) ? 0 : ch + 1;
-                        }
-                    }
-                    for (; g < g_hi; g += img_S) {
-                        float f[4];
-                        if constexpr (kEB == 1) {
-                            const uint32_t x = smem_u32_unaligned(buf32, base + 4 * g);
-#pragma unroll
-                            for (int k = 0; k < 4; k++) {
-                                // byte k -> float, exactly: 0x4B000000 | v is 2^23 + v
-                                const float v = __uint_as_float(__byte_perm(x, 0x4B000000u, 0x7540 + k)) - 8388608.0f;
-                                const float d = __fsub_rn(v, mu[k]);
-                                f[k] = exact_div ? __fdiv_rn(d, sd[k]) : norm_fast(d, sd[k], rc[k]);
-                            }
-                        } else {
-                            // FloatList payloads start at any byte residue: four funnel-shifted words
-#pragma unroll
-                            for (int k = 0; k < 4; k++) {
-                                const float v = __uint_as_float(smem_u32_unaligned(buf32, base + 16 * g + 4 * k));
-                                f[k] = __fdiv_rn(__fsub_rn(v, mu[k]), sd[k]);
-                            }
-                        }
-                        if (g < full4) {
-                            st_cs(reinterpret_cast<float4*>(dst) + g, make_float4(f[0], f[1], f[2], f[3]));
-                        } else {   // the payload's last 1..3 elements
-                            if (4 * g + 0 < pl) dst[4 * g + 0] = f[0];
-                            if (4 * g + 1 < pl) dst[4 * g + 1] = f[1];
-                            if (4 * g + 2 < pl) dst[4 * g + 2] = f[2];
-                        }
-                    }
-                }
+                if (a.sink.img_out && (uint32_t)tid < img_S && tile_holds(ts, te, j.img_off, j.img_len))
+                    sink_image<kEB>(buf32, ts, te, j.img_off, j.img_len,
+                                    reinterpret_cast<float*>(static_cast<uint8_t*>(a.sink.img_out) + (uint64_t)(j.r & a.row_mask) * a.sink.img_stride),
+                                    img_S, s_mean, s_std, s_rcp, C, exact_div);
                 PROF_MARK(2);
-                // ---- target -> one-hot float32
-                const uint64_t tpo = j.tgt_off, tpl64 = j.tgt_len;
-                if (a.sink.tgt_out && tpl64 && tpo < te && tpo + tpl64 > ts) {
+                if (a.sink.tgt_out && tile_holds(ts, te, j.tgt_off, j.tgt_len)) {
                     float* dst = reinterpret_cast<float*>(static_cast<uint8_t*>(a.sink.tgt_out) + (uint64_t)(j.r & a.row_mask) * a.sink.tgt_stride);
-                    const uint64_t po = tpo;
-                    const uint32_t pl = (uint32_t)(tpl64 / kEB);   // labels
-                    const uint64_t lo = po > ts ? po : ts, hi = (po + (uint64_t)pl * kEB < te) ? po + (uint64_t)pl * kEB : te;
-                    const uint32_t base = (uint32_t)(po - ts);
-                    if (use_hot) {
-                        // Each warp owns blocks of kHotLabels*K floats in shared memory — zero except ONE 1.0f per label,
-                        // so a label costs one 4-byte shared-memory write — and pushes a block to HBM with a single TMA
-                        // bulk store; out-of-range labels write a dummy float past the block, so nothing is predicated.
-                        // Work unit = 4 labels (4K floats: a whole number of 16-byte groups, 16-byte aligned in the
-                        // output); a unit belongs to the tile holding its first label, later labels may sit in the halo.
-                        const uint32_t j_lo = (uint32_t)((lo - po + 4 * kEB - 1) / (4 * kEB)), j_hi = (uint32_t)((hi - po + 4 * kEB - 1) / (4 * kEB));
-                        const uint32_t L_beg = 4 * j_lo, L_end = (4 * j_hi < pl) ? 4 * j_hi : pl;
-                        for (uint32_t L0 = L_beg + warp * kHotLabels; L0 < L_end; L0 += kConsumerWarps * kHotLabels) {
-                            const uint32_t hb = kHotBlocks > 1 ? (hot_it & 1) : 0;
-                            hot_it++;
-                            float* hot = hot_w + hb * (kHotLabels * K + 4);
-                            if (lane == 0) bulk_wait_read<kHotBlocks - 1>();   // the store that last used this block has read it
-                            __syncwarp();
-                            hot[hb ? slotB0 : slotA0] = 0.0f;
-                            hot[hb ? slotB1 : slotA1] = 0.0f;
-                            constexpr uint32_t kPerLane = kHotLabels / 32;
-                            const uint32_t l0 = L0 + kPerLane * lane;
-                            uint32_t slot0 = hot_dummy, slot1 = hot_dummy;
-                            if constexpr (kEB == 1) {
-                                if (l0 < L_end) {
-                                    const uint32_t lab = buf8[base + l0];
-                                    if (lab < (uint32_t)K) slot0 = (kPerLane * lane) * K + lab;
-                                }
-                                if (kPerLane > 1 && l0 + 1 < L_end) {
-                                    const uint32_t lab = buf8[base + l0 + 1];
-                                    if (lab < (uint32_t)K) slot1 = (kPerLane * lane + 1) * K + lab;
-                                }
-                            } else {
-                                if (l0 < L_end) {
-                                    const int k = f32_label(buf32, base, l0, K);
-                                    if (k >= 0) slot0 = (kPerLane * lane) * K + k;
-                                }
-                                if (kPerLane > 1 && l0 + 1 < L_end) {
-                                    const int k = f32_label(buf32, base, l0 + 1, K);
-                                    if (k >= 0) slot1 = (kPerLane * lane + 1) * K + k;
-                                }
-                            }
-                            hot[slot0] = 1.0f;
-                            hot[slot1] = 1.0f;
-                            if (hb) { slotB0 = slot0; slotB1 = slot1; } else { slotA0 = slot0; slotA1 = slot1; }
-                            fence_proxy_async();
-                            __syncwarp();
-                            const uint32_t nl = (L_end - L0 < (uint32_t)kHotLabels) ? L_end - L0 : (uint32_t)kHotLabels;
-                            const uint32_t nfl = nl * K, nb16 = (nfl * 4) & ~15u;
-                            if (lane == 0) {
-                                if (nb16) bulk_s2g(dst + (size_t)L0 * K, hot, nb16);
-                                bulk_commit();
-                            }
-                            if ((uint32_t)lane < (nfl & 3)) dst[(size_t)L0 * K + (nfl & ~3u) + lane] = hot[(nfl & ~3u) + lane];
-                        }
-                    } else {
-                        // generic path (K > 32): float4 group g holds one-hot floats [4g, 4g+4), owned by the tile of label 4g/K
-                        const uint32_t nfl = pl * (uint32_t)K;
-                        const uint32_t g_lo = (uint32_t)(((lo - po + kEB - 1) / kEB * K + 3) >> 2),
-                                       g_hi = (uint32_t)(((hi - po + kEB - 1) / kEB * K + 3) >> 2), full4 = nfl >> 2;
-                        for (uint32_t g = g_lo + tid; g < g_hi; g += kTileThreads) {
-                            const uint32_t f0 = 4 * g;
-                            uint32_t l = f0 / (uint32_t)K;
-                            uint32_t cc = f0 - l * (uint32_t)K;
-                            float f[4];
-#pragma unroll
-                            for (int k = 0; k < 4; k++) {
-                                uint32_t lab;
-                                if constexpr (kEB == 1) lab = (l < pl) ? buf8[base + l] : 0xFFFFFFFFu;
-                                else lab = (l < pl) ? (uint32_t)f32_label(buf32, base, l, K) : 0xFFFFFFFFu;
-                                f[k] = (lab == cc) ? 1.0f : 0.0f;
-                                if (++cc == (uint32_t)K) {
-                                    cc = 0;
-                                    l++;
-                                }
-                            }
-                            if (g < full4) {
-                                st_cs(reinterpret_cast<float4*>(dst) + g, make_float4(f[0], f[1], f[2], f[3]));
-                            } else {
-                                if (f0 + 0 < nfl) dst[f0 + 0] = f[0];
-                                if (f0 + 1 < nfl) dst[f0 + 1] = f[1];
-                                if (f0 + 2 < nfl) dst[f0 + 2] = f[2];
-                            }
-                        }
-                    }
+                    if (use_hot) sink_onehot_smem<kEB>(buf8, buf32, ts, te, j.tgt_off, j.tgt_len, dst, K, hot);
+                    else sink_onehot_generic<kEB>(buf8, buf32, ts, te, j.tgt_off, j.tgt_len, dst, K);
                 }
                 PROF_MARK(3);
             }
@@ -720,11 +705,7 @@ using namespace b2;
 
 namespace {
 
-struct LaunchCfg {
-    bool ready = false;
-    int ctas_per_sm[3] = {0, 0, 0};
-};
-LaunchCfg g_cfg[64];
+bool g_smem_ready[64];   // per device: the kernels' shared-memory opt-ins are set
 
 constexpr size_t dyn_bytes(int mode, int K) {
     return (size_t)stages_for(mode) * kBufBytes +
@@ -746,32 +727,31 @@ int set_dyn_smem(F* kernel, size_t dyn, int device) {
     return 0;
 }
 
+// The kernel that runs a sink mode; prof picks the NORM_ONEHOT instantiation with the per-phase cycle counters.
+using ParseKernel = void (*)(const ParseArgs);
+ParseKernel fused_kernel(int mode, bool prof) {
+    const ParseKernel k[] = {fused_parse_kernel<B2_SINK_NONE>, fused_parse_kernel<B2_SINK_RAW>, fused_parse_kernel<B2_SINK_NORM_ONEHOT>,
+                             fused_parse_kernel<B2_SINK_NORM_ONEHOT_F32>};
+    if (mode == B2_SINK_NORM_ONEHOT && prof) return fused_parse_kernel<B2_SINK_NORM_ONEHOT, true>;
+    return mode >= B2_SINK_NONE && mode <= B2_SINK_NORM_ONEHOT_F32 ? k[mode] : nullptr;
+}
+
 int launch_fused(b2_ctx* ctx, const ParseArgs& pa, uint64_t max_tiles, cudaStream_t s) {
-    LaunchCfg& cfg = g_cfg[ctx->device & 63];
-    if (!cfg.ready) {
-        // opt-in ceilings; NORM_ONEHOT and NORM_ONEHOT_F32: what their largest launch (K = kHotMaxK) asks for.  A
-        // ceiling only: occupancy follows each launch's actual request.
-        if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NONE>, 96 * 1024, ctx->device)) return e;
-        if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_RAW>, 96 * 1024, ctx->device)) return e;
-        if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NORM_ONEHOT>, kNormDynMax, ctx->device)) return e;
-        if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NORM_ONEHOT, true>, kNormDynMax, ctx->device)) return e;
-        if (int e = set_dyn_smem(fused_parse_kernel<B2_SINK_NORM_ONEHOT_F32>, kNormDynMax, ctx->device)) return e;
-        cfg.ready = true;
+    if (!g_smem_ready[ctx->device & 63]) {
+        // opt-in ceilings of every kernel; the normalise + one-hot modes: what their largest launch (K = kHotMaxK) asks
+        // for.  A ceiling only: occupancy follows each launch's actual request.
+        for (int mode = B2_SINK_NONE; mode <= B2_SINK_NORM_ONEHOT_F32; mode++)
+            for (int prof = 0; prof <= (mode == B2_SINK_NORM_ONEHOT); prof++)   // only NORM_ONEHOT has a profiling twin
+                if (int e = set_dyn_smem(fused_kernel(mode, prof), is_norm(mode) ? kNormDynMax : 96 * 1024, ctx->device)) return e;
+        g_smem_ready[ctx->device & 63] = true;
     }
+    const ParseKernel kernel = fused_kernel(pa.sink.mode, pa.prof != nullptr);
+    B2_REQUIRE(kernel, "fused parse: no kernel for this sink mode");
     // persistent grid: as many CTAs as fit on the GPU at once (4 per SM), never more than there are chunks
     const uint64_t chunks = (max_tiles + pa.q - 1) / pa.q;
     const uint64_t resident = (uint64_t)ctx->sm_count * (is_norm(pa.sink.mode) ? 3 : 5);
     const unsigned grid = (unsigned)(chunks < resident ? chunks : resident);
-    const size_t dyn = dyn_bytes(pa.sink.mode, pa.sink.num_classes);
-    switch (pa.sink.mode) {
-        case B2_SINK_NONE: fused_parse_kernel<B2_SINK_NONE><<<grid, kCtaThreads, dyn, s>>>(pa); break;
-        case B2_SINK_RAW: fused_parse_kernel<B2_SINK_RAW><<<grid, kCtaThreads, dyn, s>>>(pa); break;
-        case B2_SINK_NORM_ONEHOT_F32: fused_parse_kernel<B2_SINK_NORM_ONEHOT_F32><<<grid, kCtaThreads, dyn, s>>>(pa); break;
-        default:
-            if (pa.prof) fused_parse_kernel<B2_SINK_NORM_ONEHOT, true><<<grid, kCtaThreads, dyn, s>>>(pa);
-            else fused_parse_kernel<B2_SINK_NORM_ONEHOT><<<grid, kCtaThreads, dyn, s>>>(pa);
-            break;
-    }
+    kernel<<<grid, kCtaThreads, dyn_bytes(pa.sink.mode, pa.sink.num_classes), s>>>(pa);
     ctx->launches++;
     B2_CUDA(cudaGetLastError());
     return 0;
@@ -829,6 +809,39 @@ unsigned long long* dev_profile(b2_ctx* ctx) {
 #endif
 }
 
+// A launch's arguments: the fields every launch sets; the rest start zeroed.
+ParseArgs parse_args(b2_ctx* ctx, const uint8_t* shard, uint64_t nbytes, const uint64_t* rec_off, const uint64_t* rec_len,
+                     const b2_example_index* index, const b2_parse_sink& sink, int32_t* status) {
+    ParseArgs pa{};
+    pa.shard = shard;
+    pa.nbytes = nbytes;
+    pa.rec_off = rec_off;
+    pa.rec_len = rec_len;
+    pa.index = index;
+    pa.sink = sink;
+    pa.tab = ctx->crc_dev;
+    pa.q = tiles_per_cta(sink.mode);
+    pa.status = status;
+    pa.row_mask = ~0u;
+    return pa;
+}
+
+// Uniform tile map for n records of at most max_len bytes: tile w belongs to record w / tiles_x.  The per-record
+// accumulators and the scheduler words live in the context workspace: calls on one context must be stream-ordered.
+int launch_uniform(b2_ctx* ctx, ParseArgs& pa, int n, uint64_t max_len, cudaStream_t s, const char* who) {
+    uint64_t tx = (max_len + 15 + kTile - 1) / kTile;
+    if (!tx) tx = 1;
+    B2_REQUIRE(tx * (uint64_t)n < (1ull << 32), std::string(who) + ": too many tiles for one call");
+    WsLock ws_lock(ctx);
+    if (int e = ws_reserve(ctx, (size_t)n * 8 + 8, s)) return e;
+    B2_CUDA(cudaMemsetAsync(ctx->ws, 0, (size_t)n * 8 + 8, s));
+    pa.tiles_x = (uint32_t)tx;
+    pa.n = (uint32_t)n;
+    pa.acc = static_cast<unsigned long long*>(ctx->ws);             // n per-record accumulators ...
+    pa.sched = reinterpret_cast<uint32_t*>(pa.acc + n);              // ... then the scheduler's two words
+    return launch_fused(ctx, pa, tx * (uint64_t)n, s);
+}
+
 }  // namespace
 
 extern "C" int b2_tfrecord_parse(b2_ctx* ctx, const uint8_t* shard, uint64_t nbytes, const uint64_t* rec_off,
@@ -842,18 +855,8 @@ extern "C" int b2_tfrecord_parse(b2_ctx* ctx, const uint8_t* shard, uint64_t nby
     if (int e = check_sink(sink, "b2_tfrecord_parse")) return e;
     if (n == 0) return 0;
     DeviceGuard g(ctx->device);
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    uint64_t tx = (max_record_len + 15 + kTile - 1) / kTile;
-    if (!tx) tx = 1;
-    B2_REQUIRE(tx * (uint64_t)n < (1ull << 32), "b2_tfrecord_parse: too many tiles for one call");
-    // per-record accumulators live in the context workspace: calls on one context must be stream-ordered
-    WsLock ws_lock(ctx);
-    if (int e = ws_reserve(ctx, (size_t)n * 8 + 8, s)) return e;
-    B2_CUDA(cudaMemsetAsync(ctx->ws, 0, (size_t)n * 8 + 8, s));
-    uint32_t* acc = static_cast<uint32_t*>(ctx->ws);
-    ParseArgs pa{shard, nbytes, rec_off, rec_len, index, *sink, ctx->crc_dev, nullptr, nullptr, nullptr,
-                 (uint32_t)tx, (uint32_t)n, tiles_per_cta(sink->mode), reinterpret_cast<unsigned long long*>(acc), status, nullptr, nullptr, acc + 2 * (size_t)n, nullptr, ~0u};
-    return launch_fused(ctx, pa, tx * (uint64_t)n, s);
+    ParseArgs pa = parse_args(ctx, shard, nbytes, rec_off, rec_len, index, *sink, status);
+    return launch_uniform(ctx, pa, n, max_record_len, static_cast<cudaStream_t>(stream), "b2_tfrecord_parse");
 }
 
 extern "C" int b2_tfrecord_parse_table(b2_ctx* ctx, const uint8_t* shard, uint64_t nbytes, uint64_t max_records,
@@ -865,9 +868,15 @@ extern "C" int b2_tfrecord_parse_table(b2_ctx* ctx, const uint8_t* shard, uint64
     if (int e = check_sink(sink, "b2_tfrecord_parse_table")) return e;
     DeviceGuard g(ctx->device);
     const TableView v = table_view(table, nbytes, max_records);
-    ParseArgs pa{shard, nbytes, v.rec_off, v.rec_len, v.index, *sink, ctx->crc_dev, v.tile2rec, v.tile_start, v.hdr,
-                 0, 0, tiles_per_cta(sink->mode), v.acc, status, nullptr, v.hdr + 4, reinterpret_cast<uint32_t*>(v.hdr + 5),
-                 dev_profile(ctx), dev_row_mask()};
+    ParseArgs pa = parse_args(ctx, shard, nbytes, v.rec_off, v.rec_len, v.index, *sink, status);
+    pa.tile2rec = v.tile2rec;
+    pa.tile_start = v.tile_start;
+    pa.hdr = v.hdr;
+    pa.acc = v.acc;
+    pa.n_bad = v.hdr + 4;
+    pa.sched = reinterpret_cast<uint32_t*>(v.hdr + 5);
+    pa.prof = dev_profile(ctx);
+    pa.row_mask = dev_row_mask();
     return launch_fused(ctx, pa, v.cap_tiles, static_cast<cudaStream_t>(stream));
 }
 
@@ -878,21 +887,11 @@ extern "C" int b2_crc32c(b2_ctx* ctx, const uint8_t* data, const uint64_t* offse
     B2_REQUIRE((reinterpret_cast<uintptr_t>(data) & 15) == 0, "b2_crc32c: data must be 16-byte aligned");
     if (n == 0) return 0;
     DeviceGuard g(ctx->device);
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    uint64_t tx = (max_len + 15 + kTile - 1) / kTile;
-    if (!tx) tx = 1;
-    B2_REQUIRE(tx * (uint64_t)n < (1ull << 32), "b2_crc32c: too many tiles for one call");
-    WsLock ws_lock(ctx);
-    if (int e = ws_reserve(ctx, (size_t)n * 8 + 8, s)) return e;
-    B2_CUDA(cudaMemsetAsync(ctx->ws, 0, (size_t)n * 8 + 8, s));
-    uint32_t* acc = static_cast<uint32_t*>(ctx->ws);
-    b2_parse_sink sink;
-    memset(&sink, 0, sizeof(sink));
-    sink.mode = B2_SINK_NONE;
+    b2_parse_sink sink{};   // B2_SINK_NONE: CRC only
     sink.verify_crc = 1;
-    ParseArgs pa{data, ~0ull, offsets, lens, nullptr, sink, ctx->crc_dev, nullptr, nullptr, nullptr,
-                 (uint32_t)tx, (uint32_t)n, tiles_per_cta(B2_SINK_NONE), reinterpret_cast<unsigned long long*>(acc), nullptr, crc_out, nullptr, acc + 2 * (size_t)n, nullptr, ~0u};
-    return launch_fused(ctx, pa, tx * (uint64_t)n, s);
+    ParseArgs pa = parse_args(ctx, data, ~0ull, offsets, lens, nullptr, sink, nullptr);
+    pa.crc_out = crc_out;
+    return launch_uniform(ctx, pa, n, max_len, static_cast<cudaStream_t>(stream), "b2_crc32c");
 }
 
 #ifdef B2_DEV_KNOBS

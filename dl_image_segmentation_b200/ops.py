@@ -150,6 +150,15 @@ def nearest_date_mosaic(stacks, valids, scene_day, scene_cf, ref_day, min_day=No
 
 
 # --------------------------------------------------------------------------------------------- K4
+def _band_constants(mean, std, device, who, C=None):
+    """mean / std as float32 device tensors with one entry per band: C of them, or as many as mean has."""
+    mean, std = (to_device(np.asarray(v, dtype=np.float32) if not isinstance(v, torch.Tensor) else v, device) for v in (mean, std))
+    C = int(mean.numel()) if C is None else C
+    if mean.numel() != C or std.numel() != C:
+        raise B2Error("%s: mean/std must have one entry per band" % who)
+    return mean, std
+
+
 def normalise_onehot(img, label, mean, std, num_classes, device=None):
     """(N,H,W,C) u8/u16/i16/f32 + (N,H,W) u8/f32 -> ((N,H,W,C) f32, (N,H,W,K) f32).  b2_normalise_onehot."""
     ctx = get_ctx(device)
@@ -159,10 +168,7 @@ def normalise_onehot(img, label, mean, std, num_classes, device=None):
     if img is not None:
         img = to_device(img, ctx.device)
         C = img.shape[-1]
-        mean_d = to_device(np.asarray(mean, dtype=np.float32) if not isinstance(mean, torch.Tensor) else mean, ctx.device)
-        std_d = to_device(np.asarray(std, dtype=np.float32) if not isinstance(std, torch.Tensor) else std, ctx.device)
-        if mean_d.numel() != C or std_d.numel() != C:
-            raise B2Error("normalise_onehot: mean/std must have one entry per band")
+        mean_d, std_d = _band_constants(mean, std, ctx.device, "normalise_onehot", C)
         img_out = torch.empty(img.shape, dtype=torch.float32, device=ctx.device)
         n_pix = img.numel() // C
         check(lib().b2_normalise_onehot(ctx.handle, ptr(img), b2_dtype(img), None, 0, ptr(mean_d), ptr(std_d), n_pix, C, 1,
@@ -351,6 +357,26 @@ def _align16(x):
     return (int(x) + 15) & ~15
 
 
+# sink mode -> (b2_parse_sink.mode, payload bytes per element of the normalise / one-hot modes, 0 for the others)
+_SINK_MODES = {"none": (_lib.SINK_NONE, 0), "raw": (_lib.SINK_RAW, 0), "norm_onehot": (_lib.SINK_NORM_ONEHOT, 1),
+               "norm_onehot_f32": (_lib.SINK_NORM_ONEHOT_F32, 4)}
+
+
+def _sink_mode(mode):
+    if mode not in _SINK_MODES:
+        raise ValueError(mode)
+    return _SINK_MODES[mode]
+
+
+def _float_rows(img_elems, tgt_elems, num_classes):
+    """Row lengths (floats) of the normalised image and one-hot buffers for payloads of img_elems / tgt_elems elements:
+    the sink needs 16-byte strides, so both are padded to 16 elements unless the rows already are whole 16-byte units."""
+    il, tl, K = int(img_elems), int(tgt_elems), int(num_classes)
+    if (il * 4) % 16 or (tl * K * 4) % 16:
+        il, tl = _align16(il), _align16(tl)
+    return il, tl * K
+
+
 def parse_shard(si: ShardIndex, mode, verify_crc=True, mean=None, std=None, num_classes=None, first=0, count=None,
                 out=None):
     """Run the fused parse kernel over records [first, first+count).  Returns (img_buf, tgt_buf, status_dev).
@@ -365,46 +391,25 @@ def parse_shard(si: ShardIndex, mode, verify_crc=True, mean=None, std=None, num_
     count = si.n - first if count is None else count
     if count <= 0:
         return None, None, None
+    _, esz = _sink_mode(mode)
     idx = si.index[first:first + count] if si.index is not None else None
-    sink = _lib.ParseSink()
-    sink.verify_crc = 1 if verify_crc else 0
     img_buf = tgt_buf = None
-    if mode == "none":
-        sink.mode = _lib.SINK_NONE
-    elif mode == "raw":
-        sink.mode = _lib.SINK_RAW
+    if mode == "raw":
         istr, tstr = _align16(max(1, idx["img_len"].max())), _align16(max(1, idx["tgt_len"].max()))
         img_buf, tgt_buf = out if out is not None else (
             torch.empty((count, istr), dtype=torch.uint8, device=ctx.device),
             torch.empty((count, tstr), dtype=torch.uint8, device=ctx.device))
-        sink.img_out, sink.img_stride = img_buf.data_ptr(), img_buf.stride(0)
-        sink.tgt_out, sink.tgt_stride = tgt_buf.data_ptr(), tgt_buf.stride(0)
-    elif mode in ("norm_onehot", "norm_onehot_f32"):
-        f32 = mode == "norm_onehot_f32"
-        sink.mode = _lib.SINK_NORM_ONEHOT_F32 if f32 else _lib.SINK_NORM_ONEHOT
-        K = int(num_classes)
-        esz = 4 if f32 else 1
-        il, tl = int(idx["img_len"].max()) // esz, int(idx["tgt_len"].max()) // esz
-        if (il * 4) % 16 or (tl * K * 4) % 16:
-            il, tl = _align16(il), _align16(tl)
+    elif esz:
+        # the band count is the sink's, as in parse_table: a record with another band count gets status 2
+        mean, std = _band_constants(mean, std, ctx.device, "parse_shard")
+        il, tl = _float_rows(int(idx["img_len"].max()) // esz, int(idx["tgt_len"].max()) // esz, num_classes)
         img_buf, tgt_buf = out if out is not None else (
             torch.empty((count, il), dtype=torch.float32, device=ctx.device),
-            torch.empty((count, tl * K), dtype=torch.float32, device=ctx.device))
-        mean_d = to_device(np.asarray(mean, dtype=np.float32) if not isinstance(mean, torch.Tensor) else mean, ctx.device)
-        std_d = to_device(np.asarray(std, dtype=np.float32) if not isinstance(std, torch.Tensor) else std, ctx.device)
-        # the band count is the sink's, as in parse_table: a record with another band count gets status 2
-        C = int(mean_d.numel())
-        if std_d.numel() != C:
-            raise B2Error("parse_shard: mean/std must have one entry per band")
-        sink.img_out, sink.img_stride = img_buf.data_ptr(), img_buf.stride(0) * 4
-        sink.tgt_out, sink.tgt_stride = tgt_buf.data_ptr(), tgt_buf.stride(0) * 4
-        sink.mean, sink.std, sink.channels, sink.num_classes = mean_d.data_ptr(), std_d.data_ptr(), C, K
-        sink._keep = (mean_d, std_d)
-    else:
-        raise ValueError(mode)
+            torch.empty((count, tl), dtype=torch.float32, device=ctx.device))
+    sink = _make_sink(mode, verify_crc, img_buf, tgt_buf, mean, std, num_classes)
     status = torch.empty((count,), dtype=torch.int32, device=ctx.device)
-    esz = ctypes.sizeof(_lib.ExampleIndex)
-    index_ptr = ctypes.c_void_p(si.index_dev.data_ptr() + first * esz) if si.index_dev is not None else None
+    isz = ctypes.sizeof(_lib.ExampleIndex)
+    index_ptr = ctypes.c_void_p(si.index_dev.data_ptr() + first * isz) if si.index_dev is not None else None
     check(lib().b2_tfrecord_parse(
         ctx.handle, ptr(si.shard), si.nbytes, ctypes.c_void_p(si.rec_off.data_ptr() + 8 * first),
         ctypes.c_void_p(si.rec_len.data_ptr() + 8 * first), index_ptr, count,
@@ -478,24 +483,20 @@ def build_records(items, device=None):
     return plan.launch(), plan.offsets, plan.total
 
 
-def _make_sink(ctx, mode, verify_crc, mean, std, num_classes, channels, img_buf, tgt_buf):
+def _make_sink(mode, verify_crc, img_buf, tgt_buf, mean=None, std=None, num_classes=None):
+    """The b2_parse_sink for a mode; mean / std are float32 device tensors (their length is the band count)."""
     sink = _lib.ParseSink()
+    sink.mode, esz = _sink_mode(mode)
     sink.verify_crc = 1 if verify_crc else 0
-    if mode == "none":
-        sink.mode = _lib.SINK_NONE
-    elif mode == "raw":
-        sink.mode = _lib.SINK_RAW
+    if mode == "raw":
         sink.img_out, sink.img_stride = img_buf.data_ptr(), img_buf.stride(0) * img_buf.element_size()
         sink.tgt_out, sink.tgt_stride = tgt_buf.data_ptr(), tgt_buf.stride(0) * tgt_buf.element_size()
-    elif mode in ("norm_onehot", "norm_onehot_f32"):
-        sink.mode = _lib.SINK_NORM_ONEHOT_F32 if mode == "norm_onehot_f32" else _lib.SINK_NORM_ONEHOT
+    elif esz:
         sink.img_out, sink.img_stride = img_buf.data_ptr(), img_buf.stride(0) * 4
         sink.tgt_out, sink.tgt_stride = tgt_buf.data_ptr(), tgt_buf.stride(0) * 4
         sink.mean, sink.std = mean.data_ptr(), std.data_ptr()
-        sink.channels, sink.num_classes = int(channels), int(num_classes)
+        sink.channels, sink.num_classes = int(mean.numel()), int(num_classes)
         sink._keep = (mean, std)
-    else:
-        raise ValueError(mode)
     return sink
 
 
@@ -512,26 +513,19 @@ def parse_table(st: ShardTable, mode, img_elems=0, tgt_elems=0, verify_crc=True,
     """
     ctx = get_ctx(st.shard.device)
     cap = st.max_records
+    _, esz = _sink_mode(mode)
     img_buf = tgt_buf = None
-    C = 1
     if mode == "raw":
         img_buf, tgt_buf = out if out is not None else (
             torch.empty((cap, _align16(max(1, img_elems))), dtype=torch.uint8, device=ctx.device),
             torch.empty((cap, _align16(max(1, tgt_elems))), dtype=torch.uint8, device=ctx.device))
-    elif mode in ("norm_onehot", "norm_onehot_f32"):
-        K = int(num_classes)
-        mean = to_device(np.asarray(mean, dtype=np.float32) if not isinstance(mean, torch.Tensor) else mean, ctx.device)
-        std = to_device(np.asarray(std, dtype=np.float32) if not isinstance(std, torch.Tensor) else std, ctx.device)
-        C = int(mean.numel())
-        if std.numel() != C:
-            raise B2Error("parse_table: mean/std must have one entry per band")
-        il, tl = int(img_elems), int(tgt_elems)
-        if (il * 4) % 16 or (tl * K * 4) % 16:
-            il, tl = _align16(il), _align16(tl)
+    elif esz:
+        mean, std = _band_constants(mean, std, ctx.device, "parse_table")
+        il, tl = _float_rows(img_elems, tgt_elems, num_classes)
         img_buf, tgt_buf = out if out is not None else (
             torch.empty((cap, il), dtype=torch.float32, device=ctx.device),
-            torch.empty((cap, tl * K), dtype=torch.float32, device=ctx.device))
-    sink = _make_sink(ctx, mode, verify_crc, mean, std, num_classes, C, img_buf, tgt_buf)
+            torch.empty((cap, tl), dtype=torch.float32, device=ctx.device))
+    sink = _make_sink(mode, verify_crc, img_buf, tgt_buf, mean, std, num_classes)
     if not want_img:
         sink.img_out = None          # the C ABI skips a NULL output
     if not want_tgt:
@@ -562,8 +556,9 @@ class ShardPipeline:
         self.mode, self.verify_crc, self.num_classes = mode, verify_crc, num_classes
         self.img_elems, self.tgt_elems, self.cap, self.depth = int(img_elems), int(tgt_elems), int(max_records), int(depth)
         self.open_ahead = max(int(open_ahead), self.depth)
-        self.mean = None if mean is None else to_device(np.asarray(mean, dtype=np.float32) if not isinstance(mean, torch.Tensor) else mean, dev)
-        self.std = None if std is None else to_device(np.asarray(std, dtype=np.float32) if not isinstance(std, torch.Tensor) else std, dev)
+        self.mean = self.std = None
+        if mean is not None:
+            self.mean, self.std = _band_constants(mean, std, dev, "ShardPipeline")
         self.open_streams = [torch.cuda.Stream(dev, priority=-1) for _ in range(min(self.open_ahead, 4))]
         self.streams = [torch.cuda.Stream(dev) for _ in range(self.depth)]
         self.oslots = [dict(stage=None, table=None, opened=torch.cuda.Event(), parsed=None) for _ in range(self.open_ahead)]

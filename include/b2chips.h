@@ -152,13 +152,13 @@ typedef struct {
 } b2_parse_sink;
 
 /* One fused pass over the records: CRC verify + payload scatter/cast.  status_dev[i]: 0 ok, 1 data-CRC mismatch
- * (TF: DataLossError), 2 index status != 0, or in NORM_ONEHOT mode a record that does not fit the template (a payload
- * that is not BytesList, image/channels != sink channels, image length != height*width*channels, target length !=
- * target height*width), 3 payload larger than its output stride.  NORM_ONEHOT_F32 (as parse_higher_dtype_array_proto
- * followed by normalise and one-hot): 2 also for a payload that is not packed FloatList (a BytesList record included),
- * image/channels != sink channels, image length != 4*height*width*channels bytes, target length != 4*target
- * height*width bytes or a negative dimension; 3 for a payload longer than its output row or of 2^31 elements or more
- * (image elements, or target elements * K).  Unpacked FloatList is status 2 from the index.  Uses the context workspace:
+ * (TF: DataLossError), 2 index status != 0, 3 payload larger than its output stride (RAW).  The two normalise + one-hot
+ * modes apply one rule with element width E (1 byte: NORM_ONEHOT, BytesList; 4 bytes: NORM_ONEHOT_F32, packed
+ * FloatList, as parse_higher_dtype_array_proto followed by normalise and one-hot): 2 for a record that does not fit the
+ * template (a payload that is not of the mode's kind, a BytesList record in NORM_ONEHOT_F32 included; image/channels != sink
+ * channels; a negative dimension; image length != E*height*width*channels bytes or target length != E*target
+ * height*width bytes), 3 for a payload whose floats do not fit its output row or of 2^31 elements or more (image
+ * elements, or target elements * K).  Unpacked FloatList is status 2 from the index.  Uses the context workspace:
  * calls on one context must be stream-ordered (b2_tfrecord_parse_table has no such restriction). */
 int b2_tfrecord_parse(b2_ctx* ctx, const uint8_t* shard_dev, uint64_t shard_nbytes, const uint64_t* rec_offsets_dev,
                       const uint64_t* rec_lens_dev, const b2_example_index* index_dev, int n,

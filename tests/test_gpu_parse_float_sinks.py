@@ -7,7 +7,7 @@ the image stride, inexact means, negative / zero / tiny stds, class counts on bo
 float labels that have no class, payloads starting at every residue mod 16, per-record statuses, the streaming
 readers, a record past 2048 CRC tiles and full-size cfg3 records.
 
-The references are restated here; the test_reference_* functions need no GPU.
+The references are restated in tests/_sink_refs.py; the test_reference_* functions need no GPU.
 """
 import functools
 import math
@@ -16,50 +16,13 @@ from fractions import Fraction
 import numpy as np
 import pytest
 
+from _sink_refs import _bits_differ, _parse_both, _record, _round_f32, ref_normalise, ref_one_hot
 from oracle import example_proto as oep
 from oracle import normalise as onorm
 from oracle import tfrecord as otfr
 
 
 # ------------------------------------------------------------------------------------------------ references (CPU)
-def ref_normalise(x, mean, std):
-    """(float32(x) - mean) / std per band (last axis), rounded to float32 after the subtraction and after the division.
-
-    Computed in float64: a float64 result of one +, - or / of float32 operands, rounded to float32, is the correctly
-    rounded float32 result (float64 has at least 2*24 + 2 bits), so this is IEEE float32 arithmetic."""
-    mean = np.asarray(mean, np.float32).astype(np.float64)
-    std = np.asarray(std, np.float32).astype(np.float64)
-    with np.errstate(all="ignore"):
-        d = (np.asarray(x).astype(np.float32).astype(np.float64) - mean).astype(np.float32)
-        return (d.astype(np.float64) / std).astype(np.float32)
-
-
-def ref_one_hot(label, K):
-    """Row k is 1.0 iff the float32 label's value equals k: NaN, +-inf, negative, non-integral and >= K labels give a
-    zero row, -0.0 is class 0."""
-    lab = np.asarray(label).astype(np.float32).astype(np.float64)
-    return (lab[..., None] == np.arange(K, dtype=np.float64)).astype(np.float32)
-
-
-def _round_f32(q, neg=False):
-    """Exact rational -> float32, round to nearest even; subnormals, underflow to a signed zero, overflow to inf."""
-    if q == 0:
-        return np.float32(-0.0 if neg else 0.0)
-    s = -1.0 if q < 0 else 1.0
-    a = abs(q)
-    e = a.numerator.bit_length() - a.denominator.bit_length()
-    while Fraction(2) ** e > a:
-        e -= 1
-    while Fraction(2) ** (e + 1) <= a:
-        e += 1
-    u = max(e - 23, -149)
-    m = round(a / Fraction(2) ** u)
-    v = m * Fraction(2) ** u
-    if v >= Fraction(2) ** 128:
-        return np.float32(s * math.inf)
-    return np.float32(math.copysign(float(v), s))
-
-
 def _exact_quotient(x, m, s):
     """(x - m) / s in float32 arithmetic, from exact rationals, for finite float32 x, m and s."""
     xm = Fraction(float(x)) - Fraction(float(m))
@@ -68,13 +31,6 @@ def _exact_quotient(x, m, s):
         return np.float32(np.nan) if d == 0 else np.float32(math.copysign(math.inf, float(d)) * math.copysign(1.0, float(s)))
     neg = (math.copysign(1.0, float(d)) < 0) != (float(s) < 0)
     return _round_f32(Fraction(float(d)) / Fraction(float(s)), neg)
-
-
-def _bits_differ(got, want):
-    """Positions where two float32 arrays differ bit for bit; NaN matches NaN whatever the payload."""
-    got, want = np.asarray(got, np.float32), np.asarray(want, np.float32)
-    gn, wn = np.isnan(got), np.isnan(want)
-    return (got.view(np.uint32) != want.view(np.uint32)) & ~(gn & wn) | (gn != wn)
 
 
 SPECIAL = np.array([0.0, -0.0, np.inf, -np.inf, np.nan, 3e38, -3e38, 1e-40, -1e-45, 16777217.0, 0.1, 65535.0, -32768.0,
@@ -167,13 +123,6 @@ def _chip(rng, h, w, C, dtype, K=40):
     return img, lab
 
 
-def _record(img, lab, ident, dims=None):
-    h, w, c = img.shape
-    th, tw = lab.shape
-    h, w, c, th, tw = dims or (h, w, c, th, tw)
-    return otfr.frame(oep.convert_to_example(img, lab, h, w, c, th, tw, ident).SerializeToString())
-
-
 @functools.lru_cache(maxsize=None)
 def _shard(C, dtype, K=40):
     """41 FloatList records of C bands; identifier lengths 0..40 move the payload starts through every residue mod 16."""
@@ -205,28 +154,6 @@ def _opened(C, dtype, dev):
     return _Opened(*_shard(C, dtype), dev)
 
 
-def _parse_both(op, mean, std, K, img_elems=None, tgt_elems=None):
-    """Yield (name, img_buf, tgt_buf, status) from parse_shard and parse_table."""
-    import torch
-
-    from dl_image_segmentation_b200 import ops
-    n = op.si.n
-    il = op.img_elems if img_elems is None else img_elems
-    tl = op.tgt_elems if tgt_elems is None else tgt_elems
-    dev = op.si.shard.device
-    out = None
-    if img_elems is not None:
-        out = (torch.empty((n, il), dtype=torch.float32, device=dev), torch.empty((n, tl * K), dtype=torch.float32, device=dev))
-    ib, tb, st = ops.parse_shard(op.si, "norm_onehot_f32", mean=mean, std=std, num_classes=K, out=out)
-    yield "parse_shard", ib, tb, st[:n].cpu().numpy()
-    del ib, tb
-    out = (torch.empty((n, il), dtype=torch.float32, device=dev), torch.empty((n, tl * K), dtype=torch.float32, device=dev))
-    ib, tb, st = ops.parse_table(op.si.table, "norm_onehot_f32", il, tl, mean=mean, std=std, num_classes=K, out=out)
-    stat = st[:n].cpu().numpy()
-    assert op.si.table.header()[4] == int((stat != 0).sum())
-    yield "parse_table", ib, tb, stat
-
-
 def _check_rows(chips, img_buf, tgt_buf, rows, mean, std, K, what):
     ib, tb = img_buf.cpu().numpy(), tgt_buf.cpu().numpy()
     for r in rows:
@@ -238,7 +165,7 @@ def _check_rows(chips, img_buf, tgt_buf, rows, mean, std, K, what):
 
 
 def _check_fused(op, mean, std, K):
-    for name, ib, tb, stat in _parse_both(op, mean, std, K):
+    for name, ib, tb, stat in _parse_both(op, "norm_onehot_f32", mean, std, K):
         assert not stat.any(), (name, np.nonzero(stat)[0], stat[np.nonzero(stat)[0]])
         _check_rows(op.chips, ib, tb, range(op.si.n), mean, std, K, name)
 
@@ -276,7 +203,7 @@ def test_fused_f32_matches_raw_then_normalise_onehot(dev):
     n = op.si.n
     rb, rt, rst = ops.parse_table(op.si.table, "raw", 4 * op.img_elems, 4 * op.tgt_elems)
     assert not rst[:n].any()
-    for name, ib, tb, stat in _parse_both(op, mean, std, K):
+    for name, ib, tb, stat in _parse_both(op, "norm_onehot_f32", mean, std, K):
         assert not stat.any(), name
         for r, (img, lab) in enumerate(op.chips):
             x = rb[r, :4 * img.size].clone().view(torch.float32).view(img.shape)
@@ -329,7 +256,7 @@ def test_fused_f32_statuses_keep_neighbours_exact(dev):
     good(24, 30)
     op = _Opened(b"".join(recs), chips, dev)
     mean, std = _stats("ordinary", C)
-    for name, ib, tb, stat in _parse_both(op, mean, std, K, img_elems=32 * 32 * C, tgt_elems=32 * 32):
+    for name, ib, tb, stat in _parse_both(op, "norm_onehot_f32", mean, std, K, img_elems=32 * 32 * C, tgt_elems=32 * 32):
         assert list(stat) == want, name
         _check_rows(chips, ib, tb, [r for r, s in enumerate(want) if s == 0], mean, std, K, name)
 
@@ -355,7 +282,7 @@ def test_fused_f32_record_past_2048_tiles(dev):
     op = _Opened(shard, chips, dev, max_records=4)
     assert int(op.si.lens_host[0]) > 2048 * 8192
     mean, std = _stats("inexact_mean", C)
-    for name, ib, tb, stat in _parse_both(op, mean, std, K):
+    for name, ib, tb, stat in _parse_both(op, "norm_onehot_f32", mean, std, K):
         assert list(stat) == [0, 0], name
         _check_rows(chips, ib, tb, [0, 1], mean, std, K, name)
 

@@ -5,8 +5,8 @@ the shared-memory one-hot up to its limit and the generic one-hot beyond it, the
 layouts (payloads starting at every residue mod 16, straddling tiles, longer than a CTA's chunk), per-record statuses,
 and records longer than 2048 CRC tiles (16 MiB) in the CRC, parse and build kernels.
 
-The references are restated here instead of taken from oracle/normalise.py, so that the oracle is checked as well: the
-test_reference_* functions need no GPU.
+The references (tests/_sink_refs.py) are restated instead of taken from oracle/normalise.py, so that the oracle is
+checked as well: the test_reference_* functions need no GPU.
 """
 import functools
 import math
@@ -15,54 +15,13 @@ from fractions import Fraction
 import numpy as np
 import pytest
 
+from _sink_refs import _bits_differ, _parse_both, _record, _round_f32, ref_normalise, ref_one_hot
 from oracle import example_proto as oep
 from oracle import normalise as onorm
 from oracle import tfrecord as otfr
 
 
 # ------------------------------------------------------------------------------------------------ references (CPU)
-def ref_normalise(x, mean, std):
-    """(float32(x) - mean) / std, rounded to float32 after the subtraction and after the division.
-
-    Computed in float64: a float64 result of one +, - or / of float32 operands, rounded to float32, is the correctly
-    rounded float32 result (float64 has at least 2*24 + 2 bits), so this is IEEE float32 arithmetic.  std = 0 gives
-    +-inf or NaN."""
-    x = np.asarray(x)
-    mean = np.asarray(mean, np.float32).astype(np.float64)
-    std = np.asarray(std, np.float32).astype(np.float64)
-    with np.errstate(all="ignore"):
-        d = (x.astype(np.float32).astype(np.float64) - mean).astype(np.float32)
-        return (d.astype(np.float64) / std).astype(np.float32)
-
-
-def ref_one_hot(label, K):
-    """Row k is 1.0 iff the label's value equals k: NaN, +-inf, negative, non-integral and >= K labels give a zero row,
-    -0.0 is class 0."""
-    lab = np.asarray(label)
-    if lab.dtype.kind == "f":
-        return (lab.astype(np.float64)[..., None] == np.arange(K, dtype=np.float64)).astype(np.float32)
-    return (lab.astype(np.int64)[..., None] == np.arange(K, dtype=np.int64)).astype(np.float32)
-
-
-def _round_f32(q, neg=False):
-    """Exact rational -> float32, round to nearest even; subnormals, underflow to a signed zero, overflow to inf."""
-    if q == 0:
-        return np.float32(-0.0 if neg else 0.0)
-    s = -1.0 if q < 0 else 1.0
-    a = abs(q)
-    e = a.numerator.bit_length() - a.denominator.bit_length()
-    while Fraction(2) ** e > a:
-        e -= 1
-    while Fraction(2) ** (e + 1) <= a:
-        e += 1
-    u = max(e - 23, -149)                       # exponent of one unit in the last place (subnormals: 2^-149)
-    m = round(a / Fraction(2) ** u)             # Fraction.__round__: ties to even
-    v = m * Fraction(2) ** u
-    if v >= Fraction(2) ** 128:
-        return np.float32(s * math.inf)
-    return np.float32(math.copysign(float(v), s))
-
-
 def _exact_table(mean, std):
     """(C, 256) float32 quotients of every u8 value, from exact rationals."""
     out = np.empty((len(mean), 256), np.float32)
@@ -75,13 +34,6 @@ def _exact_table(mean, std):
                 neg = (math.copysign(1.0, float(d)) < 0) != (float(s) < 0)
                 out[c, x] = _round_f32(Fraction(float(d)) / Fraction(float(s)), neg)
     return out
-
-
-def _bits_differ(got, want):
-    """Positions where two float32 arrays differ bit for bit; NaN matches NaN whatever the payload."""
-    got, want = np.asarray(got, np.float32), np.asarray(want, np.float32)
-    gn, wn = np.isnan(got), np.isnan(want)
-    return (got.view(np.uint32) != want.view(np.uint32)) & ~(gn & wn) | (gn != wn)
 
 
 REF_MEAN = np.array([100.0, -3.3e4, 127.5, 0.1, 1e6, 100.0, 3.1e7], np.float32)
@@ -137,13 +89,6 @@ def _stats(kind, C):
         if C > 1:
             std[0] = 0.0
     return mean.astype(np.float32), std.astype(np.float32)
-
-
-def _record(img, lab, ident, dims=None):
-    h, w, c = img.shape
-    th, tw = lab.shape
-    h, w, c, th, tw = dims or (h, w, c, th, tw)
-    return otfr.frame(oep.convert_to_example(img, lab, h, w, c, th, tw, ident).SerializeToString())
 
 
 def _chip(rng, h, w, C):
@@ -225,32 +170,8 @@ def _check_rows(op, img_buf, tgt_buf, rows, mean, std, C, K, what):
     _assert_same_bits(got_t, _expect_hot([op.lab[r] for r in rows], K), what + " one-hot")
 
 
-def _parse_both(op, mean, std, K, img_elems=None, tgt_elems=None):
-    """Yield (name, img_buf, tgt_buf, status) from the uniform tile map (parse_shard) and the opened-table map
-    (parse_table, what ShardPipeline runs)."""
-    import torch
-
-    from dl_image_segmentation_b200 import ops
-    n = op.si.n
-    il = op.img_elems if img_elems is None else img_elems
-    tl = op.tgt_elems if tgt_elems is None else tgt_elems
-    dev = op.x[0].device
-    out = None
-    if img_elems is not None:
-        out = (torch.empty((n, il), dtype=torch.float32, device=dev), torch.empty((n, tl * K), dtype=torch.float32, device=dev))
-    ib, tb, st = ops.parse_shard(op.si, "norm_onehot", mean=mean, std=std, num_classes=K, out=out)
-    yield "parse_shard", ib, tb, st[:n].cpu().numpy()
-    del ib, tb
-    # parse_table writes only the rows of the table's records: rows for those are enough
-    out = (torch.empty((n, il), dtype=torch.float32, device=dev), torch.empty((n, tl * K), dtype=torch.float32, device=dev))
-    ib, tb, st = ops.parse_table(op.si.table, "norm_onehot", il, tl, mean=mean, std=std, num_classes=K, out=out)
-    stat = st[:n].cpu().numpy()
-    assert op.si.table.header()[4] == int((stat != 0).sum())
-    yield "parse_table", ib, tb, stat
-
-
 def _check_fused(op, mean, std, C, K):
-    for name, ib, tb, stat in _parse_both(op, mean, std, K):
+    for name, ib, tb, stat in _parse_both(op, "norm_onehot", mean, std, K):
         assert not stat.any(), (name, np.nonzero(stat)[0], stat[np.nonzero(stat)[0]])
         _check_rows(op, ib, tb, range(op.si.n), mean, std, C, K, name)
 
@@ -313,7 +234,7 @@ def test_fused_statuses_keep_neighbours_exact(dev):
     good(40, 50)
     op = _Opened(b"".join(recs), chips, dev)
     mean, std = _stats("ordinary", C)
-    for name, ib, tb, stat in _parse_both(op, mean, std, K, img_elems=64 * 64 * C, tgt_elems=64 * 64):
+    for name, ib, tb, stat in _parse_both(op, "norm_onehot", mean, std, K, img_elems=64 * 64 * C, tgt_elems=64 * 64):
         assert list(stat) == want, name
         _check_rows(op, ib, tb, [r for r, s in enumerate(want) if s == 0], mean, std, C, K, name)
 
@@ -422,7 +343,7 @@ def test_parse_record_past_2048_tiles(dev):
         assert torch.equal(ib[r, :op.x[r].numel()], op.x[r]) and torch.equal(tb[r, :op.lab[r].numel()], op.lab[r])
     del ib, tb
     mean, std = _stats("ordinary", C)
-    for name, ib, tb, stat in _parse_both(op, mean, std, K):
+    for name, ib, tb, stat in _parse_both(op, "norm_onehot", mean, std, K):
         assert list(stat) == [0, 0], name
         _check_rows(op, ib, tb, [0, 1], mean, std, C, K, name)
     del ib, tb
