@@ -231,9 +231,48 @@ static bool dispatch_median(int P, const uint16_t* stack, const uint8_t* valid, 
 // Main loop: one thread per pixel walks `order`, probing one validity byte per scene (coalesced across
 // the warp) and stops at the first valid scene; only that scene's pixel is read.  Filtered-out scenes
 // are never touched, so the kernel moves far fewer bytes than the dense T-deep definition.
-// kStats = element size (1 or 2 bytes) when the exact integer band statistics {n, sum x, sum x^2 lo16, sum x^2 hi} of the
+// kStats = element size (1 or 2 bytes) when the exact integer band statistics {n, sum x, lo, hi} (sum x^2 = lo + 2^16 hi) of the
 // valid output pixels are accumulated in the same pass (B = PB / kStats <= 4 bands); 0 = no statistics.  Fusing them
 // saves the separate statistics pass its re-read of the whole output.
+//
+// The prologue, shared by both mosaic kernels.  max_day == INT32_MAX means no upper bound, as min_day == INT32_MIN
+// already means no lower one.  The distance is exact: |day - ref| < 2^32 fits a uint32_t, and eligibility is kept apart
+// from it, so distances of 2^31 and more still rank by value.  Shared memory (mosaic_smem_bytes): dist[T] uint32,
+// order[T] int32, elig[T] uint8.  Returns the number of eligible scenes; order[0, n) holds them, best first.
+__host__ __device__ constexpr size_t mosaic_smem_bytes(int T) { return (size_t)T * (2 * sizeof(uint32_t) + 1); }
+
+__device__ __forceinline__ int rank_scenes(uint32_t* sm, const int32_t* __restrict__ scene_day, const float* __restrict__ scene_cf,
+                                           int32_t ref_day, int32_t min_day, int32_t max_day, float max_cf, int T) {
+    uint32_t* dist = sm;
+    int32_t* order = reinterpret_cast<int32_t*>(sm + T);
+    uint8_t* elig = reinterpret_cast<uint8_t*>(sm + 2 * T);
+    __shared__ int32_t n_el;
+    for (int t = threadIdx.x; t < T; t += blockDim.x) {
+        const int32_t d = scene_day[t];
+        const float cf = scene_cf[t];
+        bool ok = d >= min_day && (max_day == INT32_MAX || d < max_day);
+        if (!isnan(max_cf)) ok = ok && (cf < max_cf);
+        dist[t] = d >= ref_day ? (uint32_t)d - (uint32_t)ref_day : (uint32_t)ref_day - (uint32_t)d;
+        elig[t] = ok;
+    }
+    if (threadIdx.x == 0) n_el = 0;
+    __syncthreads();
+    for (int t = threadIdx.x; t < T; t += blockDim.x) {
+        if (elig[t]) {
+            const uint32_t k = dist[t];
+            int r = 0;
+            for (int u = 0; u < T; u++) {
+                const uint32_t ku = dist[u];
+                r += elig[u] && (ku < k || (ku == k && u > t));
+            }
+            order[r] = t;
+            atomicAdd(&n_el, 1);
+        }
+    }
+    __syncthreads();
+    return n_el;
+}
+
 template <int PB, int kStats = 0>  // PB = bytes per pixel (all bands), 0 = runtime
 __global__ void __launch_bounds__(256)
 mosaic_kernel(const void* const* __restrict__ stacks, const uint8_t* const* __restrict__ valids,
@@ -241,37 +280,11 @@ mosaic_kernel(const void* const* __restrict__ stacks, const uint8_t* const* __re
               int32_t min_day, int32_t max_day, float max_cf, int T, uint32_t hw, int pb_runtime,
               uint8_t* __restrict__ out, uint8_t* __restrict__ out_mask, int16_t* __restrict__ src_index,
               int32_t* __restrict__ n_eligible, unsigned long long* __restrict__ stats) {
-    extern __shared__ int32_t sm[];  // key[T], order[T], n
-    int32_t* key = sm;
-    int32_t* order = sm + T;
-    __shared__ int32_t n_el;
+    extern __shared__ uint32_t sm[];  // rank_scenes: dist[T], order[T], elig[T]
+    const int32_t* order = reinterpret_cast<const int32_t*>(sm + T);
     const int chip = blockIdx.y;
     const int pb = PB ? PB : pb_runtime;
-    for (int t = threadIdx.x; t < T; t += blockDim.x) {
-        const int32_t d = scene_day[(size_t)chip * T + t];
-        const float cf = scene_cf[(size_t)chip * T + t];
-        bool ok = d >= min_day && d < max_day;
-        if (!isnan(max_cf)) ok = ok && (cf < max_cf);
-        const int64_t diff = (int64_t)d - (int64_t)ref_day;
-        const int64_t ad = diff < 0 ? -diff : diff;
-        key[t] = ok ? (int32_t)(ad > 0x7FFFFFFE ? 0x7FFFFFFE : ad) : -1;
-    }
-    if (threadIdx.x == 0) n_el = 0;
-    __syncthreads();
-    for (int t = threadIdx.x; t < T; t += blockDim.x) {
-        const int32_t k = key[t];
-        if (k >= 0) {
-            int r = 0;
-            for (int u = 0; u < T; u++) {
-                const int32_t ku = key[u];
-                r += (ku >= 0) && (ku < k || (ku == k && u > t));
-            }
-            order[r] = t;
-            atomicAdd(&n_el, 1);
-        }
-    }
-    __syncthreads();
-    const int ne = n_el;
+    const int ne = rank_scenes(sm, scene_day + (size_t)chip * T, scene_cf + (size_t)chip * T, ref_day, min_day, max_day, max_cf, T);
     if (n_eligible && blockIdx.x == 0 && threadIdx.x == 0) n_eligible[chip] = ne;
     const uint8_t* vchip = valids[chip];
     const uint8_t* schip = static_cast<const uint8_t*>(stacks[chip]);
@@ -395,36 +408,10 @@ mosaic_vec8_kernel(const void* const* __restrict__ stacks, const uint8_t* const*
                    const int32_t* __restrict__ scene_day, const float* __restrict__ scene_cf, int32_t ref_day, int32_t min_day,
                    int32_t max_day, float max_cf, int T, uint32_t hw, uint8_t* __restrict__ out, uint8_t* __restrict__ out_mask,
                    int16_t* __restrict__ src_index, int32_t* __restrict__ n_eligible, unsigned long long* __restrict__ stats) {
-    extern __shared__ int32_t sm[];  // key[T], order[T]
-    int32_t* key = sm;
-    int32_t* order = sm + T;
-    __shared__ int32_t n_el;
+    extern __shared__ uint32_t sm[];  // rank_scenes: dist[T], order[T], elig[T]
+    const int32_t* order = reinterpret_cast<const int32_t*>(sm + T);
     const int chip = blockIdx.y;
-    for (int t = threadIdx.x; t < T; t += blockDim.x) {
-        const int32_t d = scene_day[(size_t)chip * T + t];
-        const float cf = scene_cf[(size_t)chip * T + t];
-        bool ok = d >= min_day && d < max_day;
-        if (!isnan(max_cf)) ok = ok && (cf < max_cf);
-        const int64_t diff = (int64_t)d - (int64_t)ref_day;
-        const int64_t ad = diff < 0 ? -diff : diff;
-        key[t] = ok ? (int32_t)(ad > 0x7FFFFFFE ? 0x7FFFFFFE : ad) : -1;
-    }
-    if (threadIdx.x == 0) n_el = 0;
-    __syncthreads();
-    for (int t = threadIdx.x; t < T; t += blockDim.x) {
-        const int32_t k = key[t];
-        if (k >= 0) {
-            int r = 0;
-            for (int u = 0; u < T; u++) {
-                const int32_t ku = key[u];
-                r += (ku >= 0) && (ku < k || (ku == k && u > t));
-            }
-            order[r] = t;
-            atomicAdd(&n_el, 1);
-        }
-    }
-    __syncthreads();
-    const int ne = n_el;
+    const int ne = rank_scenes(sm, scene_day + (size_t)chip * T, scene_cf + (size_t)chip * T, ref_day, min_day, max_day, max_cf, T);
     if (n_eligible && blockIdx.x == 0 && threadIdx.x == 0) n_eligible[chip] = ne;
     const uint8_t* vchip = valids[chip];
     const uint2* schip = static_cast<const uint2*>(stacks[chip]);
@@ -558,7 +545,7 @@ mosaic_vec8_kernel(const void* const* __restrict__ stacks, const uint8_t* const*
     }
 }
 
-// fold the slot copies into the caller's accumulators {n, sum x, sum x^2 & 0xFFFF, sum x^2 >> 16} per band
+// fold the slot copies into the caller's accumulators {n, sum x, lo, hi} per band (sum x^2 = lo + 2^16 hi, b2chips.h)
 __global__ void stats_fold_kernel(const unsigned long long* __restrict__ slots, unsigned long long* __restrict__ stats) {
     const int b = threadIdx.x >> 5, lane = threadIdx.x & 31;       // one warp per band
     unsigned long long n = 0, sv = 0, qv = 0;
@@ -628,8 +615,8 @@ extern "C" int b2_nearest_date_mosaic(b2_ctx* ctx, const void* const* stacks, co
     const unsigned want = (unsigned)((ctx->sm_count * 8 + n_chips - 1) / n_chips);
     if (per_chip > want) per_chip = want > 0 ? want : 1;
     dim3 grid(per_chip, n_chips);
-    const size_t smem = 2 * (size_t)T * sizeof(int32_t);
-    const bool al = reinterpret_cast<uintptr_t>(out) % 16 == 0;  // per-chip stack alignment is the caller's contract
+    const size_t smem = mosaic_smem_bytes(T);     // at most 36 KiB (T <= 4096): no opt-in needed
+    const bool al = reinterpret_cast<uintptr_t>(out) % 16 == 0;  // each stack aligned to its pixel load: the caller's contract
 #define B2_MOSAIC(PBV)                                                                                              \
     mosaic_kernel<PBV><<<grid, 256, smem, s>>>(stacks, valids, scene_day, scene_cf, ref_day, min_day, max_day, max_cf, \
                                                T, hw, pb, static_cast<uint8_t*>(out), out_mask, src_index, n_eligible, nullptr)

@@ -110,7 +110,13 @@ def nearest_date_mosaic(stacks, valids, scene_day, scene_cf, ref_day, min_day=No
     scene_day (N,T) int32; scene_cf (N,T) float32.  Returns out (N,H,W,B), mask (N,H,W) bool,
     src (N,H,W) int16 or None, n_eligible (N,) int32 — all on the device.  stats_acc: optional (B,4) int64
     CUDA tensor; the band statistics of the valid output pixels are accumulated into it in the same pass.
+    Days are int32: a day argument outside that range raises B2Error instead of wrapping to another day.  Each stack
+    must be aligned to its pixel's load width (the pixel size when that is 2, 4, 8 or 16 bytes); with ptr_tables the
+    tables' pointers are the caller's to align.
     """
+    for name, d in (("ref_day", ref_day), ("min_day", min_day), ("max_day", max_day)):
+        if d is not None and not _I32_MIN <= int(d) <= _I32_MAX:
+            raise B2Error("nearest_date_mosaic: %s = %d is outside int32" % (name, int(d)))
     ctx = get_ctx(device)
     if isinstance(stacks, (list, tuple)):
         st = [to_device(s, ctx.device) for s in stacks]
@@ -122,11 +128,15 @@ def nearest_date_mosaic(stacks, valids, scene_day, scene_cf, ref_day, min_day=No
         va = [v_all[i] for i in range(v_all.shape[0])]
     n = len(st)
     T, H, W, B = st[0].shape
+    eb = st[0].element_size()
+    load = B * eb if B * eb in (2, 4, 8, 16) else 1          # the kernels read a whole pixel of these sizes at once
     for s, v in zip(st, va):
         if tuple(s.shape) != (T, H, W, B) or s.dtype != st[0].dtype or not s.is_contiguous():
             raise B2Error("nearest_date_mosaic: all stacks must be contiguous with one shape and dtype")
         if tuple(v.shape) != (T, H, W) or v.dtype != torch.uint8 or not v.is_contiguous():
             raise B2Error("nearest_date_mosaic: valids must be contiguous uint8 (T,H,W)")
+        if ptr_tables is None and s.data_ptr() % load:
+            raise B2Error("nearest_date_mosaic: a stack must be aligned to its %d-byte pixels (address %#x)" % (load, s.data_ptr()))
     day = to_device(np.ascontiguousarray(scene_day, dtype=np.int32) if not isinstance(scene_day, torch.Tensor) else scene_day, ctx.device)
     cf = to_device(np.ascontiguousarray(scene_cf, dtype=np.float32) if not isinstance(scene_cf, torch.Tensor) else scene_cf, ctx.device)
     if tuple(day.shape) != (n, T) or tuple(cf.shape) != (n, T) or day.dtype != torch.int32 or cf.dtype != torch.float32:
@@ -136,7 +146,6 @@ def nearest_date_mosaic(stacks, valids, scene_day, scene_cf, ref_day, min_day=No
         vp = torch.tensor([v.data_ptr() for v in va], dtype=torch.int64).to(ctx.device)
     else:
         sp, vp = ptr_tables
-    eb = st[0].element_size()
     out = torch.empty((n, H, W, B), dtype=st[0].dtype, device=ctx.device)
     mask = torch.empty((n, H, W), dtype=torch.uint8, device=ctx.device)
     src = torch.empty((n, H, W), dtype=torch.int16, device=ctx.device) if want_src else None

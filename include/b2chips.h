@@ -57,14 +57,16 @@ int b2_median_composite_u16(b2_ctx* ctx, const uint16_t* stack_dev, const uint8_
  *   (_descartes_img_chips.py:603-626, key function :461-469).  For each of n_chips chips:
  *   scene t is eligible iff min_day <= scene_day[t] < max_day and (max_cf is NaN or scene_cf[t] < max_cf);
  *   out pixel = stack[t*] with t* the eligible scene, valid at that pixel, of least |scene_day - ref_day|,
- *   ties to the HIGHER scene index (stable descending sort, painted last).  INT32_MIN / INT32_MAX disable
- *   the date bounds.  stacks_dev / valids_dev: device arrays of n_chips device pointers to (T,H,W,B) and
- *   (T,H,W) u8.  scene_day_dev / scene_cf_dev: (n_chips,T).  out (n_chips,H,W,B) same element type;
+ *   ties to the HIGHER scene index (stable descending sort, painted last).  The distance is exact over the whole
+ *   int32 range (up to 2^32 - 1).  min_day = INT32_MIN means no lower bound and max_day = INT32_MAX no upper bound:
+ *   a scene dated INT32_MAX is then eligible.  stacks_dev / valids_dev: device arrays of n_chips device pointers to
+ *   (T,H,W,B) and (T,H,W) u8; each stack aligned to its pixel size B * elem_bytes when that is 2, 4, 8 or 16.
+ *   scene_day_dev / scene_cf_dev: (n_chips,T).  out (n_chips,H,W,B) same element type;
  *   out_mask (n_chips,H,W) u8 = 1 where no valid scene (out = 0); src_index (n_chips,H,W) int16 or NULL;
  *   n_eligible (n_chips) int32 or NULL — 0 means the reference returns None (:614-615).
  *   stats_acc (B,4) uint64 or NULL: the exact band statistics of b2_band_stats over the VALID output pixels are
  *   accumulated in the same pass (uint8 / uint16 chips of at most 4 bands), so configs[4]'s per-band mean / std cost
- *   no second read of the output.
+ *   no second read of the output.  The counters are those of b2_band_stats, split the same way.
  */
 int b2_nearest_date_mosaic(b2_ctx* ctx, const void* const* stacks_dev, const uint8_t* const* valids_dev,
                            const int32_t* scene_day_dev, const float* scene_cf_dev,
@@ -83,8 +85,10 @@ int b2_normalise_onehot(b2_ctx* ctx, const void* img_dev, int img_dtype, const v
                         const float* mean_dev, const float* std_dev, uint64_t n_pixels, int C, int K,
                         float* img_out_dev, float* onehot_out_dev, b2_stream stream);
 
-/* Exact integer per-band statistics: acc (B,4) uint64 += { n, sum x, sum (x*x & 0xFFFF), sum (x*x >> 16) } over
- *   pixels with valid != 0 (valid NULL = all).  dtype B2_U8 or B2_U16.  Accumulates (caller zeroes acc). */
+/* Exact integer per-band statistics over pixels with valid != 0 (valid NULL = all): acc (B,4) uint64 += { n, sum x,
+ *   lo, hi } with sum x*x = lo + 2^16 * hi.  The kernels split partial sums of x*x (per CTA or per slot, not per pixel)
+ *   into their low 16 bits and the rest, so lo and hi on their own depend on the launch: only lo + 2^16 * hi is
+ *   defined.  dtype B2_U8 or B2_U16.  Accumulates (caller zeroes acc). */
 int b2_band_stats(b2_ctx* ctx, const void* img_dev, int dtype, const uint8_t* valid_dev, uint64_t n_pixels, int B,
                   uint64_t* acc_dev, b2_stream stream);
 
