@@ -28,6 +28,8 @@
 //   * when the run ends, one GF(2)[x] multiplication by x^(-128 i) aligns thread i's state with the tile end,
 //     the states XOR together, and one more multiplication by a tabulated power of x moves the partial to the
 //     end of the record.  The 0xFFFFFFFF init is XORed into the first four data bytes.
+#include <type_traits>
+
 #include "tfrecord_common.cuh"
 
 #ifndef B2_WAIT_HINT_NS
@@ -55,9 +57,17 @@ constexpr int kHotBlocks = B2_HOT_BLOCKS;            // blocks per warp: the bul
 // waiting for a tile with two).
 // The two normalise + one-hot modes (uint8 BytesList and float32 FloatList payloads) share every resource decision.
 __host__ __device__ constexpr bool is_norm(int mode) { return mode == B2_SINK_NORM_ONEHOT || mode == B2_SINK_NORM_ONEHOT_F32; }
+// The two statistics modes read the same payloads and write nothing but per-CTA counters: they take the CRC-only pass's
+// resources (four buffers, five CTAs per SM).
+__host__ __device__ constexpr bool is_stats(int mode) { return mode == B2_SINK_STATS || mode == B2_SINK_STATS_F32; }
 // bytes per payload element: 1 for BytesList, 4 for packed FloatList
-__host__ __device__ constexpr uint32_t elem_bytes(int mode) { return mode == B2_SINK_NORM_ONEHOT_F32 ? 4u : 1u; }
+__host__ __device__ constexpr uint32_t elem_bytes(int mode) {
+    return mode == B2_SINK_NORM_ONEHOT_F32 || mode == B2_SINK_STATS_F32 ? 4u : 1u;
+}
 __host__ __device__ constexpr int stages_for(int mode) { return is_norm(mode) ? B2_STAGES : 4; }
+// Resident CTAs per SM.  The statistics modes keep per-thread partial sums for four bands, which do not fit the 40
+// registers of five CTAs (ptxas spills); four leave 56.
+__host__ __device__ constexpr int ctas_per_sm(int mode) { return is_norm(mode) ? 3 : is_stats(mode) ? 4 : 5; }
 constexpr int kMaxStages = 4;
 constexpr int kConsumerWarps = kTileThreads / 32;
 constexpr int kCtaThreads = kTileThreads + 32;   // 8 consumer warps + 1 producer warp
@@ -137,12 +147,13 @@ struct RecCache {
 // status) cannot disagree.  0: they run.  2: the index refused the record, or it does not fit the normalise + one-hot
 // template: both payloads BytesList (NORM_ONEHOT) or packed FloatList (NORM_ONEHOT_F32), the sink's band count, payloads
 // as long as the record's dimensions say (else the reference's decode_raw / reshape raises).  3: a payload does not fit
-// its output row, or has 2^31 elements or more (the sinks index elements with 32 bits).
+// its output row, or has 2^31 elements or more (the sinks index elements with 32 bits).  The statistics modes apply the
+// same template (STATS as NORM_ONEHOT, STATS_F32 as NORM_ONEHOT_F32) and the element limit; they have no rows to fit.
 template <int kMode>
 __device__ __forceinline__ int32_t sink_status(const b2_example_index* ix, const b2_parse_sink& sink) {
     if (ix->status != 0) return 2;
     if (kMode == B2_SINK_RAW) return ix->img_len <= sink.img_stride && ix->tgt_len <= sink.tgt_stride ? 0 : 3;
-    constexpr int kKind = kMode == B2_SINK_NORM_ONEHOT_F32 ? 2 : 1;
+    constexpr int kKind = elem_bytes(kMode) == 4 ? 2 : 1;
     constexpr uint64_t kEB = elem_bytes(kMode);
     const int C = sink.channels;
     if (ix->img_kind != kKind || ix->tgt_kind != kKind || ix->channels != C) return 2;
@@ -150,6 +161,7 @@ __device__ __forceinline__ int32_t sink_status(const b2_example_index* ix, const
     const uint64_t hw = (uint64_t)ix->height * (uint64_t)ix->width;   // < 2^62; C <= 64 (check_sink)
     const uint64_t thw = (uint64_t)ix->tgt_height * (uint64_t)ix->tgt_width;
     if (hw >= (1ull << 48) || hw * (uint64_t)C * kEB != ix->img_len || thw * kEB != ix->tgt_len) return 2;
+    if (is_stats(kMode)) return hw * (uint64_t)C < (1ull << 31) && thw < (1ull << 31) ? 0 : 3;
     const uint64_t ie = hw * (uint64_t)C, te = thw, K = (uint64_t)sink.num_classes;
     return ie * 4 <= sink.img_stride && te * K * 4 <= sink.tgt_stride && ie < (1ull << 31) && te * K < (1ull << 31) ? 0 : 3;
 }
@@ -424,6 +436,140 @@ __device__ __forceinline__ void sink_onehot_generic(const uint8_t* buf8, const u
     }
 }
 
+// ---------------------------------------------------------------- statistics sinks (STATS, STATS_F32)
+// Per-CTA counters in dynamic shared memory after the tile ring: per band { elements, sum x, sum x^2, excluded }, then the
+// 257 label bins as 32-bit low and high words (a 64-bit shared atomic add is a compare-and-swap loop on sm_100; the
+// label bins take one atomic per distinct label of a warp step).  Flushed to the caller's counters once, when the
+// consumers leave the tile loop.
+constexpr int kStatWords = 4 * 64 + 257;   // 64-bit words
+struct StatSmem {
+    unsigned long long* cnt;    // [64] elements of the band in the records counted (excluded ones included)
+    unsigned long long* sum;    // [64] two's complement
+    unsigned long long* sq;     // [64]
+    unsigned long long* exc;    // [64] STATS_F32 values that are not integers in [-2^16, 2^16)
+    uint32_t* hist_lo;          // [257]
+    uint32_t* hist_hi;          // [257] carries out of hist_lo
+};
+
+// image -> per-band sums.  Thread tid < S takes the groups g (elements [4g, 4g + 4) from the payload start) with
+// g = tid mod S: C divides 4 S, so element 4g + k is always of band (4 tid + k) mod C, wherever the tile starts.  A group
+// is counted by the tile holding its first byte (its last bytes may sit in the halo); elements past the payload end are
+// skipped.  The tile holding the payload's first byte also adds each band's element count.  Warp-uniform (callers check
+// tile_holds).
+// The partials are folded into the shared counters at the end of every tile: kept across tiles they cost the registers of
+// four CTAs per SM (ptxas spills).  Per tile a uint8 thread adds at most 10 elements per band (S >= 215), so after the
+// 32-lane reduction sum x < 2^17 and sum x^2 < 2^25 fit 32 bits; float squares reach 2^32 and take 64.
+template <uint32_t kEB>
+__device__ __forceinline__ void sink_image_stats(const uint32_t* buf32, uint64_t ts, uint64_t te, uint64_t po, uint64_t len,
+                                                 uint32_t S, uint32_t m, int C, const StatSmem& sm) {
+    using Sq = typename std::conditional<kEB == 1, uint32_t, unsigned long long>::type;
+    const uint32_t tid = threadIdx.x, lane = tid & 31;
+    const uint32_t pl = (uint32_t)(len / kEB);   // elements
+    if (po >= ts && tid < (uint32_t)C)
+        atomicAdd(&sm.cnt[tid], (unsigned long long)(pl / (uint32_t)C + (tid < pl % (uint32_t)C ? 1u : 0u)));
+    int32_t sum[4] = {0, 0, 0, 0};
+    Sq sq[4] = {0, 0, 0, 0};
+    if (tid < S) {
+        const uint64_t lo = po > ts ? po : ts, hi = (po + (uint64_t)pl * kEB < te) ? po + (uint64_t)pl * kEB : te;
+        const uint32_t g_lo = (uint32_t)((lo - po + 4 * kEB - 1) / (4 * kEB)), g_hi = (uint32_t)((hi - po + 4 * kEB - 1) / (4 * kEB));
+        const uint32_t base = (uint32_t)(po - ts);
+        for (uint32_t g = g_lo + (tid + S - g_lo % S) % S; g < g_hi; g += S) {
+            const bool whole = 4 * g + 4 <= pl;
+            if constexpr (kEB == 1) {
+                const uint32_t x = smem_u32_unaligned(buf32, base + 4 * g);
+#pragma unroll
+                for (int k = 0; k < 4; k++) {
+                    const uint32_t v = (whole || 4 * g + k < pl) ? (x >> (8 * k)) & 0xFFu : 0u;
+                    sum[k] += (int32_t)v;
+                    sq[k] += v * v;
+                }
+            } else {
+#pragma unroll
+                for (int k = 0; k < 4; k++) {
+                    if (!whole && 4 * g + k >= pl) continue;
+                    const float f = __uint_as_float(smem_u32_unaligned(buf32, base + 16 * g + 4 * k));
+                    if (f >= -65536.0f && f < 65536.0f && f == truncf(f)) {   // NaN fails the comparisons
+                        const int32_t v = (int32_t)f;
+                        const uint32_t av = (uint32_t)(v < 0 ? -v : v);
+                        sum[k] += v;
+                        sq[k] += (unsigned long long)av * av;
+                    } else {
+                        atomicAdd(&sm.exc[(4 * tid + k) % (uint32_t)C], 1ull);   // out of scope (float-valued chips)
+                    }
+                }
+            }
+        }
+    }
+    // lanes l and l' of a warp hold the same band for each k exactly when l = l' mod m (m = C / gcd(C, 4)): reduce over
+    // those lanes, then lanes l < m add their bands' totals (threads at or past S hold zeros)
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        int32_t s = sum[k];
+        Sq q = sq[k];
+        for (uint32_t off = m; off < 32; off <<= 1) {
+            const int32_t s2 = __shfl_down_sync(0xffffffffu, s, off);
+            const Sq q2 = __shfl_down_sync(0xffffffffu, q, off);
+            if (lane + off < 32) {
+                s += s2;
+                q += q2;
+            }
+        }
+        if (lane < m) {
+            const uint32_t band = (4 * tid + k) % (uint32_t)C;
+            if (s) atomicAdd(&sm.sum[band], (unsigned long long)(long long)s);
+            if (q) atomicAdd(&sm.sq[band], (unsigned long long)q);
+        }
+    }
+}
+
+// a float label's bin: v for a value equal to an integer v in 0..255 (-0.0 is 0), 256 for anything else (NaN included)
+__device__ __forceinline__ uint32_t float_label_bin(uint32_t word) {
+    const float f = __uint_as_float(word);
+    return f >= 0.0f && f <= 255.0f && f == truncf(f) ? (uint32_t)f : 256u;
+}
+
+// Add weight to bin `key` for every lane of the warp, one shared atomic per distinct key: label rasters are spatially
+// smooth, so a warp's labels usually share a bin and per-lane atomics would serialise on it.  kNoBin: nothing to add.
+constexpr uint32_t kNoBin = 0xFFFFFFFFu;
+__device__ __forceinline__ void hist_add(const StatSmem& sm, uint32_t key, uint32_t weight) {
+    const uint32_t peers = __match_any_sync(0xffffffffu, key);
+    if (key != kNoBin && (threadIdx.x & 31) == (uint32_t)(__ffs(peers) - 1)) {
+        const uint32_t add = weight * __popc(peers);
+        if (atomicAdd(&sm.hist_lo[key], add) > 0xFFFFFFFFu - add) atomicAdd(&sm.hist_hi[key], 1u);
+    }
+}
+
+// label -> histogram.  Unit j = 4 labels (uint8) or 1 label (float32), owned by the tile holding its first byte; a warp
+// takes 32 consecutive units per step (warp-uniform loop: every lane reaches the match).  A uint8 unit whose four labels
+// are equal counts once with weight 4 when the whole warp's units are.
+template <uint32_t kEB>
+__device__ __forceinline__ void sink_label_hist(const uint32_t* buf32, uint64_t ts, uint64_t te, uint64_t po, uint64_t len,
+                                                const StatSmem& sm) {
+    constexpr uint32_t kU = kEB == 1 ? 4 : 1;   // labels per unit
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t pl = (uint32_t)(len / kEB);   // labels
+    const uint64_t lo = po > ts ? po : ts, hi = (po + (uint64_t)pl * kEB < te) ? po + (uint64_t)pl * kEB : te;
+    const uint32_t j_lo = (uint32_t)((lo - po + kU * kEB - 1) / (kU * kEB)), j_hi = (uint32_t)((hi - po + kU * kEB - 1) / (kU * kEB));
+    const uint32_t base = (uint32_t)(po - ts);
+    for (uint32_t j0 = j_lo + 32 * warp; j0 < j_hi; j0 += kTileThreads) {
+        const uint32_t j = j0 + lane;
+        const bool own = j < j_hi;
+        const uint32_t x = own ? smem_u32_unaligned(buf32, base + kU * kEB * j) : 0u;
+        if constexpr (kEB == 1) {
+            const bool same = own && kU * j + kU <= pl && x == __byte_perm(x, 0, 0);
+            if (__all_sync(0xffffffffu, same || !own)) {
+                hist_add(sm, own ? (x & 0xFFu) : kNoBin, 4);
+            } else {
+#pragma unroll
+                for (uint32_t k = 0; k < kU; k++)
+                    hist_add(sm, own && kU * j + k < pl ? (x >> (8 * k)) & 0xFFu : kNoBin, 1);
+            }
+        } else {
+            hist_add(sm, own ? float_label_bin(x) : kNoBin, 1);
+        }
+    }
+}
+
 struct RecRef {   // what finalize_record needs to know about the record
     uint32_t r, nt;
     uint64_t d0, d1;
@@ -543,7 +689,7 @@ __device__ __forceinline__ void run_flush(const ParseArgs& a, Run& run, uint32_t
 // CONSUMERS (CRC, payload sinks).  They meet only through mbarriers: full[s] flips when tile s has landed, empty[s]
 // when all eight consumer warps are done with it — there is no __syncthreads in the steady state.
 template <int kMode, bool kProf = false>
-__global__ void __launch_bounds__(kCtaThreads, is_norm(kMode) ? 3 : 5)
+__global__ void __launch_bounds__(kCtaThreads, ctas_per_sm(kMode))
 fused_parse_kernel(const ParseArgs a) {
     constexpr int kStages = stages_for(kMode);
     static_assert(kStages <= kMaxStages && kRunSlots > kStages, "ring sizes");
@@ -561,8 +707,13 @@ fused_parse_kernel(const ParseArgs a) {
     const int C = a.sink.channels, K = a.sink.num_classes;
     const bool use_hot = K <= kHotMaxK;
     float* hot_all = reinterpret_cast<float*>(dyn + kStages * kBufBytes);
+    unsigned long long* stat_all = reinterpret_cast<unsigned long long*>(dyn + kStages * kBufBytes);
+    const StatSmem sm{stat_all, stat_all + 64, stat_all + 128, stat_all + 192, reinterpret_cast<uint32_t*>(stat_all + 256),
+                      reinterpret_cast<uint32_t*>(stat_all + 256) + 257};
 
     if (want_crc) load_crc_tables(&cs, a.tab);
+    if (is_stats(kMode))
+        for (int i = tid; i < kStatWords; i += kCtaThreads) stat_all[i] = 0ull;
     if (is_norm(kMode)) {
         if (tid == 0) s_exact_div = 0;
         for (int c = tid; c < C; c += kCtaThreads) {
@@ -630,16 +781,18 @@ fused_parse_kernel(const ParseArgs a) {
     const bool exact_div = kMode == B2_SINK_NORM_ONEHOT && s_exact_div != 0;
     // image loop stride: the largest S <= 256 with 4 S a multiple of C, so that a thread's four bytes always fall on
     // the same four bands and their constants stay in registers
-    uint32_t img_S = kTileThreads;
-    if (is_norm(kMode)) {
+    uint32_t img_S = kTileThreads, img_m = 1;
+    if (is_norm(kMode) || is_stats(kMode)) {
         const uint32_t m = (C % 4 == 0) ? C / 4 : ((C % 2 == 0) ? C / 2 : C);
         img_S = kTileThreads - (kTileThreads % m);
+        img_m = m;
     }
     uint32_t s = 0;                       // running CRC state of this thread
     Run run;
     run.open = false;
     const uint32_t hot_dummy = kHotLabels * K;
     HotBlocks hot{hot_all + warp * kHotBlocks * (kHotLabels * K + 4), hot_dummy, hot_dummy, hot_dummy, hot_dummy, 0};
+    constexpr uint32_t kEB = elem_bytes(kMode);
     PROF_BEGIN();
 
     for (uint32_t it = 0;; it++) {
@@ -677,7 +830,6 @@ fused_parse_kernel(const ParseArgs a) {
                     sink_raw(buf32, buf8, ts, te, j.tgt_off, j.tgt_len, static_cast<uint8_t*>(a.sink.tgt_out) + (uint64_t)(j.r & a.row_mask) * a.sink.tgt_stride);
             }
             if (is_norm(kMode) && (flags & 2)) {
-                constexpr uint32_t kEB = elem_bytes(kMode);
                 if (a.sink.img_out && (uint32_t)tid < img_S && tile_holds(ts, te, j.img_off, j.img_len))
                     sink_image<kEB>(buf32, ts, te, j.img_off, j.img_len,
                                     reinterpret_cast<float*>(static_cast<uint8_t*>(a.sink.img_out) + (uint64_t)(j.r & a.row_mask) * a.sink.img_stride),
@@ -690,12 +842,37 @@ fused_parse_kernel(const ParseArgs a) {
                 }
                 PROF_MARK(3);
             }
+            if (is_stats(kMode) && (flags & 2)) {
+                if (a.sink.img_out && tile_holds(ts, te, j.img_off, j.img_len))
+                    sink_image_stats<kEB>(buf32, ts, te, j.img_off, j.img_len, img_S, img_m, C, sm);
+                if (a.sink.tgt_out && tile_holds(ts, te, j.tgt_off, j.tgt_len))
+                    sink_label_hist<kEB>(buf32, ts, te, j.tgt_off, j.tgt_len, sm);
+            }
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(&empty[slot]);   // this warp is done with the buffer and its job
         PROF_MARK(4);
     }
     if (is_norm(kMode) && lane == 0) bulk_wait_read<0>();   // shared memory must outlive the bulk stores
+    if (is_stats(kMode)) {
+        // The producer warp has returned: the eight consumer warps meet on named barrier 1, then add the CTA's counters
+        // to the caller's, one 64-bit atomic per non-zero word (acc[c] = { n, sum x, sum x^2 lo, sum x^2 hi, excluded }).
+        asm volatile("bar.sync 1, %0;" ::"n"(kTileThreads) : "memory");
+        unsigned long long* acc = static_cast<unsigned long long*>(a.sink.img_out);
+        if (acc && tid < C) {
+            const unsigned long long sq = sm.sq[tid];
+            const unsigned long long v[5] = {sm.cnt[tid] - sm.exc[tid], sm.sum[tid], sq & 0xFFFFull, sq >> 16, sm.exc[tid]};
+#pragma unroll
+            for (int k = 0; k < 5; k++)
+                if (v[k]) atomicAdd(&acc[5 * tid + k], v[k]);
+        }
+        unsigned long long* hist = static_cast<unsigned long long*>(a.sink.tgt_out);
+        if (hist)
+            for (int b = tid; b < 257; b += kTileThreads) {
+                const unsigned long long v = ((unsigned long long)sm.hist_hi[b] << 32) | sm.hist_lo[b];
+                if (v) atomicAdd(&hist[b], v);
+            }
+    }
     PROF_END();
 }
 
@@ -709,7 +886,8 @@ bool g_smem_ready[64];   // per device: the kernels' shared-memory opt-ins are s
 
 constexpr size_t dyn_bytes(int mode, int K) {
     return (size_t)stages_for(mode) * kBufBytes +
-           (is_norm(mode) && K <= kHotMaxK ? (size_t)(kTileThreads / 32) * kHotBlocks * (kHotLabels * K + 4) * sizeof(float) : 0);
+           (is_norm(mode) && K <= kHotMaxK ? (size_t)(kTileThreads / 32) * kHotBlocks * (kHotLabels * K + 4) * sizeof(float) : 0) +
+           (is_stats(mode) ? (size_t)kStatWords * sizeof(unsigned long long) : 0);
 }
 // The one-hot blocks at K = kHotMaxK need 145 KiB; the kernel's static shared memory (~9 KiB, ptxas -v) comes on top, and
 // both must fit the 227 KiB a block may opt into on sm_100.
@@ -731,25 +909,26 @@ int set_dyn_smem(F* kernel, size_t dyn, int device) {
 using ParseKernel = void (*)(const ParseArgs);
 ParseKernel fused_kernel(int mode, bool prof) {
     const ParseKernel k[] = {fused_parse_kernel<B2_SINK_NONE>, fused_parse_kernel<B2_SINK_RAW>, fused_parse_kernel<B2_SINK_NORM_ONEHOT>,
-                             fused_parse_kernel<B2_SINK_NORM_ONEHOT_F32>};
+                             fused_parse_kernel<B2_SINK_NORM_ONEHOT_F32>, fused_parse_kernel<B2_SINK_STATS>,
+                             fused_parse_kernel<B2_SINK_STATS_F32>};
     if (mode == B2_SINK_NORM_ONEHOT && prof) return fused_parse_kernel<B2_SINK_NORM_ONEHOT, true>;
-    return mode >= B2_SINK_NONE && mode <= B2_SINK_NORM_ONEHOT_F32 ? k[mode] : nullptr;
+    return mode >= B2_SINK_NONE && mode <= B2_SINK_STATS_F32 ? k[mode] : nullptr;
 }
 
 int launch_fused(b2_ctx* ctx, const ParseArgs& pa, uint64_t max_tiles, cudaStream_t s) {
     if (!g_smem_ready[ctx->device & 63]) {
         // opt-in ceilings of every kernel; the normalise + one-hot modes: what their largest launch (K = kHotMaxK) asks
         // for.  A ceiling only: occupancy follows each launch's actual request.
-        for (int mode = B2_SINK_NONE; mode <= B2_SINK_NORM_ONEHOT_F32; mode++)
+        for (int mode = B2_SINK_NONE; mode <= B2_SINK_STATS_F32; mode++)
             for (int prof = 0; prof <= (mode == B2_SINK_NORM_ONEHOT); prof++)   // only NORM_ONEHOT has a profiling twin
                 if (int e = set_dyn_smem(fused_kernel(mode, prof), is_norm(mode) ? kNormDynMax : 96 * 1024, ctx->device)) return e;
         g_smem_ready[ctx->device & 63] = true;
     }
     const ParseKernel kernel = fused_kernel(pa.sink.mode, pa.prof != nullptr);
     B2_REQUIRE(kernel, "fused parse: no kernel for this sink mode");
-    // persistent grid: as many CTAs as fit on the GPU at once (4 per SM), never more than there are chunks
+    // persistent grid: as many CTAs as fit on the GPU at once, never more than there are chunks
     const uint64_t chunks = (max_tiles + pa.q - 1) / pa.q;
-    const uint64_t resident = (uint64_t)ctx->sm_count * (is_norm(pa.sink.mode) ? 3 : 5);
+    const uint64_t resident = (uint64_t)ctx->sm_count * ctas_per_sm(pa.sink.mode);
     const unsigned grid = (unsigned)(chunks < resident ? chunks : resident);
     kernel<<<grid, kCtaThreads, dyn_bytes(pa.sink.mode, pa.sink.num_classes), s>>>(pa);
     ctx->launches++;
@@ -765,6 +944,12 @@ int check_sink(const b2_parse_sink* sink, const char* who) {
         B2_REQUIRE((reinterpret_cast<uintptr_t>(sink->img_out) & 15) == 0 && (sink->img_stride & 15) == 0 &&
                    (reinterpret_cast<uintptr_t>(sink->tgt_out) & 15) == 0 && (sink->tgt_stride & 15) == 0,
                    std::string(who) + m + " outputs and strides must be 16-byte aligned");
+    } else if (is_stats(sink->mode)) {
+        const std::string m = sink->mode == B2_SINK_STATS ? ": STATS" : ": STATS_F32";
+        B2_REQUIRE(sink->channels >= 1 && sink->channels <= 64, std::string(who) + m + " needs 1..64 channels");
+        B2_REQUIRE((reinterpret_cast<uintptr_t>(sink->img_out) & 7) == 0 && (reinterpret_cast<uintptr_t>(sink->tgt_out) & 7) == 0 &&
+                       sink->img_stride == 0 && sink->tgt_stride == 0,
+                   std::string(who) + m + " counters must be 8-byte aligned, with strides 0");
     } else {
         B2_REQUIRE(sink->mode == B2_SINK_NONE || sink->mode == B2_SINK_RAW, std::string(who) + ": unknown sink mode");
     }

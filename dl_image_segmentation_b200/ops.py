@@ -322,9 +322,13 @@ class ShardTable:
             raise B2Error("%s holds more than max_records=%d records" % (what, self.max_records))
         if st != 0:
             raise DataLossError("corrupted record #%d in %s (bad frame or length CRC)" % (n, what))
-        if bad:
-            raise DataLossError("%d record(s) of %s failed the data CRC or the feature template" % (bad, what))
+        _check_bad_records(bad, what)
         return n
+
+
+def _check_bad_records(bad, what):
+    if bad:
+        raise DataLossError("%d record(s) of %s failed the data CRC or the feature template" % (bad, what))
 
 
 def open_shard_async(data, device=None, max_records=4096, nbytes=None, table=None):
@@ -368,7 +372,9 @@ def _align16(x):
 
 # sink mode -> (b2_parse_sink.mode, payload bytes per element of the normalise / one-hot modes, 0 for the others)
 _SINK_MODES = {"none": (_lib.SINK_NONE, 0), "raw": (_lib.SINK_RAW, 0), "norm_onehot": (_lib.SINK_NORM_ONEHOT, 1),
-               "norm_onehot_f32": (_lib.SINK_NORM_ONEHOT_F32, 4)}
+               "norm_onehot_f32": (_lib.SINK_NORM_ONEHOT_F32, 4), "stats": (_lib.SINK_STATS, 0),
+               "stats_f32": (_lib.SINK_STATS_F32, 0)}
+_STATS_MODES = ("stats", "stats_f32")
 
 
 def _sink_mode(mode):
@@ -386,14 +392,31 @@ def _float_rows(img_elems, tgt_elems, num_classes):
     return il, tl * K
 
 
+def _stats_out(out, channels, device):
+    """The (acc (C,5) int64, hist (257,) int64) counters of the statistics modes: zeroed new ones, or the caller's (either
+    may be None: the kernel then skips it)."""
+    if out is not None:
+        acc, hist = out
+        if acc is not None and (acc.dtype != torch.int64 or tuple(acc.shape) != (channels, 5) or not acc.is_contiguous()):
+            raise B2Error("statistics counters: acc must be a contiguous (%d, 5) int64 tensor" % channels)
+        if hist is not None and (hist.dtype != torch.int64 or tuple(hist.shape) != (257,) or not hist.is_contiguous()):
+            raise B2Error("statistics counters: hist must be a contiguous (257,) int64 tensor")
+        return acc, hist
+    return (torch.zeros((channels, 5), dtype=torch.int64, device=device),
+            torch.zeros((257,), dtype=torch.int64, device=device))
+
+
 def parse_shard(si: ShardIndex, mode, verify_crc=True, mean=None, std=None, num_classes=None, first=0, count=None,
-                out=None):
+                out=None, channels=None):
     """Run the fused parse kernel over records [first, first+count).  Returns (img_buf, tgt_buf, status_dev).
 
     mode 'raw': img_buf (count, img_stride) uint8 holding each record's payload bytes as stored;
     mode 'norm_onehot': uint8 BytesList records -> img_buf (count, img_len) float32, tgt_buf (count, tgt_len*K) float32;
     mode 'norm_onehot_f32': packed float32 FloatList records (the higher-dtype array format) -> the same outputs, with
     img_len / tgt_len counted in float elements (the index's byte lengths / 4);
+    mode 'stats' (records as 'norm_onehot') / 'stats_f32' (records as 'norm_onehot_f32'): img_buf = acc (channels, 5)
+    int64 per-band { n, sum x, sum x^2 lo, sum x^2 hi, excluded }, tgt_buf = hist (257,) int64 label bins (b2chips.h
+    B2_SINK_STATS); both accumulate into out=(acc, hist) when it is given.  Defined only if every status is 0;
     mode 'none': CRC verification only.
     """
     ctx = get_ctx(si.shard.device)
@@ -403,7 +426,9 @@ def parse_shard(si: ShardIndex, mode, verify_crc=True, mean=None, std=None, num_
     _, esz = _sink_mode(mode)
     idx = si.index[first:first + count] if si.index is not None else None
     img_buf = tgt_buf = None
-    if mode == "raw":
+    if mode in _STATS_MODES:
+        img_buf, tgt_buf = _stats_out(out, channels, ctx.device)
+    elif mode == "raw":
         istr, tstr = _align16(max(1, idx["img_len"].max())), _align16(max(1, idx["tgt_len"].max()))
         img_buf, tgt_buf = out if out is not None else (
             torch.empty((count, istr), dtype=torch.uint8, device=ctx.device),
@@ -415,7 +440,7 @@ def parse_shard(si: ShardIndex, mode, verify_crc=True, mean=None, std=None, num_
         img_buf, tgt_buf = out if out is not None else (
             torch.empty((count, il), dtype=torch.float32, device=ctx.device),
             torch.empty((count, tl), dtype=torch.float32, device=ctx.device))
-    sink = _make_sink(mode, verify_crc, img_buf, tgt_buf, mean, std, num_classes)
+    sink = _make_sink(mode, verify_crc, img_buf, tgt_buf, mean, std, num_classes, channels)
     status = torch.empty((count,), dtype=torch.int32, device=ctx.device)
     isz = ctypes.sizeof(_lib.ExampleIndex)
     index_ptr = ctypes.c_void_p(si.index_dev.data_ptr() + first * isz) if si.index_dev is not None else None
@@ -492,12 +517,17 @@ def build_records(items, device=None):
     return plan.launch(), plan.offsets, plan.total
 
 
-def _make_sink(mode, verify_crc, img_buf, tgt_buf, mean=None, std=None, num_classes=None):
-    """The b2_parse_sink for a mode; mean / std are float32 device tensors (their length is the band count)."""
+def _make_sink(mode, verify_crc, img_buf, tgt_buf, mean=None, std=None, num_classes=None, channels=None):
+    """The b2_parse_sink for a mode; mean / std are float32 device tensors (their length is the band count).  The
+    statistics modes take their band count from channels and their counters (or None) in img_buf / tgt_buf."""
     sink = _lib.ParseSink()
     sink.mode, esz = _sink_mode(mode)
     sink.verify_crc = 1 if verify_crc else 0
-    if mode == "raw":
+    if mode in _STATS_MODES:
+        sink.img_out = img_buf.data_ptr() if img_buf is not None else None
+        sink.tgt_out = tgt_buf.data_ptr() if tgt_buf is not None else None
+        sink.channels = int(channels)
+    elif mode == "raw":
         sink.img_out, sink.img_stride = img_buf.data_ptr(), img_buf.stride(0) * img_buf.element_size()
         sink.tgt_out, sink.tgt_stride = tgt_buf.data_ptr(), tgt_buf.stride(0) * tgt_buf.element_size()
     elif esz:
@@ -510,13 +540,15 @@ def _make_sink(mode, verify_crc, img_buf, tgt_buf, mean=None, std=None, num_clas
 
 
 def parse_table(st: ShardTable, mode, img_elems=0, tgt_elems=0, verify_crc=True, mean=None, std=None, num_classes=None,
-                out=None, status=None, want_img=True, want_tgt=True):
+                out=None, status=None, want_img=True, want_tgt=True, channels=None):
     """Enqueue the fused pass over EVERY record of an opened shard; no host synchronisation.
 
     The record count lives on the device, so outputs are sized for st.max_records rows:
     mode 'raw': (max_records, img_elems) / (max_records, tgt_elems) uint8 rows of payload bytes as stored;
     mode 'norm_onehot' (uint8 BytesList records) and 'norm_onehot_f32' (packed float32 FloatList records):
     (max_records, img_elems) float32 and (max_records, tgt_elems*K) float32, sizes in elements (H*W*C and H*W);
+    mode 'stats' / 'stats_f32': the (acc, hist) counters of parse_shard, added to out=(acc, hist) when given
+    (img_elems / tgt_elems are not used);
     mode 'none': CRC verification only.  A payload longer than its row gives status 3.
     Returns (img_buf, tgt_buf, status_dev[max_records]); rows / entries >= the record count are untouched.
     """
@@ -524,7 +556,9 @@ def parse_table(st: ShardTable, mode, img_elems=0, tgt_elems=0, verify_crc=True,
     cap = st.max_records
     _, esz = _sink_mode(mode)
     img_buf = tgt_buf = None
-    if mode == "raw":
+    if mode in _STATS_MODES:
+        img_buf, tgt_buf = _stats_out(out, channels, ctx.device)
+    elif mode == "raw":
         img_buf, tgt_buf = out if out is not None else (
             torch.empty((cap, _align16(max(1, img_elems))), dtype=torch.uint8, device=ctx.device),
             torch.empty((cap, _align16(max(1, tgt_elems))), dtype=torch.uint8, device=ctx.device))
@@ -534,7 +568,7 @@ def parse_table(st: ShardTable, mode, img_elems=0, tgt_elems=0, verify_crc=True,
         img_buf, tgt_buf = out if out is not None else (
             torch.empty((cap, il), dtype=torch.float32, device=ctx.device),
             torch.empty((cap, tl), dtype=torch.float32, device=ctx.device))
-    sink = _make_sink(mode, verify_crc, img_buf, tgt_buf, mean, std, num_classes)
+    sink = _make_sink(mode, verify_crc, img_buf, tgt_buf, mean, std, num_classes, channels)
     if not want_img:
         sink.img_out = None          # the C ABI skips a NULL output
     if not want_tgt:
@@ -555,11 +589,12 @@ class ShardPipeline:
     passes and must be queued well before they are needed.  PARSE slots (`depth` of them) own the status array
     and the output buffers.  Iterating yields (img_buf, tgt_buf, status_dev, table) with the producing work already
     ordered before the caller's current stream; a parse slot is recycled `depth` shards later, after whatever
-    the caller enqueued on its buffers.
+    the caller enqueued on its buffers.  In the statistics modes ('stats', 'stats_f32'; channels= bands) every slot adds
+    into ONE (acc, hist) counter pair (self.stats_out, or out=), which each iteration yields as img_buf / tgt_buf.
     """
 
     def __init__(self, mode, img_elems, tgt_elems, max_records, verify_crc=True, mean=None, std=None, num_classes=None,
-                 device=None, depth=3, max_shard_bytes=0, open_ahead=8):
+                 device=None, depth=3, max_shard_bytes=0, open_ahead=8, channels=None, out=None):
         self.ctx = get_ctx(device)
         dev = self.ctx.device
         self.mode, self.verify_crc, self.num_classes = mode, verify_crc, num_classes
@@ -573,7 +608,10 @@ class ShardPipeline:
         self.oslots = [dict(stage=None, table=None, opened=torch.cuda.Event(), parsed=None) for _ in range(self.open_ahead)]
         self.ready = [torch.cuda.Event() for _ in range(self.depth)]
         self.release = [None] * self.depth
-        self.slots = [dict(status=torch.zeros((self.cap,), dtype=torch.int32, device=dev), out=None) for _ in range(self.depth)]
+        self.channels = channels
+        self.stats_out = _stats_out(out, int(channels), dev) if mode in _STATS_MODES else None
+        self.slots = [dict(status=torch.zeros((self.cap,), dtype=torch.int32, device=dev), out=self.stats_out)
+                      for _ in range(self.depth)]
         self.max_shard_bytes = int(max_shard_bytes)
 
     def reset_events(self):
@@ -612,7 +650,8 @@ class ShardPipeline:
         stream.wait_event(o["opened"])
         with torch.cuda.stream(stream):
             img, tgt, status = parse_table(st, self.mode, self.img_elems, self.tgt_elems, self.verify_crc, self.mean,
-                                           self.std, self.num_classes, out=sl["out"], status=sl["status"])
+                                           self.std, self.num_classes, out=sl["out"], status=sl["status"],
+                                           channels=self.channels)
             if sl["out"] is None and img is not None:
                 sl["out"] = (img, tgt)
             self.ready[slot].record(stream)
@@ -680,21 +719,81 @@ class CapturedPass:
 
 
 def iter_parsed_shards(shards, mode, verify_crc=True, mean=None, std=None, num_classes=None, out=None, device=None,
-                       img_elems=None, tgt_elems=None, max_records=None, depth=3):
+                       img_elems=None, tgt_elems=None, max_records=None, depth=3, channels=None):
     """Parse a sequence of shards (CUDA-resident or pinned-host uint8 tensors).
 
     With img_elems / tgt_elems / max_records given (the chip shape and records-per-shard bound a reader knows from
     its dataset), the shards stream through ShardPipeline without any host synchronisation.  Otherwise each shard
     is opened synchronously to learn its shapes.  Yields (img_buf, tgt_buf, status_dev, table-or-ShardIndex).
+    The statistics modes take channels= and add every shard into one counter pair (out=, or new zeroed counters).
     """
     ctx = get_ctx(device)
     if img_elems is not None and max_records is not None:
-        pipe = ShardPipeline(mode, img_elems, tgt_elems or 0, max_records, verify_crc, mean, std, num_classes, ctx.device, depth)
+        pipe = ShardPipeline(mode, img_elems, tgt_elems or 0, max_records, verify_crc, mean, std, num_classes, ctx.device, depth,
+                             channels=channels, out=out)
         yield from pipe.run(shards)
         return
+    if mode in _STATS_MODES:
+        out = _stats_out(out, int(channels), ctx.device)
     for s in shards:
         si = open_shard(s, ctx.device)
-        yield parse_shard(si, mode, verify_crc=verify_crc, mean=mean, std=std, num_classes=num_classes, out=out) + (si,)
+        yield parse_shard(si, mode, verify_crc=verify_crc, mean=mean, std=std, num_classes=num_classes, out=out,
+                          channels=channels) + (si,)
+
+
+_STATS_KINDS = {"bytes": "stats", "float": "stats_f32"}
+
+
+def shard_stats(shards, channels, kind="bytes", verify_crc=True, max_records=None, device=None, all_reduce=False):
+    """Exact per-band image statistics and the label histogram of whole shards, each shard read once by the fused parse
+    (b2chips.h B2_SINK_STATS / B2_SINK_STATS_F32).
+
+    shards: CUDA-resident or pinned-host uint8 tensors (or bytes), streamed through ShardPipeline with no per-shard host
+    synchronisation.  kind 'bytes': uint8 BytesList records; 'float': packed float32 FloatList records of integer values
+    (uint8 / uint16 / int16 sources).  max_records bounds the records of one shard (default 4096).
+    Returns (bands, histogram): bands = [(n, sum x, sum x^2)] exact Python ints per band, ready for mean_std_from_stats;
+    histogram = 257 ints, bin v counting labels equal to v (0..255) and bin 256 every other label.
+    Raises DataLossError when a frame, a data CRC or the feature template fails (the counters are then undefined), and
+    B2Error when an image value of a 'float' shard is not an integer in [-2^16, 2^16).  With all_reduce=True and
+    torch.distributed initialised, one all_reduce(SUM) of the packed integer counters (the failure counts included) gives
+    every rank the same result, whatever the number of GPUs.  One device-to-host read, at the end.
+    """
+    if kind not in _STATS_KINDS:
+        raise ValueError(kind)
+    ctx = get_ctx(device)
+    C, cap = int(channels), 4096 if max_records is None else int(max_records)
+    src = [torch.from_numpy(np.frombuffer(s, np.uint8).copy()) if isinstance(s, (bytes, bytearray, memoryview)) else s
+           for s in shards]
+    pipe = ShardPipeline(_STATS_KINDS[kind], 0, 0, cap, verify_crc, device=ctx.device, channels=C,
+                         max_shard_bytes=max((int(s.numel()) for s in src), default=0))
+    # records with status != 0, shards with a bad frame, shards with more than cap records, shards
+    tally = torch.zeros((4,), dtype=torch.int64, device=ctx.device)
+    one = torch.ones((), dtype=torch.int64, device=ctx.device)
+    for _, _, _, table in pipe.run(src):
+        h = table.hdr_dev
+        tally.add_(torch.stack((h[4], (h[1] == 1).long(), (h[1] == 2).long(), one)))
+    acc, hist = pipe.stats_out
+    packed = torch.cat((acc.reshape(-1), hist, tally))
+    if all_reduce:
+        import torch.distributed as dist
+        if dist.is_available() and dist.is_initialized():
+            t = packed if dist.get_backend() == "nccl" else packed.cpu()
+            dist.all_reduce(t)                  # exact integer counters: the sum is the same in any order
+            packed = t
+    a = [int(x) for x in packed.cpu().numpy().view(np.uint64)]
+    bad, frame, full, n_shards = a[-4:]
+    if full:
+        raise B2Error("%d shard(s) hold more than max_records=%d records" % (full, cap))
+    if frame:
+        raise DataLossError("corrupted record in %d shard(s) (bad frame or length CRC)" % frame)
+    _check_bad_records(bad, "%d shard(s)" % n_shards)
+    bands = []
+    for c in range(C):
+        n, sx, lo, hi, exc = a[5 * c:5 * c + 5]
+        if exc:
+            raise B2Error("shard_stats: band %d has %d value(s) that are not integers in [-65536, 65536)" % (c, exc))
+        bands.append((n, sx - (1 << 64) if sx >> 63 else sx, lo + 65536 * hi))
+    return bands, a[5 * C:5 * C + 257]
 
 
 # ------------------------------------------------------------------------------------------------ label rasterisation

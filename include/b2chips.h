@@ -135,7 +135,8 @@ int b2_tfrecord_table_layout(uint64_t shard_nbytes, uint64_t max_records, uint64
 int b2_tfrecord_open(b2_ctx* ctx, const uint8_t* shard_dev, uint64_t shard_nbytes, uint64_t max_records,
                      uint8_t* table_dev, b2_stream stream);
 
-enum { B2_SINK_NONE = 0, B2_SINK_RAW = 1, B2_SINK_NORM_ONEHOT = 2, B2_SINK_NORM_ONEHOT_F32 = 3 };
+enum { B2_SINK_NONE = 0, B2_SINK_RAW = 1, B2_SINK_NORM_ONEHOT = 2, B2_SINK_NORM_ONEHOT_F32 = 3, B2_SINK_STATS = 4,
+       B2_SINK_STATS_F32 = 5 };
 typedef struct {
     int32_t mode;        /* B2_SINK_NONE: CRC only.  RAW: payload bytes copied as stored (uint8 arrays; packed
                             little-endian float32 == float arrays).  NORM_ONEHOT: uint8 image -> normalised float32,
@@ -143,7 +144,23 @@ typedef struct {
                             packed float32 FloatList payloads (the higher-dtype array records): image ->
                             (x - mean[c]) / std[c] with IEEE float32 division, target -> one-hot where a label
                             equal to an integer k < K is class k (-0.0 is class 0; NaN, +-inf, negative,
-                            non-integral and >= K labels give an all-zero row).                              */
+                            non-integral and >= K labels give an all-zero row).
+                            STATS (records as NORM_ONEHOT) and STATS_F32 (records as NORM_ONEHOT_F32): exact
+                            per-band statistics of the images and a histogram of the labels, read in the same
+                            pass as the CRC; nothing else is written.  channels = C (1..64); mean, std and
+                            num_classes are not read.  img_out = uint64 acc[C][5] += { n, sum x (two's
+                            complement int64), sum x^2 lo, sum x^2 hi, excluded } per band, with sum x^2 =
+                            lo + 2^16 * hi: the kernel splits per-CTA partial sums, so only that sum is defined.
+                            tgt_out = uint64 hist[257] += labels equal to v in bin v (0..255; -0.0 is 0), bin 256
+                            for labels equal to no such integer (NaN, +-inf, negative, non-integral, > 255;
+                            always 0 in STATS).  STATS_F32 counts an image value that is an integer in
+                            [-2^16, 2^16) (u8, u16 and i16 sources); any other value goes to its band's
+                            `excluded` and into no sum.  STATS excludes nothing.  Either output may be NULL
+                            (skipped); both must be 8-byte aligned with img_stride = tgt_stride = 0.  The
+                            counters ACCUMULATE (the caller zeroes them), also from several launches on
+                            several streams.  A record with status 2 or 3 adds nothing, but a record's data
+                            CRC is known only after its bytes were counted: the counters are defined only
+                            when every record's status is 0 (check hdr[4] or the status array).             */
     int32_t verify_crc;  /* non-zero: compute each record's data CRC and compare with the stored masked CRC   */
     void* img_out;       /* record i lands at img_out + i*img_stride (bytes)                                  */
     uint64_t img_stride;
