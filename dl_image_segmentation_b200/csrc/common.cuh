@@ -13,11 +13,9 @@ namespace b2 {
 struct CrcTables {
     uint32_t t4[4][256];     // standard slice-by-4: t4[k][v] = state v<<(8k) advanced by 4 zero bytes
     uint32_t s4096[4][256];  // same, advanced by 4 + 4096 - 16 bytes (second vector of a thread in a 8 KiB tile)
-    uint32_t fix[256];       // fix[i] = x^(-128 i): undo the 16*i byte over-advance of thread i
-    uint32_t xinv16[514];    // xinv16[q] = x^(-128 q): un-advance by q 16-byte vectors (tile padding)
+    uint32_t xinv16[514];    // xinv16[q] = x^(-128 q): un-advance by q 16-byte vectors (thread alignment, tile padding)
     uint32_t xinvb[16];      // xinvb[r]  = x^(-8 r)
     uint32_t x2n[64];        // x^(2^k) for x2n pow
-    uint32_t xtile;          // x^(8*8192): advance by one tile
     uint32_t tpow[2048];     // tpow[j] = x^(8*8192*j): advance by j tiles (records up to 16 MiB; beyond -> xpow8)
 };
 

@@ -63,21 +63,14 @@ static void build_tables(CrcTables* t) {
         }
     t->x2n[0] = 0x40000000u;  // x^1
     for (int k = 1; k < 64; k++) t->x2n[k] = multmodp(t->x2n[k - 1], t->x2n[k - 1]);
-    t->xtile = t->x2n[16];    // x^(8*8192) = x^(2^16)
+    const uint32_t xtile = t->x2n[16];    // x^(8*8192) = x^(2^16)
     t->tpow[0] = 0x80000000u;
-    for (int j = 1; j < 2048; j++) t->tpow[j] = multmodp(t->tpow[j - 1], t->xtile);
-    // thread i of a tile ends 4080-16*i bytes short of the tile end
-    uint32_t x128 = t->x2n[7];  // x^128 : advance by 16 bytes
-    uint32_t p = 0x80000000u;   // x^0
-    for (int i = 255; i >= 0; i--) {
-        t->fix[i] = p;
-        p = multmodp(p, x128);
-    }
+    for (int j = 1; j < 2048; j++) t->tpow[j] = multmodp(t->tpow[j - 1], xtile);
     uint32_t xi8 = 0x80000000u;
     for (int k = 0; k < 8; k++) xi8 = div_x(xi8);      // x^-8
     uint32_t xi128 = xi8;
     for (int k = 0; k < 4; k++) xi128 = multmodp(xi128, xi128);  // x^-128
-    p = 0x80000000u;
+    uint32_t p = 0x80000000u;
     for (int r = 0; r < 16; r++) {
         t->xinvb[r] = p;
         p = multmodp(p, xi8);

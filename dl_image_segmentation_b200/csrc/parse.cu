@@ -18,16 +18,10 @@
 //   * producer and consumers meet only through mbarriers (full / empty per buffer); there is no __syncthreads in
 //     the steady state and no second kernel: the CRC state of a thread runs on across the consecutive tiles of a
 //     record, the warps of a CTA fold their states through a shared-memory slot when the run of tiles ends, and
-//     the last warp there merges { CRC partial, tiles done } into the record's 64-bit accumulator (atomic XOR
-//     + atomic add on one address); whoever completes a record un-advances the zero padding, compares with the stored
-//     masked CRC and writes the record's status.
+//     the last warp there merges the run into the record's accumulator; whoever completes a record compares its CRC
+//     with the stored masked CRC and writes the record's status.
 //
-// CRC-32C without a CRC instruction: the pure CRC (zero init) is linear over GF(2), so
-//   * thread i consumes vectors i and i+256 (16 bytes each) of every tile with slice-by-4 table steps; the step
-//     after a vector's last word also skips the 4080 bytes to the thread's next vector, in this tile or the next;
-//   * when the run ends, one GF(2)[x] multiplication by x^(-128 i) aligns thread i's state with the tile end,
-//     the states XOR together, and one more multiplication by a tabulated power of x moves the partial to the
-//     end of the record.  The 0xFFFFFFFF init is XORed into the first four data bytes.
+// The record CRC-32C (tiles, runs, accumulator, padding) is described in tfrecord_common.cuh.
 #include <type_traits>
 
 #include "tfrecord_common.cuh"
@@ -580,31 +574,14 @@ __device__ inline void finalize_record(const ParseArgs& a, const RecRef& j, uint
     const uint32_t r = j.r;
     const uint64_t d0 = j.d0, len = j.d1 - j.d0;
     const bool want_crc = a.sink.verify_crc || a.crc_out;
-    uint32_t crc = 0;
-    if (want_crc) {
-        if (len < 4) {   // the init XOR does not fit in the message: bytewise
-            uint32_t s = 0xFFFFFFFFu;
-            for (uint64_t i = 0; i < len; i++) s = (s >> 8) ^ __ldg(&a.tab->t4[3][(s ^ a.shard[d0 + i]) & 0xff]);
-            crc = ~s;
-        } else {
-            // acc sits at the end of the last tile; un-advance by the zero padding after the record end
-            const uint64_t pad = (d0 & ~15ull) + (uint64_t)j.nt * kTile - j.d1;
-            acc = multmodp(__ldg(&a.tab->xinv16[pad >> 4]), acc);
-            acc = multmodp(__ldg(&a.tab->xinvb[pad & 15]), acc);
-            crc = ~acc;
-        }
-    }
+    const uint32_t crc = want_crc ? record_crc(a.tab, acc, (d0 & ~15ull) + (uint64_t)j.nt * kTile - j.d1, a.shard + d0, len) : 0;
     if (a.crc_out) {
         a.crc_out[r] = crc;
         return;
     }
     int32_t st = 0;
     if (a.sink.verify_crc) {
-        uint32_t stored = ~mask_crc(crc);
-        if (a.nbytes == ~0ull || j.d1 + 4 <= a.nbytes) {
-            stored = 0;
-            for (int k = 0; k < 4; k++) stored |= (uint32_t)a.shard[j.d1 + k] << (8 * k);
-        }
+        const uint32_t stored = a.nbytes == ~0ull || j.d1 + 4 <= a.nbytes ? rd_u32(a.shard + j.d1) : ~mask_crc(crc);
         if (stored != mask_crc(crc)) st = 1;
     }
     if (kMode != B2_SINK_NONE && st == 0 && a.index) st = sink_status<kMode>(a.index + r, a.sink);
@@ -627,36 +604,27 @@ struct RunAcc {          // shared-memory meeting point of the eight consumer wa
 };
 
 // Close a run.  No CTA-wide barrier: every consumer warp folds its lanes' CRC states, XORs the result into the run's
-// shared-memory slot and counts itself; the warp that arrives last moves the partial to the end of the record and
-// merges { CRC, tiles } into the record's 64-bit accumulator with an atomic XOR and an atomic add on the same address
-// (applied in program order, so no fences are needed), finalising the record when its tile count is complete.  The other warps are already working
-// on the next tile.  Every warp flushes a run in the same loop iteration `it`, at most one run per iteration, and its
-// slot is `it` mod kRunSlots: a slot comes round again kRunSlots iterations later, and no warp can be more than kStages
+// shared-memory slot and counts itself; the warp that arrives last merges the run into the record's accumulator,
+// finalising the record when its tile count is complete.  The other warps are already working on the next tile.
+// Every warp flushes a run in the same loop iteration `it`, at most one run per iteration, and its slot is `it` mod kRunSlots: a slot comes round again kRunSlots iterations later, and no warp can be more than kStages
 // (< kRunSlots) iterations ahead of the slowest, whose arrival on the buffer's empty barrier the producer waits for.
 template <int kMode>
 __device__ __forceinline__ void run_flush(const ParseArgs& a, Run& run, uint32_t& s, uint32_t it, bool want_crc,
                                           RunAcc* racc) {
     const int tid = threadIdx.x, lane = tid & 31;
     RunAcc* ra = racc + (it & (kRunSlots - 1));
-    const bool crc = want_crc && run.d1 - run.d0 >= 4;
-    if (crc) {
-        uint32_t t = multmodp_fast(__ldg(&a.tab->xinv16[tid]), s);
-#pragma unroll
-        for (int o = 16; o; o >>= 1) t ^= __shfl_xor_sync(0xffffffffu, t, o);
+    if (want_crc && crc_tiled(run.d1 - run.d0)) {
+        const uint32_t t = crc_lane_partial(a.tab, s);
         if (lane == 0 && t) atomicXor(&ra->crc, t);
     }
     if (lane == 0) {
         __threadfence_block();
         if (atomicAdd(&ra->warps, 1u) == kConsumerWarps - 1) {
             __threadfence_block();
-            uint32_t c = atomicExch(&ra->crc, 0u);
+            const uint32_t c = atomicExch(&ra->crc, 0u);
             ra->warps = 0;
-            if (crc) c = multmodp_fast(tile_power(a.tab, run.nt - 1 - run.last_tile), c);
-            // XOR into the low word, then count in the high word: two atomics on ONE address are applied in program
-            // order, so whoever sees the count complete also sees every partial (no fence, no retry loop)
             unsigned long long* acc = a.acc + run.r;
-            if (c) atomicXor(acc, (unsigned long long)c);
-            const unsigned long long upd = atomicAdd(acc, (unsigned long long)run.tiles << 32) + ((unsigned long long)run.tiles << 32);
+            const unsigned long long upd = record_acc_merge(a.tab, acc, c, run.nt - 1 - run.last_tile, run.tiles);
             if ((uint32_t)(upd >> 32) == run.nt) {
                 *acc = 0ull;               // re-arm for the next launch; nobody else touches a finished record
                 RecRef rr{run.r, run.nt, run.d0, run.d1};
@@ -821,7 +789,7 @@ fused_parse_kernel(const ParseArgs a) {
             }
             run.tiles++;
             run.last_tile = j.tile;
-            if (want_crc && d1 - d0 >= 4) s = crc_tile_step(s, buf4, &cs, j, j.tile != 0 && te <= d1);
+            if (crc_tiled(d1 - d0) && want_crc) s = crc_tile_step(s, buf4, &cs, j, j.tile != 0 && te <= d1);
             PROF_MARK(1);
             if (kMode == B2_SINK_RAW && (flags & 2)) {
                 if (a.sink.img_out)

@@ -7,18 +7,7 @@
 //                                   parse_single_example / decode_raw / reshape
 //                                                               _tfrecord_image_translation.py:249,306-314,394-407
 //
-// Data layout: a shard is one contiguous device buffer.  Record data is cut into 8 KiB tiles on a 16-byte
-// aligned grid anchored at the record's (aligned-down) data start; one 256-thread CTA owns one tile.  A tile is
-// staged ONCE in shared memory with coalesced 128-bit loads and then serves both the CRC and the payload sinks,
-// so every input byte crosses HBM exactly once.
-//
-// CRC-32C without a CRC instruction: the pure CRC (zero init) is linear over GF(2), so
-//   * thread i CRCs its two 16-byte vectors (tile offsets 16 i and 16 i + 4096) with table steps whose
-//     "advance" also skips the gap between them,
-//   * one GF(2)[x] multiplication by x^(8*(4080-16 i)) moves its partial to the end of the tile,
-//   * partials XOR together (warp shuffles, then 8 words of shared memory) into one word per tile,
-//   * a warp per record folds the tile words left to right (Horner with x^(8*8192)) and un-advances by the
-//     zero padding after the record end.  The 0xFFFFFFFF init is XORed into the first four data bytes.
+// Data layout: a shard is one contiguous device buffer.  The record CRC-32C is described in tfrecord_common.cuh.
 #include <cstring>
 #include <vector>
 
@@ -44,24 +33,6 @@ constexpr int kScanR = 128;
 constexpr int kScanHW = 112;
 constexpr int kScanWB = 2 * kScanHW + 32;   // bytes per window (multiple of 16)
 
-__device__ __forceinline__ uint32_t crc_hdr8(uint64_t l, const uint32_t* t) {   // t = byte table (reflected CRC-32C)
-    uint32_t s = 0xFFFFFFFFu;
-#pragma unroll
-    for (int i = 0; i < 8; i++) s = (s >> 8) ^ t[(s ^ (uint32_t)(l >> (8 * i))) & 0xff];
-    return mask_crc(~s);
-}
-__device__ __forceinline__ uint64_t rd_u64(const uint8_t* p) {
-    uint64_t v = 0;
-#pragma unroll
-    for (int i = 0; i < 8; i++) v |= (uint64_t)p[i] << (8 * i);
-    return v;
-}
-__device__ __forceinline__ uint32_t rd_u32(const uint8_t* p) {
-    uint32_t v = 0;
-#pragma unroll
-    for (int i = 0; i < 4; i++) v |= (uint32_t)p[i] << (8 * i);
-    return v;
-}
 // 8 bytes at an arbitrary byte offset of a 4-byte aligned shared-memory buffer: three word loads + two funnel shifts
 __device__ __forceinline__ uint64_t smem_u64_unaligned(const uint8_t* base, uint32_t off) {
     const uint32_t* w = reinterpret_cast<const uint32_t*>(base) + (off >> 2);
@@ -483,8 +454,6 @@ struct BuildArgs {
     uint8_t* out;
     const CrcTables* tab;
     unsigned long long* acc;   // per record { CRC partial, tiles done }, zero on entry
-    uint32_t tiles_x;
-    int n;
 };
 
 __device__ __forceinline__ uint32_t elem_as_f32_bits(const void* src, int dtype, uint64_t i, uint64_t count) {
@@ -543,11 +512,7 @@ __global__ void __launch_bounds__(kTileThreads, 8) build_kernel(const BuildArgs 
     if (t_lo >= t_end) return;
     const uint32_t t_hi = t_lo + kBuildRun < t_end ? t_lo + kBuildRun : t_end;
     load_crc_tables(&cs, a.tab);
-    if (threadIdx.x == 0) {
-        uint32_t s = 0xFFFFFFFFu;
-        for (int i = 0; i < 8; i++) s = (s >> 8) ^ __ldg(&a.tab->t4[3][(s ^ (uint32_t)((L >> (8 * i)) & 0xFF)) & 0xff]);
-        hdr_crc = mask_crc(~s);
-    }
+    if (threadIdx.x == 0) hdr_crc = crc_hdr8(L, a.tab->t4[3]);
     __syncthreads();
     uint32_t crc_state = 0;                                              // this thread's running CRC over the run
   for (uint32_t tile = t_lo; tile < t_hi; tile++) {
@@ -649,43 +614,24 @@ staged:
         }
     }
     // running CRC over the data range; the tile grid is anchored at A = rs & ~15
-    if (L >= 4 && te > d0) crc_state = crc_running_step(crc_state, buf4, &cs, ts, d0, d1, ts <= d0 && d0 < te, ts >= d0 && te <= d1);
+    if (crc_tiled(L) && te > d0) crc_state = crc_running_step(crc_state, buf4, &cs, ts, d0, d1, ts <= d0 && d0 < te, ts >= d0 && te <= d1);
     __syncthreads();                                                       // buf4 is restaged by the next tile
   }
-    // End of the run: align the per-thread states with the end of the run's last tile, fold them, move the partial to
-    // the end of the record's last tile and merge { CRC, tiles } into the record's 64-bit accumulator (atomic XOR +
-    // atomic add on one address, applied in program order); the CTA that completes the record un-advances the zero
-    // padding and writes the masked CRC footer.
-    uint32_t t = multmodp_fast(__ldg(&a.tab->xinv16[threadIdx.x]), crc_state);
-#pragma unroll
-    for (int o = 16; o; o >>= 1) t ^= __shfl_xor_sync(0xffffffffu, t, o);
+    // End of the run: fold the threads' states (a record too short for a partial leaves them zero) and merge the run into
+    // the record's accumulator; the CTA that completes the record writes the masked CRC footer.
+    const uint32_t t = crc_lane_partial(a.tab, crc_state);
     if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = t;
     __syncthreads();
     if (threadIdx.x == 0) {
         uint32_t c = 0;
 #pragma unroll
         for (int k = 0; k < kTileThreads / 32; k++) c ^= red[k];
-        if (L >= 4 && c) c = multmodp_fast(tile_power(a.tab, t_end - t_hi), c);
-        unsigned long long* acc = a.acc + r;
-        if (L >= 4 && c) atomicXor(acc, (unsigned long long)c);
-        const unsigned long long add = (unsigned long long)(t_hi - t_lo) << 32;
-        const unsigned long long upd = atomicAdd(acc, add) + add;
+        const unsigned long long upd = record_acc_merge(a.tab, a.acc + r, c, t_end - t_hi, t_hi - t_lo);
         if ((uint32_t)(upd >> 32) == t_end) {
-            uint32_t crc;
-            if (L < 4) {   // an Example shorter than 4 bytes has no payload: its bytes are scaffold bytes
-                const uint8_t* sc = a.scaffold + d.scaffold_off;
-                uint32_t s = 0xFFFFFFFFu;
-                for (uint64_t i = 0; i < L; i++) s = (s >> 8) ^ __ldg(&a.tab->t4[3][(s ^ sc[i]) & 0xff]);
-                crc = ~s;
-            } else {
-                uint32_t accv = (uint32_t)upd;
-                const uint64_t pad = A + (uint64_t)t_end * kTile - (d0 + L);
-                accv = multmodp(__ldg(&a.tab->xinv16[pad >> 4]), accv);
-                accv = multmodp(__ldg(&a.tab->xinvb[pad & 15]), accv);
-                crc = ~accv;
-            }
-            const uint32_t m = mask_crc(crc);
-            for (int j = 0; j < 4; j++) a.out[d0 + L + j] = (uint8_t)(m >> (8 * j));
+            // an Example shorter than 4 bytes has no payload: its bytes are scaffold bytes
+            const uint32_t m = mask_crc(record_crc(a.tab, (uint32_t)upd, A + (uint64_t)t_end * kTile - d1,
+                                                   a.scaffold + d.scaffold_off, L));
+            for (int j = 0; j < 4; j++) a.out[d1 + j] = (uint8_t)(m >> (8 * j));
         }
     }
 }
@@ -772,7 +718,7 @@ extern "C" int b2_tfrecord_build(b2_ctx* ctx, const b2_build_desc* descs, int n,
     WsLock ws_lock(ctx);
     if (int e = ws_reserve(ctx, (size_t)n * sizeof(unsigned long long), s)) return e;
     B2_CUDA(cudaMemsetAsync(ctx->ws, 0, (size_t)n * sizeof(unsigned long long), s));
-    BuildArgs ba{descs, scaffold, out, ctx->crc_dev, static_cast<unsigned long long*>(ctx->ws), tx, n};
+    BuildArgs ba{descs, scaffold, out, ctx->crc_dev, static_cast<unsigned long long*>(ctx->ws)};
     build_kernel<<<dim3((tx + kBuildRun - 1) / kBuildRun, n), kTileThreads, 0, s>>>(ba);
     ctx->launches++;
     B2_CUDA(cudaGetLastError());

@@ -53,46 +53,7 @@ __device__ __forceinline__ uint32_t multmodp_fast(uint32_t a, uint32_t b) {
     return p;
 }
 
-// CRC partial of one staged tile (vectors already zero outside [d0,d1)).  Returns the CTA-wide XOR in thread 0.
-// init_lo/init_hi: absolute range whose bytes get the 0xFF init XOR (d0..d0+4), only relevant for tile 0.
-__device__ __forceinline__ uint32_t tile_crc(const uint4* buf4, const CrcSmem* cs, const CrcTables* tab, uint64_t ts,
-                                             uint64_t d0, uint64_t d1, bool first_tile, uint32_t* red) {
-    const int i = threadIdx.x;
-    uint4 v0 = mask_vec(buf4[i], ts + 16ull * i, d0, d1);
-    uint4 v1 = mask_vec(buf4[i + 256], ts + 4096 + 16ull * i, d0, d1);
-    if (first_tile && i < 2) {  // init XOR lives in the first 4 data bytes, i.e. inside vectors 0/1 of tile 0
-        uint32_t w[4] = {v0.x, v0.y, v0.z, v0.w};
-#pragma unroll
-        for (int q = 0; q < 4; q++)
-#pragma unroll
-            for (int j = 0; j < 4; j++) {
-                const uint64_t p = ts + 16ull * i + 4 * q + j;
-                if (p >= d0 && p < d0 + 4) w[q] ^= 0xFFu << (8 * j);
-            }
-        v0 = make_uint4(w[0], w[1], w[2], w[3]);
-    }
-    uint32_t s = adv4(cs->t4, v0.x);
-    s = adv4(cs->t4, s ^ v0.y);
-    s = adv4(cs->t4, s ^ v0.z);
-    s = adv4(cs->s, s ^ v0.w);
-    s = adv4(cs->t4, s ^ v1.x);
-    s = adv4(cs->t4, s ^ v1.y);
-    s = adv4(cs->t4, s ^ v1.z);
-    s = adv4(cs->t4, s ^ v1.w);
-    s = multmodp_fast(__ldg(&tab->fix[i]), s);
-#pragma unroll
-    for (int o = 16; o; o >>= 1) s ^= __shfl_xor_sync(0xffffffffu, s, o);
-    if ((i & 31) == 0) red[i >> 5] = s;
-    __syncthreads();
-    uint32_t r = 0;
-    if (i == 0) {
-#pragma unroll
-        for (int k = 0; k < kTileThreads / 32; k++) r ^= red[k];
-    }
-    return r;
-}
-
-// stage [ts, ts + kTile + 32) of `base` into shared memory, zero beyond `nbytes`
+// 4 bytes at an arbitrary byte offset of a 4-byte aligned shared-memory buffer: two word loads + one funnel shift
 __device__ __forceinline__ uint32_t smem_u32_unaligned(const uint32_t* buf32, uint32_t off) {
     const uint32_t w0 = buf32[off >> 2], w1 = buf32[(off >> 2) + 1];
     return __funnelshift_r(w0, w1, (off & 3) * 8);
@@ -110,16 +71,35 @@ __device__ inline uint32_t xpow8(const CrcTables* tab, uint64_t n) {
     return p;
 }
 
-// Fold the per-tile partials of one record into its CRC-32C (one warp per record, all lanes return it).
+// TFRecord's masked CRC, as stored in a frame's header and footer
 __device__ __forceinline__ uint32_t mask_crc(uint32_t c) { return ((c >> 15) | (c << 17)) + 0xa282ead8u; }
 
-// Per-thread running CRC state over consecutive tiles of one record.  A thread owns vectors i and i+256 of every tile; the
-// distance from the end of one of its vectors to the start of its next one is always 4080 bytes, inside a tile and
-// from one tile to the next, so the same "consume 4 bytes and skip 4080" table step chains them all and the
-// expensive per-thread alignment (one GF(2)[x] multiplication) is paid once per run of tiles, not once per tile.
-// On return the state sits at (tile end + 16 i): the caller un-advances by 16 i (xinv16[i]) when the run ends.
-// ts = absolute start of the tile; [d0, d1) = the record's data; first = the tile holding d0 (the 0xFFFFFFFF init is
-// XORed into the first four data bytes); interior = no byte of the tile lies outside [d0, d1).
+// ---------------------------------------------------------------- record CRC-32C (reader: parse.cu, writer: build_kernel)
+// A record's data CRC is computed over 8 KiB tiles on a 16-byte aligned grid, a run of consecutive tiles per CTA, without
+// a CRC instruction.  The pure CRC (zero init) is linear over GF(2), so:
+//   * bytes outside the record count as zero and the 0xFFFFFFFF init is XORed into its first four data bytes;
+//   * thread i owns vectors i and i + 256 (16 bytes each) of every tile.  From the end of one of its vectors to the start
+//     of its next one is always 4080 bytes, inside a tile and from one tile to the next, so one slice-by-4 step that
+//     consumes 4 bytes and skips 4080 chains them all (crc_running_step) and the per-thread alignment (one GF(2)[x]
+//     multiplication) is paid once per run of tiles, not once per tile;
+//   * when a run ends, thread i's state sits 16 i bytes past the end of the run's last tile: multiplying by x^(-128 i)
+//     aligns it and the lanes of a warp XOR together (crc_lane_partial); each kernel folds its warps in its own way;
+//   * the run's partial moves to the end of the record's last tile and merges, with the run's tile count, into one
+//     64-bit accumulator word per record, { CRC partial (low 32 bits) | tiles done (high 32) }, zero before the first
+//     run (record_acc_merge);
+//   * whoever completes the tile count un-advances the zero padding between the record end and the end of its last
+//     tile and complements (record_crc).
+// The grid is anchored at the aligned-down start of what a kernel stages: the record data for the reader (d0 & ~15), the
+// frame for the writer ((d0 - 12) & ~15).  So the callers, not record_crc, know where the grid ends: they pass the padding.
+// A record shorter than 4 bytes has no room for the init XOR: it carries no partial (crc_tiled) and record_crc takes
+// its CRC bytewise.
+
+// Whether a record of len data bytes carries a tiled CRC partial (else it is CRC'd bytewise when it completes)
+__device__ __forceinline__ bool crc_tiled(uint64_t len) { return len >= 4; }
+
+// One tile of a thread's running CRC state.  On return the state sits at (tile end + 16 i).
+// ts = absolute start of the tile; [d0, d1) = the record's data; first = the tile holding d0; interior = no byte of the
+// tile lies outside [d0, d1).
 __device__ __forceinline__ uint32_t crc_running_step(uint32_t s, const uint4* buf4, const CrcSmem* cs, uint64_t ts, uint64_t d0,
                                                      uint64_t d1, bool first, bool interior) {
     const int i = threadIdx.x;
@@ -153,6 +133,67 @@ __device__ __forceinline__ uint32_t crc_running_step(uint32_t s, const uint4* bu
 // x^(8*8192*j): advance a tile partial by j tiles
 __device__ __forceinline__ uint32_t tile_power(const CrcTables* tab, uint32_t j) {
     return j < 2048 ? __ldg(&tab->tpow[j]) : xpow8(tab, (uint64_t)j * kTile);
+}
+
+// End of a run: align thread threadIdx.x's running state with the end of the run's last tile and XOR the warp's lanes
+// together (every lane returns the warp's partial)
+__device__ __forceinline__ uint32_t crc_lane_partial(const CrcTables* tab, uint32_t s) {
+    uint32_t t = multmodp_fast(__ldg(&tab->xinv16[threadIdx.x]), s);
+#pragma unroll
+    for (int o = 16; o; o >>= 1) t ^= __shfl_xor_sync(0xffffffffu, t, o);
+    return t;
+}
+
+// Merge a run into its record's accumulator word: the run's CTA-wide partial (at the end of the run's last tile) moves
+// on by the tiles_after tiles that follow the run in the record, then `tiles` tiles are counted.  Returns the word after
+// the merge: whoever sees the count complete finalises the record.  The XOR into the low word and the add to the high
+// word are two atomics on ONE address, applied in program order, so whoever sees the count complete also sees every
+// partial: no fence, no retry loop.
+__device__ __forceinline__ unsigned long long record_acc_merge(const CrcTables* tab, unsigned long long* acc, uint32_t partial,
+                                                               uint32_t tiles_after, uint32_t tiles) {
+    if (partial) atomicXor(acc, (unsigned long long)multmodp_fast(tile_power(tab, tiles_after), partial));
+    const unsigned long long add = (unsigned long long)tiles << 32;
+    return atomicAdd(acc, add) + add;
+}
+
+// Bytewise CRC-32C of n bytes (init 0xFFFFFFFF, complemented)
+__device__ __forceinline__ uint32_t crc_bytes(const CrcTables* tab, const uint8_t* p, uint64_t n) {
+    uint32_t s = 0xFFFFFFFFu;
+    for (uint64_t i = 0; i < n; i++) s = (s >> 8) ^ __ldg(&tab->t4[3][(s ^ p[i]) & 0xff]);
+    return ~s;
+}
+
+// A completed record's unmasked CRC-32C.  acc: the low word of its accumulator (the partial at the end of its last tile);
+// pad: the bytes from the record end to the end of its last tile; data, len: the record's bytes, read only when the
+// record is too short to carry a partial.
+__device__ __forceinline__ uint32_t record_crc(const CrcTables* tab, uint32_t acc, uint64_t pad, const uint8_t* data,
+                                               uint64_t len) {
+    if (!crc_tiled(len)) return crc_bytes(tab, data, len);
+    acc = multmodp(__ldg(&tab->xinv16[pad >> 4]), acc);
+    acc = multmodp(__ldg(&tab->xinvb[pad & 15]), acc);
+    return ~acc;
+}
+
+// Masked CRC of a frame's 8 little-endian length bytes (the header CRC); t = byte table (t4[3], or a shared-memory copy)
+__device__ __forceinline__ uint32_t crc_hdr8(uint64_t l, const uint32_t* t) {
+    uint32_t s = 0xFFFFFFFFu;
+#pragma unroll
+    for (int i = 0; i < 8; i++) s = (s >> 8) ^ t[(s ^ (uint32_t)(l >> (8 * i))) & 0xff];
+    return mask_crc(~s);
+}
+
+// little-endian integers at any byte address
+__device__ __forceinline__ uint64_t rd_u64(const uint8_t* p) {
+    uint64_t v = 0;
+#pragma unroll
+    for (int i = 0; i < 8; i++) v |= (uint64_t)p[i] << (8 * i);
+    return v;
+}
+__device__ __forceinline__ uint32_t rd_u32(const uint8_t* p) {
+    uint32_t v = 0;
+#pragma unroll
+    for (int i = 0; i < 4; i++) v |= (uint32_t)p[i] << (8 * i);
+    return v;
 }
 
 // 16 bytes at shard + a (a is 16-aligned), zero beyond nbytes
