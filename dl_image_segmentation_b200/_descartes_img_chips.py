@@ -220,15 +220,19 @@ def _cat_last(arrays):
 
 
 # ------------------------------------------------------------------------------------------------ label rasterisation
+def _load_geojson(path_or_dict):
+    import json
+    if isinstance(path_or_dict, dict):
+        return path_or_dict
+    with open(path_or_dict, "r") as f:
+        return json.load(f)
+
+
 def read_geojson_layer(path_or_dict):
     """A label layer from GeoJSON (the format of the reference's label data, .MISSING_LARGE_BLOBS): list of
     (rings, properties) per Polygon / MultiPolygon feature, in file order — what iterating the OGR layer yields.
-    Coordinates are taken as they are: they must already be in the tile's CRS (OGR's on-the-fly reprojection is PROJ's)."""
-    import json
-    gj = path_or_dict
-    if not isinstance(gj, dict):
-        with open(gj, "r") as f:
-            gj = json.load(f)
+    Coordinates are returned as they are, in the layer's CRS (geojson_crs_epsg)."""
+    gj = _load_geojson(path_or_dict)
     feats = gj["features"] if gj.get("type") == "FeatureCollection" else [gj]
     layer = []
     for ft in feats:
@@ -243,21 +247,109 @@ def read_geojson_layer(path_or_dict):
     return layer
 
 
-def create_label_array_for_tile(ctx, label_data, attrib_to_burn=None, layer_idx=0, background_value=255, device=None):
+_CRS84 = "URN:OGC:DEF:CRS:OGC:1.3:CRS84"
+
+
+def _epsg_of_name(name):
+    """'EPSG:n', 'urn:ogc:def:crs:EPSG::n' or the CRS84 URN (longitude / latitude on WGS84, = 4326) -> n."""
+    u = str(name).strip().upper()
+    if u == _CRS84:
+        return 4326
+    for prefix in ("EPSG:", "URN:OGC:DEF:CRS:EPSG::"):
+        if u.startswith(prefix) and u[len(prefix):].isdigit():
+            return int(u[len(prefix):])
+    raise B2Error("label CRS %r is not supported (EPSG:4326, CRS84 or a WGS84 UTM zone EPSG:326zz / 327zz)" % (name,))
+
+
+def geojson_crs_epsg(gj):
+    """EPSG code of a GeoJSON object's ``crs`` member ({"type": "name", "properties": {"name": ...}}), None without one."""
+    crs = gj.get("crs")
+    if crs is None:
+        return None
+    name = (crs.get("properties") or {}).get("name") if isinstance(crs, dict) else None
+    if name is None:
+        raise B2Error("label CRS %r is not supported: only named CRSs ({'type': 'name', ...}) are read" % (crs,))
+    return _epsg_of_name(name)
+
+
+def _is_utm(epsg):
+    return epsg // 100 in (326, 327) and 1 <= epsg % 100 <= 60
+
+
+def label_layer_epsg(tile_epsg, label_crs=None, crs_member=None, layer=()):
+    """The CRS a label layer is in, as RasterizeLayer would learn it from the layer's SRS: ``label_crs`` (an EPSG int or
+    'EPSG:n') if given, else the GeoJSON ``crs`` member's code (geojson_crs_epsg), else — no CRS declared — longitude /
+    latitude (4326) when the tile is in UTM and every coordinate lies in [-180, 180] x [-90, 90] (GeoJSON's default CRS; a
+    UTM easting is never below ~160 km, so a layer in the tile's own CRS never passes), else the tile's CRS.  Raises B2Error
+    for a declared CRS other than 4326 / WGS84 UTM, or a layer that needs projecting onto a tile that is not in UTM."""
+    if label_crs is not None:
+        epsg = int(label_crs) if isinstance(label_crs, (int, np.integer)) else _epsg_of_name(label_crs)
+    else:
+        epsg = crs_member
+    if epsg is None:
+        xy = [np.asarray(r, dtype=np.float64).reshape(-1, 2) for rings, _ in layer for r in rings]
+        xy = np.concatenate(xy) if xy else np.zeros((0, 2))
+        lonlat = len(xy) > 0 and bool((np.abs(xy[:, 0]) <= 180.0).all() and (np.abs(xy[:, 1]) <= 90.0).all())
+        return 4326 if _is_utm(tile_epsg) and lonlat else tile_epsg
+    if epsg != 4326 and not _is_utm(epsg):
+        raise B2Error("label CRS EPSG:%d is not supported (EPSG:4326 or a WGS84 UTM zone EPSG:326zz / 327zz)" % epsg)
+    if epsg != tile_epsg and not _is_utm(tile_epsg):
+        raise B2Error("labels in EPSG:%d cannot be projected onto a tile in %s: only WGS84 UTM tiles are supported"
+                      % (epsg, "EPSG:%d" % tile_epsg if tile_epsg else "an unknown CRS"))
+    return epsg
+
+
+def _project_layer(layer, src_epsg, dst_epsg, device):
+    """Every vertex of the layer in one upload, one b2_project_points launch and one download; vertices only, as
+    OGRGeometry::transform does (edges are not densified).  A feature with a vertex the projection is not valid for is
+    dropped with a warning: OGR refuses to transform such a geometry, so it burns nothing."""
+    rings = [np.asarray(r, dtype=np.float64).reshape(-1, 2) for rs, _ in layer for r in rs]
+    if not rings:
+        return layer
+    xy = ops.project_points(np.concatenate(rings), src_epsg, dst_epsg, device=device).cpu().numpy()
+    ring_end = np.cumsum([len(r) for r in rings])
+    feat_end = np.cumsum([len(rs) for rs, _ in layer])
+    nan_upto = np.concatenate([[0], np.cumsum(np.isnan(xy).any(axis=1))])          # NaN vertices before vertex i
+    vert_end = np.concatenate([[0], ring_end])[feat_end]                             # first vertex after feature f
+    bad = np.diff(np.concatenate([[0], nan_upto[vert_end]])) > 0
+    projected = [xy[i:j] for i, j in zip([0] + ring_end[:-1].tolist(), ring_end.tolist())]
+    out, at = [], 0
+    for (rs, props), end, b in zip(layer, feat_end, bad):
+        if not b:
+            out.append((projected[at:end], props))
+        at = end
+    skipped = int(bad.sum())
+    if skipped:
+        import warnings
+        warnings.warn("create_label_array_for_tile: %d label feature(s) have vertices that cannot be projected from EPSG:%d "
+                      "to EPSG:%d; they are not burnt" % (skipped, src_epsg, dst_epsg))
+    return out
+
+
+def create_label_array_for_tile(ctx, label_data, attrib_to_burn=None, layer_idx=0, background_value=255, device=None,
+                                label_crs=None):
     """Rasterises the label polygons within the geocontext -> (S, S) uint8 CUDA tensor, S = tilesize + 2 * pad
     (reference :633-689: GDAL MEM raster filled with background_value, RasterizeLayer ALL_TOUCHED with the attribute or 1).
 
-    ctx needs ``tilesize``, ``pad`` and ``geotrans`` (GDAL order) like a DLTile.  label_data: a GeoJSON path / dict
-    (read_geojson_layer), or a list of layers / one layer = list of (rings in the tile's map coordinates, properties)."""
+    ctx needs ``tilesize``, ``pad`` and ``geotrans`` (GDAL order) like a DLTile, and ``epsg`` or ``crs`` for labels in another
+    CRS.  label_data: a GeoJSON path / dict (read_geojson_layer), or a list of layers / one layer = list of (rings,
+    properties).  The layer's CRS is resolved by label_layer_epsg (label_crs, then the GeoJSON ``crs`` member, then
+    longitude / latitude detection); longitude / latitude (EPSG:4326) and WGS84 UTM layers are projected into the tile's
+    UTM zone on the device before the burn, as RasterizeLayer transforms each geometry into the raster's SRS."""
     size = int(ctx.tilesize) + int(ctx.pad) * 2                 # reference :660
-    layer = label_data
+    layer, crs_member = label_data, None
     if isinstance(label_data, (str, bytes, dict)) or hasattr(label_data, "__fspath__"):
-        layer = read_geojson_layer(label_data)
+        gj = _load_geojson(label_data)
+        layer, crs_member = read_geojson_layer(gj), geojson_crs_epsg(gj)
     elif len(label_data) and isinstance(label_data[0], list):   # several layers: GetLayerByIndex(layer_idx), :668
         layer = label_data[layer_idx]
     gt = [float(v) for v in ctx.geotrans]
     if gt[2] != 0.0 or gt[4] != 0.0:
         raise B2Error("create_label_array_for_tile: rotated geotransforms are out of scope (DLTiles are north-up)")
+    tile_epsg = _tile_epsg(ctx)
+    layer_epsg = label_layer_epsg(tile_epsg, label_crs, crs_member, layer)
+    if layer_epsg != tile_epsg:
+        layer = _project_layer(layer, layer_epsg, tile_epsg, device)
     inv1, inv5 = 1.0 / gt[1], 1.0 / gt[5]                       # GDALInvGeoTransform for a north-up raster
     inv0, inv3 = -gt[0] * inv1, -gt[3] * inv5
     feats = []

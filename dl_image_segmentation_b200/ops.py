@@ -797,6 +797,21 @@ def shard_stats(shards, channels, kind="bytes", verify_crc=True, max_records=Non
 
 
 # ------------------------------------------------------------------------------------------------ label rasterisation
+def project_points(xy, src_epsg, dst_epsg, device=None):
+    """(N, 2) float64 vertices (NumPy or tensor) from one CRS to another -> (N, 2) float64 CUDA tensor.  b2_project_points.
+
+    EPSG:4326 (longitude, latitude in degrees, GeoJSON axis order) and WGS84 UTM 326zz / 327zz, both ways and zone to zone;
+    vertices the projection is not valid for come back as (NaN, NaN).  Raises B2Error for any other code.  Replaces the
+    reprojection gdal.RasterizeLayer applies to each geometry (_descartes_img_chips.py:667-688)."""
+    ctx = get_ctx(device)
+    xy = to_device(xy, ctx.device)
+    if xy.dtype != torch.float64 or xy.dim() != 2 or xy.shape[1] != 2:
+        raise B2Error("project_points: expected (N, 2) float64 vertices, got %s %s" % (tuple(xy.shape), xy.dtype))
+    out = torch.empty_like(xy)
+    check(lib().b2_project_points(ctx.handle, ptr(xy), ptr(out), xy.shape[0], int(src_epsg), int(dst_epsg), ctx.stream()))
+    return out
+
+
 def rasterize_polygons(features, size, background_value=255, all_touched=True, device=None):
     """Burn polygons into a (H, W) uint8 CUDA tensor with GDAL's RasterizeLayer semantics (ALL_TOUCHED by default).
 

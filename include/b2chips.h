@@ -469,6 +469,17 @@ int b2_rasterize_polygons(b2_ctx* ctx, const double* fill_segs, const uint32_t* 
                           uint32_t n_line_segs, const uint8_t* values, int n_features, int width, int height, int background,
                           uint32_t max_ints, int32_t* owner_ws, int32_t* ints_ws, uint8_t* out, b2_stream stream);
 
+/* Replaces the on-the-fly reprojection RasterizeLayer applies to every geometry, from the layer's SRS to the raster's, before
+ * it burns (_descartes_img_chips.py:667-688; OGRGeometry::transform, PROJ's `utm`): n interleaved (x, y) double vertices,
+ * in_dev -> out_dev (may be the same buffer).  src_epsg / dst_epsg: 4326 (x = longitude, y = latitude, degrees, GeoJSON axis
+ * order; longitudes come out in [-180, 180)), 326zz (WGS84 UTM north, zone zz = 1..60) or 327zz (south, false northing
+ * 10 000 000 m); k0 = 0.9996, false easting 500 000 m, central meridian -183 + 6 zz degrees.  Krueger series of order 6 in
+ * the third flattening (Karney 2011), FP64; UTM -> UTM goes through latitude / longitude in the same thread; equal codes
+ * copy.  A vertex that is not finite, lies beyond a pole or 90 degrees or more from the destination's central meridian
+ * becomes (NaN, NaN).  An unsupported code is an error.  No datum shifts. */
+int b2_project_points(b2_ctx* ctx, const double* in_dev, double* out_dev, uint64_t n, int src_epsg, int dst_epsg,
+                      b2_stream stream);
+
 #ifdef __cplusplus
 }
 #endif
