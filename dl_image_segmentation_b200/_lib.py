@@ -81,7 +81,7 @@ SIGNATURES = {
     "b2_example_layout_batch": (_i, [_i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _u64, ctypes.POINTER(_u64), ctypes.POINTER(_u64), ctypes.POINTER(_u64)]),
     "b2_tfrecord_build": (_i, [_vp, _vp, _i, _u64, _vp, _vp, _vp]),
     "b2_rasterize_polygons": (_i, [_vp, _vp, _vp, _vp, _vp, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32, _vp, _i, _i, _i, _i,
-                                   ctypes.c_uint32, _vp, _vp, _vp, _vp]),
+                                   _vp, _vp, _vp, _vp, _vp]),
     # the layer -> raster reprojection of gdal.RasterizeLayer (_descartes_img_chips.py:667-688)
     "b2_project_points": (_i, [_vp, _vp, _vp, _u64, _i, _i, _vp]),
 }

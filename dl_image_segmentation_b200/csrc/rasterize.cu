@@ -37,14 +37,15 @@ __device__ __forceinline__ int find_owner(const uint32_t* __restrict__ off, int 
 
 __global__ void __launch_bounds__(128)
 raster_fill_kernel(const double4* __restrict__ segs, const uint32_t* __restrict__ seg_off, const int32_t* __restrict__ feat_miny,
-                   const uint32_t* __restrict__ job_off, int n_features, uint32_t n_jobs, int W, int H, uint32_t max_ints,
-                   int32_t* __restrict__ ints_ws, int32_t* __restrict__ owner) {
+                   const uint32_t* __restrict__ job_off, int n_features, uint32_t n_jobs, int W, int H,
+                   const uint64_t* __restrict__ job_ints_off, int32_t* __restrict__ ints_ws, int32_t* __restrict__ owner) {
     const uint32_t job = blockIdx.x * blockDim.x + threadIdx.x;
     if (job >= n_jobs) return;
     const int f = find_owner(job_off, n_features, job);
     const int y = feat_miny[f] + (int)(job - job_off[f]);
     const double dy = (double)y + 0.5;
-    int32_t* ints = ints_ws + (size_t)job * max_ints;
+    int32_t* ints = ints_ws + job_ints_off[job];
+    const uint32_t cap = (uint32_t)(job_ints_off[job + 1] - job_ints_off[job]);
     uint32_t n = 0;
     for (uint32_t s = seg_off[f]; s < seg_off[f + 1]; s++) {
         const double4 e = segs[s];                                   // (x1, y1) -> (x2, y2), ind1 = the earlier vertex
@@ -62,11 +63,11 @@ raster_fill_kernel(const double4* __restrict__ segs, const uint32_t* __restrict_
         }
         if (dy < dy2 && dy >= dy1) {
             const double inter = dadd(ddiv(dmul(dsub(dy, dy1), dsub(dx2, dx1)), dsub(dy2, dy1)), dx1);
-            if (n < max_ints) ints[n] = (int)floor(dadd(inter, 0.5));
+            if (n < cap) ints[n] = (int)floor(dadd(inter, 0.5));
             n++;
         }
     }
-    if (n > max_ints) n = max_ints;                                  // cannot happen: max_ints = the feature's edge count
+    if (n > cap) n = cap;                                            // cannot happen: cap >= the edges this row can cross
     for (uint32_t i = 1; i < n; i++) {                               // crossings per scanline are few: insertion sort
         const int32_t v = ints[i];
         uint32_t j = i;
@@ -304,13 +305,13 @@ using namespace b2;
 extern "C" int b2_rasterize_polygons(b2_ctx* ctx, const double* fill_segs, const uint32_t* fill_seg_off, const int32_t* feat_miny,
                                      const uint32_t* job_off, uint32_t n_jobs, const double* line_segs, const uint32_t* line_seg_feat,
                                      uint32_t n_line_segs, const uint8_t* values, int n_features, int width, int height,
-                                     int background, uint32_t max_ints, int32_t* owner_ws, int32_t* ints_ws, uint8_t* out,
+                                     int background, const uint64_t* job_ints_off, int32_t* owner_ws, int32_t* ints_ws, uint8_t* out,
                                      b2_stream stream) {
     B2_REQUIRE(ctx && out && owner_ws, "b2_rasterize_polygons: NULL argument");
     B2_REQUIRE(width > 0 && height > 0 && (uint64_t)width * height < (1ull << 31), "b2_rasterize_polygons: bad raster size");
     B2_REQUIRE(n_features >= 0 && background >= 0 && background <= 255, "b2_rasterize_polygons: bad argument");
     B2_REQUIRE(n_features == 0 || (fill_seg_off && feat_miny && job_off && values), "b2_rasterize_polygons: NULL feature table");
-    B2_REQUIRE(n_jobs == 0 || (fill_segs && ints_ws && max_ints > 0), "b2_rasterize_polygons: NULL fill table");
+    B2_REQUIRE(n_jobs == 0 || (fill_segs && job_ints_off && ints_ws), "b2_rasterize_polygons: NULL fill table");
     B2_REQUIRE(n_line_segs == 0 || (line_segs && line_seg_feat), "b2_rasterize_polygons: NULL line table");
     DeviceGuard g(ctx->device);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -320,7 +321,8 @@ extern "C" int b2_rasterize_polygons(b2_ctx* ctx, const double* fill_segs, const
     ctx->launches++;
     if (n_jobs) {
         raster_fill_kernel<<<(n_jobs + 127) / 128, 128, 0, s>>>(reinterpret_cast<const double4*>(fill_segs), fill_seg_off, feat_miny,
-                                                                  job_off, n_features, n_jobs, width, height, max_ints, ints_ws, owner_ws);
+                                                                  job_off, n_features, n_jobs, width, height, job_ints_off, ints_ws,
+                                                                  owner_ws);
         ctx->launches++;
     }
     if (n_line_segs) {

@@ -812,60 +812,109 @@ def project_points(xy, src_epsg, dst_epsg, device=None):
     return out
 
 
+class RasterLayout:
+    """The tables b2_rasterize_polygons reads, as NumPy arrays (include/b2chips.h): fill (E, 4) / fill_off, miny / job_off
+    (one job per (feature, scanline)), job_ints_off (each job's room for its crossings), lines (L, 4) / line_feat, values."""
+
+    def __init__(self, fill, fill_off, miny, job_off, job_ints_off, lines, line_feat, values):
+        self.fill, self.fill_off, self.miny, self.job_off = fill, fill_off, miny, job_off
+        self.job_ints_off, self.lines, self.line_feat, self.values = job_ints_off, lines, line_feat, values
+
+    @property
+    def n_jobs(self):
+        return int(self.job_off[-1])
+
+
+def rasterize_layout(features, size, all_touched=True):
+    """The host half of rasterize_polygons (same arguments), on the CPU: lays the edges out and sizes the scanline
+    workspace.  Raises B2Error for a burn value outside 0..255 or a non-finite vertex.
+
+    A feature's scanlines are GDAL's [max((int) min y, 0), min((int) max y, H - 1)]; a feature whose y-range misses the
+    raster has none.  A job's workspace is the number of the feature's non-horizontal edges whose y-span can hold its
+    pixel-centre line (y_lo <= row + 0.5 < y_hi, widened by one row at each end), so it follows the crossings a scanline
+    can have, not the size of the largest feature in the layer."""
+    H, W = (int(size), int(size)) if np.isscalar(size) else (int(size[0]), int(size[1]))
+    verts, vert_feat, fill, n_edges, ring_y, ring_feat, lines, line_feat, values = [], [], [], [], [], [], [], [], []
+    for f, (rings, value) in enumerate(features):
+        if not 0 <= int(value) <= 255:
+            raise B2Error("rasterize_polygons: burn values must be 0..255 (GDT_Byte raster)")
+        values.append(int(value))
+        ne = 0
+        for r in rings:
+            r = np.asarray(r, dtype=np.float64).reshape(-1, 2)
+            verts.append(r)
+            vert_feat.append(np.full(len(r), f, np.int64))
+            if len(r) < 2:
+                continue
+            ring_y.append(r[:, 1])
+            ring_feat.append(f)
+            closed = r[0, 0] == r[-1, 0] and r[0, 1] == r[-1, 1]
+            o = r[:-1] if closed else r                          # fill: every vertex with its predecessor, wrapping around
+            fill.append(np.concatenate([np.roll(o, 1, axis=0), o], axis=1))
+            ne += len(o)
+            if all_touched:                                      # edge walk: the ring as given (GDAL does not close it)
+                lines.append(np.concatenate([r[:-1], r[1:]], axis=1))
+                line_feat.append(np.full(len(r) - 1, f, np.uint32))
+        n_edges.append(ne)
+    nF = len(values)
+    if verts:
+        bad = ~np.isfinite(np.concatenate(verts)).all(axis=1)
+        if bad.any():
+            raise B2Error("rasterize_polygons: feature %d has a non-finite vertex"
+                          % int(np.concatenate(vert_feat)[int(np.argmax(bad))]))
+    # scanlines: (int) truncation of the feature's y-range, as GDAL's miny / maxy, clipped to the raster before any
+    # integer conversion (a feature wholly above or below the raster, however far, has none)
+    ymin, ymax = np.full(nF, np.inf), np.full(nF, -np.inf)
+    if ring_y:
+        np.minimum.at(ymin, ring_feat, [y.min() for y in ring_y])
+        np.maximum.at(ymax, ring_feat, [y.max() for y in ring_y])
+    lo, hi = np.clip(np.trunc(ymin), 0, H), np.clip(np.trunc(ymax), -1, H - 1)
+    rows = np.maximum(hi - lo + 1, 0).astype(np.int64)
+    miny = np.where(rows > 0, lo, 0).astype(np.int32)
+    job_off = np.zeros(nF + 1, np.uint32)
+    np.cumsum(rows, out=job_off[1:])
+    n_jobs = int(job_off[-1])
+    fill_a = np.ascontiguousarray(np.concatenate(fill)) if fill else np.zeros((0, 4))
+    fill_off = np.zeros(nF + 1, np.uint32)
+    np.cumsum(n_edges, out=fill_off[1:])
+    # workspace: every non-horizontal edge adds one slot to each job whose row it can cross, counted in a difference
+    # array over job indices
+    fe = np.repeat(np.arange(nF), n_edges)
+    y1, y2 = fill_a[:, 1], fill_a[:, 3]
+    r0 = np.maximum(np.ceil(np.minimum(y1, y2) - 0.5) - 1, lo[fe])
+    r1 = np.minimum(np.ceil(np.maximum(y1, y2) - 0.5), hi[fe])
+    keep = (y1 != y2) & (r1 >= r0)
+    start = job_off[fe[keep]].astype(np.int64) + (r0[keep] - lo[fe[keep]]).astype(np.int64)
+    end = start + (r1[keep] - r0[keep]).astype(np.int64) + 1
+    diff = np.bincount(start, minlength=n_jobs + 1) - np.bincount(end, minlength=n_jobs + 1)
+    job_ints_off = np.zeros(n_jobs + 1, np.uint64)
+    np.cumsum(np.cumsum(diff[:n_jobs]), out=job_ints_off[1:])
+    line_a = np.ascontiguousarray(np.concatenate(lines)) if lines else np.zeros((0, 4))
+    lf = np.concatenate(line_feat) if line_feat else np.zeros(0, np.uint32)
+    return RasterLayout(fill_a, fill_off, miny, job_off, job_ints_off, line_a, lf, np.asarray(values, np.uint8))
+
+
 def rasterize_polygons(features, size, background_value=255, all_touched=True, device=None):
     """Burn polygons into a (H, W) uint8 CUDA tensor with GDAL's RasterizeLayer semantics (ALL_TOUCHED by default).
 
     features: list of (rings, value) in burn order; rings = list of (N, 2) arrays in PIXEL space (x = column, y = line),
     first ring the shell, the others holes or further polygons (even-odd rule over all of them); value 0..255.
-    The host only lays the edges out (NumPy); the scanline fill, the edge walk and the last-feature-wins resolution run in
-    b2_rasterize_polygons.  Replaces gdal.RasterizeLayer in create_label_array_for_tile (_descartes_img_chips.py:667-688)."""
+    Raises B2Error for a burn value outside 0..255 or a non-finite vertex, naming the feature.
+    The host only lays the edges out (rasterize_layout, NumPy); the scanline fill, the edge walk and the last-feature-wins
+    resolution run in b2_rasterize_polygons.  Replaces gdal.RasterizeLayer in create_label_array_for_tile
+    (_descartes_img_chips.py:667-688)."""
     ctx = get_ctx(device)
     H, W = (int(size), int(size)) if np.isscalar(size) else (int(size[0]), int(size[1]))
-    fill, fill_off, miny, rows, lines, line_feat, values, max_edges = [], [0], [], [], [], [], [], 1
-    for f, (rings, value) in enumerate(features):
-        if not 0 <= int(value) <= 255:
-            raise B2Error("rasterize_polygons: burn values must be 0..255 (GDT_Byte raster)")
-        values.append(int(value))
-        n_edges, ys = 0, []
-        for r in rings:
-            r = np.asarray(r, dtype=np.float64).reshape(-1, 2)
-            if len(r) < 2:
-                continue
-            ys.append(r[:, 1])
-            closed = r[0, 0] == r[-1, 0] and r[0, 1] == r[-1, 1]
-            o = r[:-1] if closed else r                          # fill: every vertex with its predecessor, wrapping around
-            if len(o):
-                fill.append(np.concatenate([np.roll(o, 1, axis=0), o], axis=1))
-                n_edges += len(o)
-            if all_touched:                                      # edge walk: the ring as given (GDAL does not close it)
-                lines.append(np.concatenate([r[:-1], r[1:]], axis=1))
-                line_feat.append(np.full(len(r) - 1, f, np.uint32))
-        fill_off.append(fill_off[-1] + n_edges)
-        max_edges = max(max_edges, n_edges)
-        if n_edges:
-            yy = np.concatenate(ys)
-            lo, hi = max(int(yy.min()), 0), min(int(yy.max()), H - 1)      # (int) truncation, as GDAL's miny / maxy
-            miny.append(lo)
-            rows.append(max(0, hi - lo + 1))
-        else:
-            miny.append(0)
-            rows.append(0)
-    nF = len(values)
-    job_off = np.zeros(nF + 1, np.uint32)
-    np.cumsum(rows, out=job_off[1:])
-    n_jobs = int(job_off[-1])
-    fill_a = np.ascontiguousarray(np.concatenate(fill)) if fill else np.zeros((0, 4))
-    line_a = np.ascontiguousarray(np.concatenate(lines)) if lines else np.zeros((0, 4))
-    lf = np.concatenate(line_feat) if line_feat else np.zeros(0, np.uint32)
-    if n_jobs * max_edges * 4 > (4 << 30):
-        raise B2Error("rasterize_polygons: layer too complex for one call (%d scanline jobs x %d edges)" % (n_jobs, max_edges))
+    L = rasterize_layout(features, (H, W), all_touched)
+    nF, n_jobs = len(L.values), L.n_jobs
     d = lambda a, dt: to_device(np.ascontiguousarray(a, dtype=dt).view(np.uint8).reshape(-1), ctx.device) if np.asarray(a).size else None
-    fill_d, off_d, miny_d, job_d = d(fill_a, np.float64), d(fill_off, np.uint32), d(miny, np.int32), d(job_off, np.uint32)
-    line_d, lf_d, val_d = d(line_a, np.float64), d(lf, np.uint32), d(values, np.uint8)
+    fill_d, off_d, miny_d, job_d = d(L.fill, np.float64), d(L.fill_off, np.uint32), d(L.miny, np.int32), d(L.job_off, np.uint32)
+    line_d, lf_d, val_d = d(L.lines, np.float64), d(L.line_feat, np.uint32), d(L.values, np.uint8)
+    ints_off_d = d(L.job_ints_off, np.uint64) if n_jobs else None
     owner = torch.empty((H * W,), dtype=torch.int32, device=ctx.device)
-    ints = torch.empty((max(1, n_jobs * max_edges),), dtype=torch.int32, device=ctx.device)
+    ints = torch.empty((max(1, int(L.job_ints_off[-1])),), dtype=torch.int32, device=ctx.device)
     out = torch.empty((H, W), dtype=torch.uint8, device=ctx.device)
     check(lib().b2_rasterize_polygons(ctx.handle, ptr(fill_d), ptr(off_d), ptr(miny_d), ptr(job_d), n_jobs, ptr(line_d), ptr(lf_d),
-                                      len(lf), ptr(val_d), nF, W, H, int(background_value), max_edges, ptr(owner), ptr(ints), ptr(out),
-                                      ctx.stream()))
+                                      len(L.line_feat), ptr(val_d), nF, W, H, int(background_value), ptr(ints_off_d), ptr(owner),
+                                      ptr(ints), ptr(out), ctx.stream()))
     return out

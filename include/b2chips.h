@@ -462,12 +462,16 @@ int b2_gather_ranges(b2_ctx* ctx, const uint8_t* src, const uint64_t* src_off, c
  *   fill_seg_off   uint32[n_features + 1]   feat_miny int32[n_features] (first scanline of the feature, clipped to the raster)
  *   job_off        uint32[n_features + 1]   prefix sum of the features' scanline counts; n_jobs = job_off[n_features]
  *   line_segs      double[4] per edge of the ALL_TOUCHED pass (n_line_segs = 0: centre-only burn), line_seg_feat its feature
- *   values         uint8[n_features] burn values; max_ints = most edges of any one feature
- *   owner_ws       int32[width * height] scratch; ints_ws int32[n_jobs * max_ints] scratch; out uint8[height * width] */
+ *   values         uint8[n_features] burn values
+ *   job_ints_off   uint64[n_jobs + 1]   job j sorts its scanline's crossings in ints_ws[job_ints_off[j] .. job_ints_off[j + 1]):
+ *                  at least the number of the feature's non-horizontal edges whose y-span holds that pixel-centre line
+ *                  (a row with more crossings than its room burns only the spans of the first ones)
+ *   owner_ws       int32[width * height] scratch; ints_ws int32[job_ints_off[n_jobs]] scratch; out uint8[height * width]
+ * width * height must be below 2^31. */
 int b2_rasterize_polygons(b2_ctx* ctx, const double* fill_segs, const uint32_t* fill_seg_off, const int32_t* feat_miny,
                           const uint32_t* job_off, uint32_t n_jobs, const double* line_segs, const uint32_t* line_seg_feat,
                           uint32_t n_line_segs, const uint8_t* values, int n_features, int width, int height, int background,
-                          uint32_t max_ints, int32_t* owner_ws, int32_t* ints_ws, uint8_t* out, b2_stream stream);
+                          const uint64_t* job_ints_off, int32_t* owner_ws, int32_t* ints_ws, uint8_t* out, b2_stream stream);
 
 /* Replaces the on-the-fly reprojection RasterizeLayer applies to every geometry, from the layer's SRS to the raster's, before
  * it burns (_descartes_img_chips.py:667-688; OGRGeometry::transform, PROJ's `utm`): n interleaved (x, y) double vertices,
